@@ -11,6 +11,10 @@ cosine logits (K0+K1) -> fused bilinear-upsample + softmax-CE fwd/bwd (K2) -> lo
 all-reduced over NCCL every step (the bucket behind the next step) and the int64 confusion matrix once per pass
 (weak scaling).  After the timed primary step short secondary legs measure BASELINE configs 3, 4, 5 and the x4
 geometry (`secondary` in the JSON line).  Prints ONE JSON line (rank 0).
+
+    python bench.py --dump-outputs DIR ...   # also write what the last timed step computed (rank 0) as DIR/<name>.npy
+
+The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -31,6 +35,7 @@ UNIT = "images/s"
 GEOM = {"A": (32, 32, 512), "B": (128, 128, 512), "5": (64, 64, 1024)}   # (h, w, H = W): SURVEY 8 G-A aux head x16,
 #                                   G-B main head x4; "5" = BASELINE config 5 (1024^2, use --classes 847 --batch 8)
 L2_BYTES = 126 * 1024 * 1024
+DUMP_BYTES = 60 * 10 ** 6          # --dump-outputs: array data of all files together, so that they stay under 64 MB
 
 
 def parse():
@@ -49,7 +54,37 @@ def parse():
     p.add_argument("--no-graph", action="store_true", help="time eager launches instead of CUDA-graph replays")
     p.add_argument("--no-secondary", action="store_true", help="skip the cfg3 / G-B / cfg4 / cfg5 legs")
     p.add_argument("--legs", default="cfg3_eval,G-B,cfg4,cfg5", help="comma-separated secondary legs to run")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the outputs of the last timed step (loss, n_valid, logits, grad_v, grad_t) and the pass's "
+                        "confusion matrix as DIR/<name>.npy (float32 / float64)")
+    a = p.parse_args()
+    if a.steps is not None and a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        p.error("--dump-outputs writes the outputs of --impl b200")
+    return a
+
+
+def write_outputs(arrays, out_dir, budget=DUMP_BYTES, seed=0):
+    """Write every tensor of `arrays` (name -> tensor) as out_dir/<name>.npy: floating point as float32, integers as
+    float64 (exact below 2**53).  Smallest first, each array gets an equal share of what is left of `budget` bytes; an
+    array larger than its share is written as a seeded sample of its flattened elements (sorted positions, the same
+    for the same shape on every run)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    left = budget
+    for i, (name, t) in enumerate(items):
+        t = t.detach().cpu()
+        t = t.float() if t.is_floating_point() else t.double()
+        share = left // (len(items) - i)
+        if t.numel() * t.element_size() > share:
+            g = torch.Generator().manual_seed(seed)
+            idx = torch.randint(t.numel(), (share // t.element_size(),), generator=g).unique()
+            t = t.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+        left -= t.numel() * t.element_size()
 
 
 def workload_name(a, h, w):
@@ -397,6 +432,12 @@ def run_b200(a):
     host_enqueue_ms = (time.perf_counter() - t_host0) * 1e3 / steps     # host time to enqueue one step
     torch.cuda.synchronize()
     sampler.stop_flag = True
+    if a.dump_outputs and rank == 0:
+        # before the eager passes below overwrite the step's buffers; grad_v is not computed without the backward
+        outs = {"loss": step.loss, "n_valid": step.n_valid, "logits": step.logits, "confmat": cm_total}
+        if backward:
+            outs.update(grad_v=step.grad_v, grad_t=step.grad_t)
+        write_outputs(outs, a.dump_outputs)
     barrier()
     launches = _lib.launch_count() - launches0
     ms_total = ev0.elapsed_time(ev1)

@@ -1,8 +1,8 @@
 """Generate the committed golden fixtures by running the REFERENCE itself.
 
-Run in the build container only (needs /root/reference, read-only):
+Needs a checkout of the reference project (LC2IS), read-only:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py /path/to/LC2IS
 
 It imports the reference modules that import cleanly (``model.loss``,
 ``model.text_patch`` - SURVEY 8c) and restates, verbatim with live torch ops, the head
@@ -11,7 +11,8 @@ un-vendored ``model.DenseCLIP`` checkout).  ``metrics.py`` cannot be imported ei
 (torchmetrics is missing), so the confusion-matrix fixtures are produced by a naive
 pure-Python double loop written here, independent of ``oracle/``.
 
-The fixtures travel to the GPU box; /root/reference does not.
+The fixtures are committed, so the tests need no reference checkout.  Every fixture stays under 1 MB:
+head_final.pt keeps the upsampled map of every 4th class only.
 """
 import os
 import sys
@@ -20,16 +21,15 @@ import torch
 import torch.nn.functional as F
 from einops import rearrange
 
-REF = "/root/reference"
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
-def main():
-    sys.path.insert(0, REF)
+def main(ref):
+    sys.path.insert(0, ref)
     from model.loss import AuxiliaryLoss            # reference class, loss.py:12-21
     from model.text_patch import TextToPatch        # reference class, text_patch.py:4-18
 
-    protos = torch.load(os.path.join(REF, "model", "ade20k_prototypes.pt")).detach().float()
+    protos = torch.load(os.path.join(ref, "model", "ade20k_prototypes.pt")).detach().float()
     g = torch.Generator().manual_seed(1024)
 
     # ---- 1. head lines of final.py:37-44 (x4 main head) and :262-268 (aux head) ----------
@@ -43,7 +43,9 @@ def main():
     score_up = F.interpolate(input=score_low, mode="bilinear", scale_factor=4)  # final.py:44
     raw = torch.matmul(v, protos.transpose(1, 0))                       # model.py:50
     raw = rearrange(raw, "b (h w) c -> b c h w", h=h)                   # model.py:53
-    torch.save(dict(v=v, score_low=score_low, score_up=score_up, raw=raw),   # t = bundled prototypes
+    up_classes = torch.arange(0, score_up.shape[1], 4)
+    torch.save(dict(v=v, score_low=score_low, score_up=score_up[:, up_classes].clone(), raw=raw,
+                    up_classes=up_classes),                             # t = bundled prototypes
                os.path.join(OUT, "head_final.pt"))
 
     # ---- 2. AuxiliaryLoss (reference class) fwd + autograd bwd ------------------------------
@@ -134,4 +136,6 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        sys.exit("usage: python tests/golden/make_golden.py /path/to/LC2IS")
+    main(sys.argv[1])

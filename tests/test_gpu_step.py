@@ -178,6 +178,40 @@ def test_one_byte_host_labels_expand_to_the_device_packing(C, ign):
     assert int(nv) == int(nv_ref) == int(((lab >= 0) & (lab < C) & (lab != ign)).sum())
 
 
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path):
+    """`bench.py --steps 2 --dump-outputs DIR`: two timed steps (the confusion matrix of the pass counts two batches)
+    and the dumped loss / n_valid / logits / gradients are those of HeadStep on the second input set."""
+    import json, os, subprocess, sys
+    import numpy as np
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = tmp_path / "dump"
+    r = subprocess.run([sys.executable, "bench.py", "--steps", "2", "--warmup", "1", "--no-e2e", "--no-secondary",
+                        "--no-cpu-baseline", "--dump-outputs", str(out)], cwd=root, capture_output=True, text=True,
+                       timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    B, h, H, C = 16, 32, 512, 150
+    assert line["steps"] == 2 and line["check"]["confmat_total"] == 2 * B * H * H
+    got = {f[:-4]: np.load(out / f) for f in os.listdir(out)}
+    assert set(got) == {"loss", "n_valid", "logits", "confmat", "grad_v", "grad_t"}
+    assert sum(x.nbytes for x in got.values()) <= 64 * 10 ** 6
+    assert got["confmat"].dtype == np.float64 and got["confmat"].sum() == 2 * B * H * H
+
+    seed = synthetic.SEED + 97 * 1                              # bench.py's input set of timed step 1
+    v = synthetic.make_patch_embeddings(B, h * h, 512, seed=seed).to(DEV)
+    lab = synthetic.make_labels(B, H, H, C, seed=seed, ignore_frac=0.1).to(DEV)
+    step = HeadStep(B, h, h, H, H, C, ignore_index=0)
+    step(v, synthetic.make_prototypes(C, 512).to(DEV), lab)
+    torch.cuda.synchronize()
+    assert got["n_valid"].tolist() == [int(step.n_valid)]
+    assert abs(float(got["loss"][0]) - float(step.loss)) <= 1e-5 * abs(float(step.loss))
+    torch.testing.assert_close(torch.from_numpy(got["logits"]), step.logits.cpu(), rtol=1e-5, atol=1e-6)
+    for name, ref in (("grad_t", step.grad_t), ("grad_v", step.grad_v)):
+        ref = ref.float().cpu()
+        assert got[name].shape == tuple(ref.shape)
+        assert float((torch.from_numpy(got[name]) - ref).abs().max()) <= 1e-2 * float(ref.abs().max()), name
+
+
 def test_default_host_step_calibrates_the_label_split():
     """Without `raw_images` the step measures the host's packing rate and the H2D rate and picks how many label maps
     cross as int64; whatever it picks, the results are those of the all-raw step."""

@@ -217,6 +217,32 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and "workload" in line["config"]
 
 
+def test_bench_write_outputs_within_budget_and_repeatable(tmp_path):
+    """bench.py --dump-outputs: float arrays as float32, integer arrays as float64; arrays within their share of the
+    byte budget are written whole, larger ones as a seeded sample of their elements; the same files on every call."""
+    import numpy as np
+    import bench
+    g = torch.Generator().manual_seed(5)
+    arrays = {"loss": torch.tensor([1.5]), "n_valid": torch.tensor([7], dtype=torch.int64),
+              "confmat": torch.randint(0, 1 << 40, (9, 9), generator=g), "logits": torch.randn(40, 30, generator=g),
+              "grad_v": torch.randn(300, 500, generator=g).bfloat16()}
+    budget = 200_000
+    for d in ("a", "b"):
+        bench.write_outputs(arrays, str(tmp_path / d), budget=budget)
+    assert sorted(os.listdir(tmp_path / "a")) == sorted(n + ".npy" for n in arrays)
+    got = {n: np.load(tmp_path / "a" / (n + ".npy")) for n in arrays}
+    assert sum(x.nbytes for x in got.values()) <= budget
+    assert {n: x.dtype for n, x in got.items()} == {"loss": np.float32, "n_valid": np.float64, "confmat": np.float64,
+                                                     "logits": np.float32, "grad_v": np.float32}
+    for n in ("loss", "n_valid", "confmat", "logits"):
+        assert np.array_equal(got[n], (arrays[n].float() if arrays[n].is_floating_point() else arrays[n].double()).numpy())
+    gv = got["grad_v"]
+    assert gv.ndim == 1 and 0.9 * budget / 2 / 4 < gv.size < 300 * 500
+    assert np.isin(gv, arrays["grad_v"].float().numpy()).all()
+    for n in arrays:
+        assert np.array_equal(got[n], np.load(tmp_path / "b" / (n + ".npy")))
+
+
 def test_ftn_decoder_mirrors_run_and_keep_the_reference_parameter_names():
     """decoder.py:36-134 mirrors (pass-through PyTorch, upstream of the head): they run on torch >= 2 (the reference's
     `_sa_block` override lacks `is_causal` there) and name their parameters like the reference."""
