@@ -279,16 +279,16 @@ int lc2is_argmax_confmat_ragged(const float* d_low, int N, int C, int h, int w, 
  * whole-step entries run when lc2is_ce_argmax_fused_supported): per job of two groups one TMA box stages the taps, a row
  * phase (lane = pixel row) does pass A of the cross-entropy and the running argmax in one sweep over the classes, a class
  * phase (lane = class) the tap gradients by Horner sweeps.  Same results as lc2is_upsample_ce_packed followed by
- * lc2is_argmax_confmat_lowres_packed (bilinear).  LC2IS_FUSED_V1=1 selects round 1's warp-specialised kernel. */
+ * lc2is_argmax_confmat_lowres_packed (bilinear). */
 int lc2is_ce_argmax_fused_supported(int C, int h, int w, int H, int W);
 int lc2is_ce_argmax_fused_packed(const float* d_low, const uint16_t* d_labels_packed,
                                  int B, int C, int h, int w, int H, int W,
                                  double* d_loss_sum, float* d_grad_low, int onehot, int64_t* d_n_valid,
                                  int64_t* d_confmat, int64_t* d_per_image, int64_t* d_pred,
                                  lc2is_stream_t stream);
-/* onehot != 0: the argmax warps also add the un-scaled -onehot term to d_grad_low (they hold the row's labels
- * anyway), so the labels only need packing + counting ahead of the kernel (d_n_valid != NULL: the CE warps count too -
- * for labels that arrive packed from the host):
+/* onehot != 0: the kernel also adds the un-scaled -onehot term to d_grad_low (it holds the row's labels anyway), so
+ * the labels only need packing + counting ahead of the kernel (d_n_valid != NULL: the kernel counts too - for labels
+ * that arrive packed from the host):
  * lc2is_pack_labels: int64 [n] -> packed uint16 [n] (same encoding as lc2is_ce_labels_prepass), n_valid += #counted.
  * n % 8 == 0. */
 int lc2is_pack_labels(const int64_t* d_labels, int64_t n, int C, int64_t ignore_index,

@@ -1,7 +1,6 @@
 // C-ABI glue: error text, device probing, scalar helpers and the whole-step-from-host entry.
 #include "common.cuh"
 #include <immintrin.h>
-#include <chrono>
 #include <condition_variable>
 #include <deque>
 #include <mutex>
@@ -239,10 +238,7 @@ long long pack_labels_range(const int64_t* src, void* dst, size_t n, int C, int6
         return have_avx2 ? pack_labels8_avx2(src, (uint8_t*)dst, n, C, ign) : pack_labels8_scalar(src, (uint8_t*)dst, n, C, ign);
     return have_avx2 ? pack_labels_avx2(src, (uint16_t*)dst, n, C, ign) : pack_labels_scalar(src, (uint16_t*)dst, n, C, ign);
 }
-int host_label_bytes(int C) {
-    static const int forced = [] { const char* e = getenv("LC2IS_HOST_LABEL_BYTES"); return e ? atoi(e) : 0; }();
-    return (C <= 254 && forced != 2) ? 1 : 2;
-}
+int host_label_bytes(int C) { return C <= 254 ? 1 : 2; }
 
 // A small persistent worker pool (created on first use, joined at process exit).
 class PackPool {
@@ -390,7 +386,7 @@ static int head_step_enqueue(const void* h_v, const float* h_t, const int64_t* h
                              int64_t ignore_index, float logit_scale, int do_backward,
                              float* h_out_loss, int64_t* h_out_n_valid, int64_t* h_out_confmat,
                              void* d_ws, lc2is_stream_t stream, lc2is_stream_t copy_stream,
-                             void* h_scratch, int n_raw, int flags, int n_chunks, bool async) {
+                             void* h_scratch, int n_raw, int flags, bool async) {
     if (int e = ensure_device()) return e;
     if (!h_v || !h_t || (!h_labels && !h_scratch) || !h_out_loss || !h_out_n_valid || !h_out_confmat || !d_ws)
         return fail(LC2IS_ERR_ARG, "null pointer%s");
@@ -446,15 +442,7 @@ static int head_step_enqueue(const void* h_v, const float* h_t, const int64_t* h
     // chunks: a blocking call overlaps copy and compute inside the step (2 chunks with packed labels, 4 with
     // int64 labels: the copy is the longest stage there); a submitted step overlaps with its neighbours and
     // runs whole-batch kernels (1 chunk)
-    int want_chunks = n_chunks > 0 ? n_chunks : (async ? 1 : (hpack ? 2 : 4));
-    if (getenv("LC2IS_STEP_CHUNKS")) want_chunks = atoi(getenv("LC2IS_STEP_CHUNKS"));
-    if (want_chunks > MAXCH) want_chunks = MAXCH;
-    const bool trace = getenv("LC2IS_STEP_TRACE") != nullptr;
-    auto now = [] { return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-    const double t_begin = now();
-    double t_chunk[MAXCH + 1] = {};
-    std::vector<std::pair<const char*, cudaEvent_t>> tev;
-    auto mark = [&](const char* name, cudaStream_t sx) { if (trace) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, sx); tev.push_back({name, e}); } };
+    const int want_chunks = async ? 1 : (hpack ? 2 : 4);
     const int nchunk = piped ? (B < want_chunks ? B : want_chunks) : 1;
     const int bc = (B + nchunk - 1) / nchunk;
     std::atomic<int> pack_pending[MAXCH];
@@ -491,7 +479,6 @@ static int head_step_enqueue(const void* h_v, const float* h_t, const int64_t* h
             STEP_CUDA(cudaStreamWaitEvent(cst, ev_start, 0));   // `stream` has drained
         }   // (a submitted step owns its workspace: the caller waited for the slot's previous step)
     }
-    mark("start", st);
     STEP_CUDA(cudaMemsetAsync(ws + L.scalars, 0, 256, st));
     STEP_CUDA(cudaMemsetAsync(d_cm, 0, (size_t)C * C * 8, st));
     if (split && do_backward) STEP_CUDA(cudaMemsetAsync(d_glow, 0, M * C * 4, st));
@@ -517,15 +504,13 @@ static int head_step_enqueue(const void* h_v, const float* h_t, const int64_t* h
                 STEP_CUDA(cudaMemcpyAsync(d_packed + lab_off, (const uint16_t*)h_scratch + lab_off,
                                           (size_t)np * H * W * 2, cudaMemcpyHostToDevice, cst));
         }
-        mark("h2d", cst);
         if (piped) {
             STEP_CUDA(cudaEventRecord(ev_copy[i], cst));
             STEP_CUDA(cudaStreamWaitEvent(st, ev_copy[i], 0));
         }
-        t_chunk[i] = now() - t_begin;
         float* lg = d_logits + (size_t)b0 * C * hw;
         float* gl = do_backward ? d_glow + (size_t)b0 * C * hw : nullptr;
-        // labels: the fused K2+K3 kernel only needs them packed and counted (its argmax warps add the -onehot term);
+        // labels: the fused K2+K3 kernel only needs them packed and counted (it adds the -onehot term itself);
         // the separate kernels need the label prepass (count, packing, -onehot)
         if (hpack) {
             // one-byte host labels are widened to the packed form here, int64 ones packed; both count the valid pixels
@@ -547,14 +532,12 @@ static int head_step_enqueue(const void* h_v, const float* h_t, const int64_t* h
                                             d_nvalid, gl, stream));
         else
             STEP_RC(lc2is_count_valid(d_labels + lab_off, (int64_t)nb * H * W, C, ignore_index, d_nvalid, stream));
-        mark("prepass", st);
         if (i == 0) STEP_RC(lc2is_proto_normalize(d_t, 1, C, D, 1, d_that, d_invt, stream));
         // (row normalisation inside the GEMM: no v_hat; the backward takes the raw V)
         STEP_RC(lc2is_cosine_logits_fwd(d_v + v_off, LC2IS_BF16, nb, hw, D, d_that, 1, C, 1, logit_scale,
                                         nullptr, d_invv + (size_t)b0 * hw, lg, stream));
-        mark("k1", st);
         if (fused) {
-            // (two-byte labels packed on the host arrive un-counted: the CE warps count them)
+            // (two-byte labels packed on the host arrive un-counted: the kernel counts them)
             STEP_RC(lc2is_ce_argmax_fused_packed(lg, d_packed + lab_off, nb, C, h, w, H, W, d_loss_sum, gl, 1,
                                                  (hpack && lb == 2) ? d_nvalid : nullptr, d_cm, nullptr, nullptr, stream));
         } else if (split) {
@@ -568,7 +551,6 @@ static int head_step_enqueue(const void* h_v, const float* h_t, const int64_t* h
                                                 d_cm, nullptr, nullptr, stream));
         }
     }
-    mark("k2k3", st);
     STEP_RC(lc2is_mean_scale(d_nvalid, 1.0f, d_gscale, stream));
     if (do_backward) {
         STEP_CUDA(cudaMemsetAsync(ws + L.grad_t, 0, (size_t)C * D * 4, st));
@@ -576,22 +558,12 @@ static int head_step_enqueue(const void* h_v, const float* h_t, const int64_t* h
                                            1, logit_scale, d_gscale, ws + L.grad_v, LC2IS_BF16,
                                            (float*)(ws + L.grad_t), ws + L.bwd_ws, stream, LC2IS_BWD_RAW_V));
     }
-    mark("bwd", st);
     STEP_RC(lc2is_finalize_loss(d_loss_sum, d_nvalid, d_loss, stream));
     // D2H of the step's results (engine.py:108 .item(); :162-163)
     STEP_CUDA(cudaMemcpyAsync(h_out_loss, d_loss, 4, cudaMemcpyDeviceToHost, st));
     STEP_CUDA(cudaMemcpyAsync(h_out_n_valid, d_nvalid, 8, cudaMemcpyDeviceToHost, st));
     STEP_CUDA(cudaMemcpyAsync(h_out_confmat, d_cm, (size_t)C * C * 8, cudaMemcpyDeviceToHost, st));
-    const double t_enq = now() - t_begin;
     if (!async) STEP_CUDA(cudaStreamSynchronize(st));
-    if (trace && !async) {
-        fprintf(stderr, "step trace: chunks %d copies-enqueued-at(us):", nchunk);
-        for (int i = 0; i < nchunk; ++i) fprintf(stderr, " %.0f", t_chunk[i]);
-        fprintf(stderr, " all-enqueued %.0f synced %.0f | gpu(us):", t_enq, now() - t_begin);
-        for (size_t k = 1; k < tev.size(); ++k) { float ms = 0; cudaEventElapsedTime(&ms, tev[0].second, tev[k].second); fprintf(stderr, " %s %.0f", tev[k].first, ms * 1e3); }
-        fprintf(stderr, "\n");
-        for (auto& e : tev) cudaEventDestroy(e.second);
-    }
     cleanup();
 #undef STEP_CUDA
 #undef STEP_RC
@@ -606,7 +578,7 @@ extern "C" int lc2is_head_step_host(const void* h_v, const float* h_t, const int
                                     void* h_scratch, int n_raw, int flags) {
     return head_step_enqueue(h_v, h_t, h_labels, B, h, w, D, C, H, W, ignore_index, logit_scale, do_backward,
                              h_out_loss, h_out_n_valid, h_out_confmat, d_ws, stream, copy_stream, h_scratch, n_raw,
-                             flags, 0, false);
+                             flags, false);
 }
 
 extern "C" int lc2is_head_step_host_submit(const void* h_v, const float* h_t, const int64_t* h_labels,
@@ -618,7 +590,7 @@ extern "C" int lc2is_head_step_host_submit(const void* h_v, const float* h_t, co
     if (!done_event) return fail(LC2IS_ERR_ARG, "done_event is NULL%s");
     if (!copy_stream || copy_stream == stream) return fail(LC2IS_ERR_ARG, "submit needs a separate copy stream%s");
     int e = head_step_enqueue(h_v, h_t, h_labels, B, h, w, D, C, H, W, ignore_index, logit_scale, do_backward,
-                              h_out_loss, h_out_n_valid, h_out_confmat, d_ws, stream, copy_stream, h_scratch, n_raw, flags, 0, true);
+                              h_out_loss, h_out_n_valid, h_out_confmat, d_ws, stream, copy_stream, h_scratch, n_raw, flags, true);
     if (e) return e;
     cudaEvent_t ev;
     LC2IS_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));

@@ -743,12 +743,10 @@ extern "C" int lc2is_linear_fwd(const void* d_x_bf16, const void* d_w_bf16, cons
     P.out = nullptr; P.out_rm = d_y; P.bias = d_bias; P.out_f32 = y_dtype == LC2IS_F32;
     P.fuse_norm = 0; P.inv_v = nullptr;
     P.B = 1; P.hw = (int)M; P.C = N; P.C_pad = N; P.n_sets = 1;
-    // 2-SM form (CTA pairs, 256 x 256 tiles) for shapes it tiles exactly and that fill the GPU more than once;
-    // LC2IS_LINEAR_2SM=0 / 1 forces the choice
-    static const int force_2sm = [] { const char* e = getenv("LC2IS_LINEAR_2SM"); return e ? atoi(e) : -1; }();
+    // 2-SM form (CTA pairs, 256 x 256 tiles) for shapes it tiles exactly and that fill the GPU more than once
     const bool fits_2sm = M % (2 * K1_BM) == 0 && N % K2SM_NB == 0;
     const long long pair_tiles = (M / (2 * K1_BM)) * (N / K2SM_NB);
-    if (fits_2sm && (force_2sm == 1 || (force_2sm != 0 && pair_tiles >= 2LL * (sm_count() / 2)))) {
+    if (fits_2sm && pair_tiles >= 2LL * (sm_count() / 2)) {
         P.num_kb = K / K1_BK; P.scale = 1.f; P.NB = K2SM_NB; P.n_ntiles = N / K2SM_NB; P.tiles_per_img = 0; P.stages = K2SM_STAGES;
         const size_t smem2 = (size_t)K2SM_STAGES * K2SM_STAGE + 1024 + 256 + K1_EPI_SCRATCH;
         CUtensorMap tmA2, tmB2;

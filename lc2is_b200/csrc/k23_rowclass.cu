@@ -22,7 +22,7 @@
 //               PAIR, chunks of 6 classes: "if (cm > best) { best = cm; chunk = k }", then the winning chunk is rescanned
 //               per pixel for the FIRST class that reaches the maximum (torch.argmax's tie rule).
 //             The row then has its log-sum-exp, U(j) = valid / S(j) (to shared memory), target logits, the exact integer
-//             -onehot tap weights (run-length reductions) and its confusion-matrix counts.
+//             -onehot tap weights and its confusion-matrix counts, by a sweep over the pixel columns (match.any over rows).
 //   class phase lane = CLASS: for a (class, group) the 16 x 16 terms are E(y) rho(y)^j with E(y+1) = E(y) sigma and
 //             rho(y+1) = rho(y) tau - four ex2 per (class, group) - and  h = sum_j U(j) rho^j,  d = dh/drho  by one Horner
 //             sweep per row pair (two FFMA2 per pixel pair, U broadcast from shared memory) give the four tap gradients
@@ -64,8 +64,7 @@ struct RCParams {
     unsigned* ctr;                   // {next job of the dynamic rounds, finished warps}: zero at launch, reset by the last warp
     unsigned cells_bytes;            // shared memory per warp: TMA landing zone (later the U tile), multiple of 128
     unsigned quads_bytes;            // shared memory per warp: quads + mbarrier
-    unsigned stagger_ns;             // start delay unit: warp w of a CTA starts ((w >> stagger_shift) & 3) units late (0 = off)
-    unsigned stagger_shift;          // 0: the four schedulers of the SM against each other; 2: the four warps of a scheduler
+    unsigned stagger_ns;             // start delay unit: warp w of a CTA starts ((w >> 2) & 3) units late (0 = off)
 };
 
 __device__ __forceinline__ void tma_load_4d(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int x, int y, int z,
@@ -120,9 +119,7 @@ __device__ __forceinline__ void rc_stage(const RCParams& P, const CUtensorMap* t
     }
 }
 
-// COLS: the labels / predictions of a job are handled by a sweep over the 16 pixel COLUMNS (match.any over the 32 rows)
-// instead of per-row run loops (LC2IS_RC_RUNS=1 selects the run loops).
-template <int S, bool COLS>
+template <int S>
 __global__ void __launch_bounds__(512, 1)
 k23_rc_kernel(const __grid_constant__ CUtensorMap tm, const __grid_constant__ RCParams P) {
     static_assert(S == 16, "x16 geometry");
@@ -177,7 +174,7 @@ k23_rc_kernel(const __grid_constant__ CUtensorMap tm, const __grid_constant__ RC
     // De-phasing: all warps start in step and stay nearly in step (equal jobs), so the SM's 16 warps are in the FMA-bound row
     // phase together and in the LDS-bound class phase together - the first job takes 73 us against 56 us once the warps have
     // drifted apart (tools/k23_timeline.py).  A staggered start trades a few us of idle warps for mixed phases from the start.
-    if (P.stagger_ns) __nanosleep((unsigned)((warp >> P.stagger_shift) & 3) * P.stagger_ns);
+    if (P.stagger_ns) __nanosleep((unsigned)((warp >> 2) & 3) * P.stagger_ns);
     // row-phase lane mapping
     const int gi = lane >> 4, i = lane & 15;
     const float ly = ((float)i + 0.5f) * RS;
@@ -397,164 +394,47 @@ k23_rc_kernel(const __grid_constant__ CUtensorMap tm, const __grid_constant__ RC
             if (vm) loss = slow_ce_row<RC_S>(SlowCtx{P.low, P.grad, P.C, P.h, P.w}, n, ky, kx, i, vm);
         }
 
-        // ---- the row's labels and predictions, by RUNS (labels are piecewise constant along a row) ------------------
-        //   * a run of equal counted labels: its target logits (closed form over the run's columns) and its -onehot term
-        //     of dL/dlogits as exact integer tap weights (lambda * 2S): four float reductions per run
-        //   * a run of equal (target, prediction) pairs: one 64-bit reduction into the confusion matrix
-        // Run starts are found with the labels still in registers; the loops over the runs index the row through
-        // (label, prediction) records in the still idle U tile.
+        // ---- the row's labels and predictions: a sweep over the 16 pixel COLUMNS (column j of all 32 rows at once) --
+        //   confusion matrix: one 64-bit reduction per distinct (target, prediction) pair of the column
+        //   cross-entropy   : the pixel's target logit; the -onehot term as exact integer tap weights summed over the
+        //                     rows of the same group that carry the same label (their row-weight sums follow from
+        //                     the match mask alone), four float reductions per distinct (label, group)
+        // The sweep reads the row's (label, prediction) records back from the still idle U tile.
         {
             const unsigned inmask = !row_in ? 0u : (x0 < 0 ? 0xff00u : (x0 + S > P.W ? 0x00ffu : 0xffffu));
             unsigned* rec = reinterpret_cast<unsigned*>(Usm) + lane;
-            if constexpr (COLS) {
-                // ---- column sweep: column j of all 32 rows at once ---------------------------------------------------
-                //   confusion matrix: one 64-bit reduction per distinct (target, prediction) pair of the column
-                //   cross-entropy   : the pixel's target logit; the -onehot term as exact integer tap weights summed over the
-                //                     rows of the same group that carry the same label (their row-weight sums follow from
-                //                     the match mask alone), four float reductions per distinct (label, group)
 #pragma unroll
-                for (int j = 0; j < S; ++j) {
-                    const unsigned lab = (lw16[j >> 1] >> (16 * (j & 1))) & 0xffffu;
-                    rec[j * 32] = lab | ((unsigned)bidx[j] << 16);
-                }
-                if (P.pred != nullptr && inmask) {
-                    long long* prow = P.pred + ((size_t)n * P.H + y) * P.W + x0;
+            for (int j = 0; j < S; ++j) {
+                const unsigned lab = (lw16[j >> 1] >> (16 * (j & 1))) & 0xffffu;
+                rec[j * 32] = lab | ((unsigned)bidx[j] << 16);
+            }
+            if (P.pred != nullptr && inmask) {
+                long long* prow = P.pred + ((size_t)n * P.H + y) * P.W + x0;
 #pragma unroll
-                    for (int j = 0; j < S; ++j)
-                        if ((inmask >> j) & 1u) prow[j] = bidx[j];
-                }
-                const int Ya = clampi2(ky, 0, P.h - 1), Yb = clampi2(ky + 1, 0, P.h - 1);
-                const int Xa = clampi2(kx, 0, P.w - 1), Xb = clampi2(kx + 1, 0, P.w - 1);
-                const int oA = Ya * P.w + Xa, oB = Ya * P.w + Xb, oC = Yb * P.w + Xa, oD = Yb * P.w + Xb;
-                const float* lbase = P.low + (size_t)n * C * plane;
-                float* gbase = (P.grad && P.onehot) ? P.grad + (size_t)n * C * plane : nullptr;
-                unsigned long long* pimg = P.per_image ? P.per_image + (size_t)n * 3 * C : nullptr;
-                constexpr float WSC = 1.f / (float)(4 * S * S);
-                float tsub = 0.f;
+                for (int j = 0; j < S; ++j)
+                    if ((inmask >> j) & 1u) prow[j] = bidx[j];
+            }
+            const int Ya = clampi2(ky, 0, P.h - 1), Yb = clampi2(ky + 1, 0, P.h - 1);
+            const int Xa = clampi2(kx, 0, P.w - 1), Xb = clampi2(kx + 1, 0, P.w - 1);
+            const int oA = Ya * P.w + Xa, oB = Ya * P.w + Xb, oC = Yb * P.w + Xa, oD = Yb * P.w + Xb;
+            const float* lbase = P.low + (size_t)n * C * plane;
+            float* gbase = (P.grad && P.onehot) ? P.grad + (size_t)n * C * plane : nullptr;
+            unsigned long long* pimg = P.per_image ? P.per_image + (size_t)n * 3 * C : nullptr;
+            constexpr float WSC = 1.f / (float)(4 * S * S);
+            float tsub = 0.f;
 #pragma unroll 2
-                for (int j = 0; j < S; ++j) {
-                    const unsigned r = rec[j * 32];
-                    const unsigned lab = r & 0xffffu;
-                    const int t = (int)(lab & 0x7fffu), pr = (int)(r >> 16);      // bit 15: ignore flag of the CE
-                    const bool c = (vm >> j) & 1u, v = ((inmask >> j) & 1u) && t < C;
-                    const unsigned actv = __ballot_sync(0xffffffffu, v);
-                    if (v) {
-                        const int key = t * C + pr;
-                        const unsigned m = __match_any_sync(actv, key);
-                        if (lane == __ffs(m) - 1) {
-                            const unsigned long long cnt = (unsigned long long)__popc(m);
-                            atomicAdd(&P.confmat[key], cnt);
-                            if (pimg) {
-                                if (t == pr) atomicAdd(&pimg[t], cnt);
-                                atomicAdd(&pimg[C + t], cnt);
-                                atomicAdd(&pimg[2 * C + pr], cnt);
-                            }
-                        }
-                    }
-                    const unsigned actc = __ballot_sync(0xffffffffu, c);
-                    if (c) {
-                        float4 q;
-                        if (!slow) q = Q[lab * 2];
-                        else {
-                            const float* t4 = lbase + (size_t)lab * plane;
-                            q = rc_quad<RC_S>(__ldg(t4 + oA), __ldg(t4 + oB), __ldg(t4 + oC), __ldg(t4 + oD));
-                        }
-                        tsub += fmaf((float)j, fmaf(ly, q.w, q.z), fmaf(ly, q.y, q.x));
-                        if (gbase) {
-                            const unsigned m = __match_any_sync(actc, lab | ((unsigned)gi << 16));
-                            if (lane == __ffs(m) - 1) {
-                                const unsigned mm = (m >> (16 * gi)) & 0xffffu;          // bit i = row i of this group
-                                const int cnt = __popc(mm);
-                                const int si = __popc(mm & 0xAAAAu) + 2 * __popc(mm & 0xCCCCu) + 4 * __popc(mm & 0xF0F0u) +
-                                               8 * __popc(mm & 0xFF00u);                // sum of the row indices
-                                const int sb = 2 * si + cnt, st = 2 * S * cnt - sb;      // sums of (2i+1), 2S - (2i+1)
-                                const float c1 = -WSC * (float)(2 * j + 1), c0 = -WSC * (float)(2 * S - (2 * j + 1));
-                                float* gp = gbase + (size_t)lab * plane;
-                                red_add_f32(gp + oA, c0 * (float)st); red_add_f32(gp + oB, c1 * (float)st);
-                                red_add_f32(gp + oC, c0 * (float)sb); red_add_f32(gp + oD, c1 * (float)sb);
-                            }
-                        }
-                    }
-                }
-                loss -= tsub;
-            } else {
-                unsigned ce_start = 0, cm_start = 0, cmv = 0;
-                int prev_lab = -1, prev_key = -1;
-    #pragma unroll
-                for (int j = 0; j < S; ++j) {
-                    const unsigned lab = (lw16[j >> 1] >> (16 * (j & 1))) & 0xffffu;
-                    const int t = (int)(lab & 0x7fffu);                           // bit 15: ignore flag of the CE
-                    const bool c = (vm >> j) & 1u, v = ((inmask >> j) & 1u) && t < C;
-                    const int key = t * C + bidx[j];
-                    if (c && (int)lab != prev_lab) ce_start |= 1u << j;
-                    if (v && key != prev_key) cm_start |= 1u << j;
-                    prev_lab = c ? (int)lab : -1;
-                    prev_key = v ? key : -1;
-                    cmv |= (v ? 1u : 0u) << j;
-                    rec[j * 32] = lab | ((unsigned)bidx[j] << 16);
-                }
-                if (P.pred != nullptr && inmask) {
-                    long long* prow = P.pred + ((size_t)n * P.H + y) * P.W + x0;
-    #pragma unroll
-                    for (int j = 0; j < S; ++j)
-                        if ((inmask >> j) & 1u) prow[j] = bidx[j];
-                }
-                // end of the run that starts at j0: the next column that starts a run or is not counted
-                auto run_end = [](unsigned starts, unsigned counted, int j0) {
-                    const unsigned brk = ((starts | ~counted) & 0xffffu) >> (j0 + 1);
-                    return brk ? j0 + __ffs(brk) : S;
-                };
-                // -- cross-entropy runs
-                {
-                    const int Ya = clampi2(ky, 0, P.h - 1), Yb = clampi2(ky + 1, 0, P.h - 1);
-                    const int Xa = clampi2(kx, 0, P.w - 1), Xb = clampi2(kx + 1, 0, P.w - 1);
-                    const int oA = Ya * P.w + Xa, oB = Ya * P.w + Xb, oC = Yb * P.w + Xa, oD = Yb * P.w + Xb;
-                    const float* lbase = P.low + (size_t)n * C * plane;
-                    float* gbase = (P.grad && P.onehot) ? P.grad + (size_t)n * C * plane : nullptr;
-                    constexpr float WSC = 1.f / (float)(4 * S * S);
-                    const float wt = -(float)(2 * S - (2 * i + 1)) * WSC, wb = -(float)(2 * i + 1) * WSC;   // top / bottom taps
-                    float tsub = 0.f;
-                    // (warp-uniform trip count: a loop the lanes leave one by one came back from its convergence barrier in
-                    // pieces, and the class phase below then ran once per piece - ncu: 16 active threads, twice the instructions)
-                    unsigned m = ce_start;
-    #pragma unroll 1
-                    while (__any_sync(0xffffffffu, m != 0)) {
-                        if (!m) continue;
-                        const int j0 = __ffs(m) - 1;
-                        m &= m - 1;
-                        const int j1 = run_end(ce_start, vm, j0);
-                        const int lab = (int)(rec[j0 * 32] & 0xffffu);
-                        const int len = j1 - j0, sumj = (len * (j0 + j1 - 1)) >> 1;     // sum of the run's column indices
-                        const int sw1 = 2 * sumj + len, sw0 = 2 * S * len - sw1;          // sums of (2j+1), 2S - (2j+1)
-                        float4 q;
-                        if (!slow) q = Q[lab * 2];
-                        else {
-                            const float* t4 = lbase + (size_t)lab * plane;
-                            q = rc_quad<RC_S>(__ldg(t4 + oA), __ldg(t4 + oB), __ldg(t4 + oC), __ldg(t4 + oD));
-                        }
-                        // sum over the run of v(j) = v0 + j * delta
-                        tsub += fmaf((float)sumj, fmaf(ly, q.w, q.z), (float)len * fmaf(ly, q.y, q.x));
-                        if (gbase) {
-                            float* gp = gbase + (size_t)lab * plane;
-                            red_add_f32(gp + oA, wt * (float)sw0); red_add_f32(gp + oB, wt * (float)sw1);
-                            red_add_f32(gp + oC, wb * (float)sw0); red_add_f32(gp + oD, wb * (float)sw1);
-                        }
-                    }
-                    loss -= tsub;
-                }
-                // -- confusion-matrix runs
-                {
-                    unsigned long long* pimg = P.per_image ? P.per_image + (size_t)n * 3 * C : nullptr;
-                    unsigned m = cm_start;
-    #pragma unroll 1
-                    while (__any_sync(0xffffffffu, m != 0)) {
-                        if (!m) continue;
-                        const int j0 = __ffs(m) - 1;
-                        m &= m - 1;
-                        const unsigned long long cnt = (unsigned long long)(run_end(cm_start, cmv, j0) - j0);
-                        const unsigned r = rec[j0 * 32];
-                        const int t = (int)(r & 0x7fffu), pr = (int)(r >> 16);
-                        atomicAdd(&P.confmat[t * C + pr], cnt);
+            for (int j = 0; j < S; ++j) {
+                const unsigned r = rec[j * 32];
+                const unsigned lab = r & 0xffffu;
+                const int t = (int)(lab & 0x7fffu), pr = (int)(r >> 16);      // bit 15: ignore flag of the CE
+                const bool c = (vm >> j) & 1u, v = ((inmask >> j) & 1u) && t < C;
+                const unsigned actv = __ballot_sync(0xffffffffu, v);
+                if (v) {
+                    const int key = t * C + pr;
+                    const unsigned m = __match_any_sync(actv, key);
+                    if (lane == __ffs(m) - 1) {
+                        const unsigned long long cnt = (unsigned long long)__popc(m);
+                        atomicAdd(&P.confmat[key], cnt);
                         if (pimg) {
                             if (t == pr) atomicAdd(&pimg[t], cnt);
                             atomicAdd(&pimg[C + t], cnt);
@@ -562,7 +442,32 @@ k23_rc_kernel(const __grid_constant__ CUtensorMap tm, const __grid_constant__ RC
                         }
                     }
                 }
+                const unsigned actc = __ballot_sync(0xffffffffu, c);
+                if (c) {
+                    float4 q;
+                    if (!slow) q = Q[lab * 2];
+                    else {
+                        const float* t4 = lbase + (size_t)lab * plane;
+                        q = rc_quad<RC_S>(__ldg(t4 + oA), __ldg(t4 + oB), __ldg(t4 + oC), __ldg(t4 + oD));
+                    }
+                    tsub += fmaf((float)j, fmaf(ly, q.w, q.z), fmaf(ly, q.y, q.x));
+                    if (gbase) {
+                        const unsigned m = __match_any_sync(actc, lab | ((unsigned)gi << 16));
+                        if (lane == __ffs(m) - 1) {
+                            const unsigned mm = (m >> (16 * gi)) & 0xffffu;          // bit i = row i of this group
+                            const int cnt = __popc(mm);
+                            const int si = __popc(mm & 0xAAAAu) + 2 * __popc(mm & 0xCCCCu) + 4 * __popc(mm & 0xF0F0u) +
+                                           8 * __popc(mm & 0xFF00u);                // sum of the row indices
+                            const int sb = 2 * si + cnt, st = 2 * S * cnt - sb;      // sums of (2i+1), 2S - (2i+1)
+                            const float c1 = -WSC * (float)(2 * j + 1), c0 = -WSC * (float)(2 * S - (2 * j + 1));
+                            float* gp = gbase + (size_t)lab * plane;
+                            red_add_f32(gp + oA, c0 * (float)st); red_add_f32(gp + oB, c1 * (float)st);
+                            red_add_f32(gp + oC, c0 * (float)sb); red_add_f32(gp + oD, c1 * (float)sb);
+                        }
+                    }
+                }
             }
+            loss -= tsub;
             __syncwarp();
         }
         // ---- log-sum-exp of the row, U = valid / S -> shared memory (class phase) ---------------------------------
@@ -793,13 +698,9 @@ int launch_k23_rc(const float* d_low, const uint16_t* d_labels_packed, int B, in
     if (P.njobs > 0x3fffffffLL) return fail(LC2IS_ERR_SHAPE, "too many groups for one launch%s");
     P.cells_bytes = (unsigned)rc_cells_bytes(C);
     P.quads_bytes = (unsigned)rc_quads_bytes(C);
-    // staggered start (see the kernel): on when a warp gets three jobs or more - with fewer the idle time is not won back;
-    // LC2IS_RC_STAGGER=<ns per step> / LC2IS_RC_STAGGER_SHIFT override (0 ns = off)
-    static const int stagger_env = getenv("LC2IS_RC_STAGGER") ? atoi(getenv("LC2IS_RC_STAGGER")) : -1;
-    static const int stagger_shift_env = getenv("LC2IS_RC_STAGGER_SHIFT") ? atoi(getenv("LC2IS_RC_STAGGER_SHIFT")) : 2;
-    P.stagger_ns = stagger_env >= 0 ? (unsigned)stagger_env : (P.njobs >= 3LL * sm_count() * nw ? 8000u : 0u);
-    P.stagger_shift = stagger_shift_env == 0 ? 0u : 2u;
-    P.use_tma = (C <= 256 && w % 4 == 0 && ((uintptr_t)d_low % 16) == 0 && !getenv("LC2IS_RC_NO_TMA")) ? 1 : 0;
+    // staggered start (see the kernel): on when a warp gets three jobs or more - with fewer the idle time is not won back
+    P.stagger_ns = P.njobs >= 3LL * sm_count() * nw ? 8000u : 0u;
+    P.use_tma = (C <= 256 && w % 4 == 0 && ((uintptr_t)d_low % 16) == 0) ? 1 : 0;
     CUtensorMap tm;
     memset(&tm, 0, sizeof(tm));
     if (P.use_tma)
@@ -809,9 +710,7 @@ int launch_k23_rc(const float* d_low, const uint16_t* d_labels_packed, int B, in
     static cudaError_t attr_err = cudaSuccess;
     static unsigned* ctr_pool = nullptr;                    // RC_CTR_SLOTS self-resetting counter pairs, used round-robin
     std::call_once(once, [] {
-        attr_err = cudaFuncSetAttribute(k23_rc_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        if (attr_err == cudaSuccess)
-            attr_err = cudaFuncSetAttribute(k23_rc_kernel<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        attr_err = cudaFuncSetAttribute(k23_rc_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         if (attr_err == cudaSuccess) attr_err = cudaMalloc(&ctr_pool, RC_CTR_SLOTS * 2 * sizeof(unsigned));
         if (attr_err == cudaSuccess) attr_err = cudaMemset(ctr_pool, 0, RC_CTR_SLOTS * 2 * sizeof(unsigned));
     });
@@ -821,9 +720,7 @@ int launch_k23_rc(const float* d_low, const uint16_t* d_labels_packed, int B, in
     P.ctr = ctr_pool + 2 * (seq.fetch_add(1, std::memory_order_relaxed) % RC_CTR_SLOTS);
     long long ctas = (P.njobs + nw - 1) / nw;
     if (ctas > sm_count()) ctas = sm_count();
-    static const bool runs = getenv("LC2IS_RC_RUNS") != nullptr;
-    if (runs) k23_rc_kernel<16, false><<<(unsigned)ctas, nw * 32, smem, st>>>(tm, P);
-    else k23_rc_kernel<16, true><<<(unsigned)ctas, nw * 32, smem, st>>>(tm, P);
+    k23_rc_kernel<16><<<(unsigned)ctas, nw * 32, smem, st>>>(tm, P);
     LC2IS_CHECK_LAUNCH("k23_rc_kernel");
     return 0;
 }

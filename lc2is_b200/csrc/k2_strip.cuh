@@ -1,5 +1,5 @@
-// K2 strip path (scale 8 / 16): device code shared by k2_strip_kernel (k2_upsample_ce.cu) and the fused K2+K3 kernel
-// (k3_confmat.cu).  See the comment block above k2_strip_warp for the algorithm.
+// K2 strip path (scale 8 / 16): device code of k2_strip_kernel / k2_strip_gtaps_kernel (k2_upsample_ce.cu); its helpers
+// (cp.async, packed fp32x2 arithmetic) serve K3 and k23_rc as well.  See the comment block above k2_strip_warp.
 #pragma once
 #include "common.cuh"
 #include <type_traits>
@@ -168,10 +168,8 @@ __device__ __noinline__ float k2_strip_slow(const TQ tq, unsigned vm, int n, int
     return loss;
 }
 
-// CSF = floats per class of the tile the warp's quads live in (16 for the stand-alone kernel's per-warp tile, 64 for
-// the 16-group CTA tile of the fused K2+K3 kernel); st = the warp's first tap quad of class 0.
-// CTA_SYNC: the taps were staged by the whole CTA (barrier instead of a warp sync).
-template <int S, bool SPLIT, int CSF, bool CTA_SYNC, int UNR = 2, bool GTAPS = false>
+// CSF = floats per class of the warp's tile of quads; st = the warp's first tap quad of class 0.
+template <int S, bool SPLIT, int CSF, bool GTAPS = false>
 __device__ __forceinline__ void k2_strip_warp(const K2SParams& P, float* st, bool active, int n, int GY0,
                                               int GX0, int lane) {
     constexpr int TPG = S / 2;                              // threads (lanes) per group
@@ -240,7 +238,7 @@ __device__ __forceinline__ void k2_strip_warp(const K2SParams& P, float* st, boo
             }
     }
     cp_async_wait_all();
-    if constexpr (CTA_SYNC) __syncthreads(); else __syncwarp();
+    __syncwarp();
     if (!active) return;                                    // (after the barrier)
     if constexpr (SPLIT) {
         if (P.n_valid != nullptr) {                             // valid count of the warp's strips: one reduction per warp
@@ -326,7 +324,7 @@ __device__ __forceinline__ void k2_strip_warp(const K2SParams& P, float* st, boo
             float2 eN, rN;
             row_exp(tq.get(0), eN, rN);
             float4 qn = tq.get(1);
-#pragma unroll UNR
+#pragma unroll 2
             for (int c = 0; c < C; ++c) {
                 float2 e2 = eN;
                 const float2 r2 = rN;
@@ -415,7 +413,7 @@ __device__ __forceinline__ void k2_strip_warp(const K2SParams& P, float* st, boo
             float2 eN, rN;
             row_exp(tq.get(0), eN, rN);
             float4 qn = tq.get(1);
-#pragma unroll UNR
+#pragma unroll 2
             for (int c = 0; c < C; ++c) {
                 const float2 e2 = eN, r2 = rN;
                 row_exp(qn, eN, rN);                         // class c+1

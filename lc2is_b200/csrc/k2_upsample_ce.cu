@@ -453,7 +453,7 @@ k2_strip_kernel(const K2SParams P) {
             else dst[c * CS] = 0.f;
         }
     }
-    k2_strip_warp<S, SPLIT, CS, false>(P, st, true, n, GY0, GX0, lane);
+    k2_strip_warp<S, SPLIT, CS>(P, st, true, n, GY0, GX0, lane);
 }
 
 // The same strips with the taps read from the class-plane-major map itself (no staged tile): for class counts whose
@@ -469,7 +469,7 @@ k2_strip_gtaps_kernel(const K2SParams P) {
     const int n = (int)(wt / tiles_per_img);
     const int trem = (int)(wt - (long long)n * tiles_per_img);
     const int tyi = trem / P.ntx, txi = trem - tyi * P.ntx;
-    k2_strip_warp<S, SPLIT, CS, false, 2, true>(P, nullptr, true, n, tyi * 2, txi * WGX, lane);
+    k2_strip_warp<S, SPLIT, CS, true>(P, nullptr, true, n, tyi * 2, txi * WGX, lane);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -759,12 +759,6 @@ extern "C" int lc2is_grad_to_bf16(const float* d_grad, int B, int C, int hw, voi
     return 0;
 }
 
-// (LC2IS_K2_GTAPS_BYTES overrides the threshold: 0 = always read the taps from global memory)
-static size_t k2_gtaps_threshold() {
-    static const long long v = [] { const char* e = getenv("LC2IS_K2_GTAPS_BYTES"); return e ? atoll(e) : -1LL; }();
-    return v >= 0 ? (size_t)v : K2_GTAPS_SMEM;
-}
-
 extern "C" int lc2is_upsample_ce_fwd_bwd(const float* d_low, const int64_t* d_labels,
                                          int B, int C, int h, int w, int H, int W,
                                          int64_t ignore_index, const float* d_grad_scale,
@@ -793,7 +787,7 @@ extern "C" int lc2is_upsample_ce_fwd_bwd(const float* d_low, const int64_t* d_la
         int wpc = 4;
         while (wpc > 1 && smem_warp * wpc > 56 * 1024) wpc /= 2;
         const size_t smem = smem_warp * wpc;
-        const bool gtaps = smem_warp > k2_gtaps_threshold();        // staged tile too large for a decent occupancy
+        const bool gtaps = smem_warp > K2_GTAPS_SMEM;               // staged tile too large for a decent occupancy
         if (smem <= 200 * 1024 || gtaps) {
             const int wgx = (64 / s) / 2;
             P.nty = (h + 1 + 1) / 2;
@@ -1015,7 +1009,7 @@ extern "C" int lc2is_upsample_ce_packed(const float* d_low, const uint16_t* d_la
     int wpc = 4;
     while (wpc > 1 && smem_warp * wpc > 56 * 1024) wpc /= 2;
     const size_t smem = smem_warp * wpc;
-    const bool gtaps = smem_warp > k2_gtaps_threshold();            // staged tile too large for a decent occupancy
+    const bool gtaps = smem_warp > K2_GTAPS_SMEM;                   // staged tile too large for a decent occupancy
     const int wgx = (64 / s) / 2;
     P.nty = (h + 1 + 1) / 2;
     P.ntx = (w + 1 + wgx - 1) / wgx;

@@ -435,7 +435,6 @@ struct K3SParams {
     unsigned long long* per_image;
     long long* pred_out;
     int N, C, h, w, H, W, lh, lw;
-    float* onehot_grad;           // fused kernel only: [N,C,h,w] fp32, receives the un-scaled -onehot term (or null)
 };
 
 __device__ __forceinline__ float k3_strip_value(const float4 q, float ly, float lx0, float rsx, int j) {
@@ -445,11 +444,9 @@ __device__ __forceinline__ float k3_strip_value(const float4 q, float ly, float 
 }
 
 // One row (S pixels) of one group per lane.  st4 = the group's tap quad of class 0, CS4 = float4 stride between
-// classes; (ly, lx0, rsx): lambda_y of the row and lambda_x(j) = lx0 + j * rsx.  FUSED: called by the argmax warps of the
-// fused K2+K3 kernel - the staged taps are index-CLAMPED there (K2's convention; identical for finite logits), so
-// non-finite taps are handled by the exact per-pixel path on the global low-resolution map with ATen's taps.
-// SYNC: 0 = the caller has synchronised, 1 = wait for this lane's cp.async + __syncwarp, 2 = ... + __syncthreads.
-template <int S, bool PACKED, int CS4, bool FUSED, int SYNC>
+// classes; (ly, lx0, rsx): lambda_y of the row and lambda_x(j) = lx0 + j * rsx.  The lane's cp.async copies of the taps
+// are waited for here, after the label loads have been issued.
+template <int S, bool PACKED, int CS4>
 __device__ __forceinline__ void k3_strip_rows(const K3SParams& P, const float4* st4, int n, int ky, int kx, int i,
                                               bool group_in, float ly, float lx0, float rsx) {
     constexpr int CH = 8;                                   // classes per chunk
@@ -480,59 +477,14 @@ __device__ __forceinline__ void k3_strip_rows(const K3SParams& P, const float4* 
                            ? __ldg((const long long*)P.labels + ((size_t)n * P.lh + y / ryl) * P.lw + x / rxl) : -1;
         }
     }
-    if constexpr (SYNC >= 1) asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory");
-    if constexpr (SYNC == 1) __syncwarp();
-    if constexpr (SYNC == 2) __syncthreads();
+    asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;" ::: "memory");
+    __syncwarp();
 
-    if constexpr (FUSED && PACKED) {
-        // -onehot term of dL/dlogits for this row: exact integer tap weights (lambda * 2S), run-length aggregated along
-        // the row (the job of k2_labels_prepass_kernel when K2 and K3 run as separate kernels)
-        if (P.onehot_grad != nullptr && row_in) {
-            constexpr float WSC = 1.f / (float)(4 * S * S);
-            const int lyi = 2 * i + 1;
-            const int Ya = clampi(ky, 0, P.h - 1), Yb = clampi(ky + 1, 0, P.h - 1);
-            const int Xa = clampi(kx, 0, P.w - 1), Xb = clampi(kx + 1, 0, P.w - 1);
-            const size_t plane = (size_t)P.h * P.w;
-            float* gbase = P.onehot_grad + (size_t)n * C * plane;
-            const size_t oA = (size_t)Ya * P.w + Xa, oB = (size_t)Ya * P.w + Xb, oC = (size_t)Yb * P.w + Xa, oD = (size_t)Yb * P.w + Xb;
-            int cur = -1, sw0 = 0, sw1 = 0;
-            auto flush = [&]() {
-                if (cur < 0) return;
-                float* gp = gbase + (size_t)cur * plane;
-                atomicAdd(gp + oA, -(float)((2 * S - lyi) * sw0) * WSC); atomicAdd(gp + oB, -(float)((2 * S - lyi) * sw1) * WSC);
-                atomicAdd(gp + oC, -(float)(lyi * sw0) * WSC);           atomicAdd(gp + oD, -(float)(lyi * sw1) * WSC);
-            };
-#pragma unroll
-            for (int j = 0; j < S; ++j) {
-                const int lab = (int)((lw16[j >> 1] >> (16 * (j & 1))) & 0xffffu);
-                if (lab < C) {                                              // counted: class id without the ignore flag
-                    if (lab != cur) { flush(); cur = lab; sw0 = 0; sw1 = 0; }
-                    sw0 += 2 * S - (2 * j + 1);
-                    sw1 += 2 * j + 1;
-                }
-            }
-            flush();
-        }
-    }
     // ---- non-finite taps? ------------------------------------------------------------------------------------
     bool exotic = false;
     for (int c = i; c < C; c += S) {
         const float4 q = st4[c * CS4];
         exotic |= !(fabsf(q.x) < INFINITY) | !(fabsf(q.y) < INFINITY) | !(fabsf(q.z) < INFINITY) | !(fabsf(q.w) < INFINITY);
-    }
-    if constexpr (FUSED) {
-        // clamped staging hides ATen's second tap of the top / left border groups (row / column 1, weight 0):
-        // look at it on the global map (0 * inf = NaN poisons those pixels in the reference)
-        if (group_in && (ky < 0 || kx < 0)) {
-            const int ya = ky < 0 ? 0 : ky, xa = kx < 0 ? 0 : kx;
-            const int yb = min(ya + 1, P.h - 1), xb = min(xa + 1, P.w - 1);
-            const float* base = P.low + (size_t)n * C * P.h * P.w;
-            for (int c = i; c < C; c += S) {
-                const float* pc = base + (size_t)c * P.h * P.w;
-                const float t1 = __ldg(pc + ya * P.w + xb), t2 = __ldg(pc + yb * P.w + xa), t3 = __ldg(pc + yb * P.w + xb);
-                exotic |= !(fabsf(t1) < INFINITY) | !(fabsf(t2) < INFINITY) | !(fabsf(t3) < INFINITY);
-            }
-        }
     }
     exotic = __any_sync(0xffffffffu, exotic);
 
@@ -592,26 +544,11 @@ __device__ __forceinline__ void k3_strip_rows(const K3SParams& P, const float4* 
         for (int j = 0; j < S; ++j) {
             ArgmaxState a;
             am_init(a);
-            if constexpr (FUSED) {
-                // ATen's taps on the global map: index0 = max(k,0), index1 = min(index0+1, size-1), lambda = 0 at k = -1
-                const int ya = ky < 0 ? 0 : ky, xa = kx < 0 ? 0 : kx;
-                const int yb = min(ya + 1, P.h - 1), xb = min(xa + 1, P.w - 1);
-                const float tyy = ky < 0 ? 0.f : ly, tx = kx < 0 ? 0.f : lx0 + (float)j * rsx;
-                const float* base = P.low + (size_t)n * C * P.h * P.w;
-                for (int c = 0; c < C && group_in; ++c) {
-                    const float* pc = base + (size_t)c * P.h * P.w;
-                    const float qx = __ldg(pc + ya * P.w + xa), qy = __ldg(pc + ya * P.w + xb);
-                    const float qz = __ldg(pc + yb * P.w + xa), qw = __ldg(pc + yb * P.w + xb);
-                    const float r0 = fmaf(qy, tx, qx * (1.f - tx)), r1 = fmaf(qw, tx, qz * (1.f - tx));
-                    am_update(a, fmaf(r1, tyy, r0 * (1.f - tyy)), c);
-                }
-            } else {
-                const float tx = lx0 + (float)j * rsx;
-                for (int c = 0; c < C; ++c) {
-                    const float4 q = st4[c * CS4];
-                    const float r0 = fmaf(q.y, tx, q.x * (1.f - tx)), r1 = fmaf(q.w, tx, q.z * (1.f - tx));
-                    am_update(a, fmaf(r1, ly, r0 * (1.f - ly)), c);
-                }
+            const float tx = lx0 + (float)j * rsx;
+            for (int c = 0; c < C; ++c) {
+                const float4 q = st4[c * CS4];
+                const float r0 = fmaf(q.y, tx, q.x * (1.f - tx)), r1 = fmaf(q.w, tx, q.z * (1.f - tx));
+                am_update(a, fmaf(r1, ly, r0 * (1.f - ly)), c);
             }
 #pragma unroll
             for (int jj = 0; jj < S; ++jj)
@@ -688,83 +625,7 @@ k3_strip_kernel(const K3SParams P) {
     const int ky = rem / (P.w + 1) - 1, kx = rem % (P.w + 1) - 1;
     const float ly = ky < 0 ? 0.f : ((float)i + 0.5f) * RS;
     const float lx0 = kx < 0 ? 0.f : LX0, rsx = kx < 0 ? 0.f : RS;      // lambda_x(j) = lx0 + j * rsx
-    k3_strip_rows<S, PACKED, GPW, false, 1>(P, reinterpret_cast<const float4*>(st) + gl, n, ky, kx, i, group_in, ly, lx0, rsx);
-}
-
-// ---------------------------------------------------------------------------------------------
-// k23_fused: K2 (split form) and K3 of the x16 geometry in ONE kernel, warp-specialised.
-// K2 is bound by the FP32 (FMA) pipe, K3 by the ALU pipe / issue slots, and the phases of equal warps coincide
-// (every warp runs the same program on the same amount of work), so neither kernel overlaps its own idle phases;
-// launched on two streams the block scheduler does not co-schedule them either.  Here a CTA of 8 warps stages the
-// taps of 16 groups ONCE; warps 4-7 ("CE warps") run k2_strip_warp on one 2x2 tile each and write their tap
-// gradients to a second shared tile (not in place: the other warps are still reading the taps), warps 0-3 ("argmax
-// warps") run k3_strip_rows over the same 16 groups in two rounds of 8 groups (one row per lane).  Three CTAs per SM:
-// 12 CE + 12 argmax warps share each SM's schedulers.  (The CE warps are the long pole; the warp arbiter favours the
-// higher warp ids.)
-#ifndef K23_UNR
-#define K23_UNR 2
-#endif
-template <int S>
-__global__ void __launch_bounds__(256, 3)
-k23_fused_kernel(const K2SParams P2, const K3SParams P3) {
-    static_assert(S == 16, "fused kernel: x16 geometry");
-    constexpr int NG = 16, CSF = NG * 4, CH = 8;            // groups per CTA, floats per class, K3's class chunk
-    constexpr float RS = 1.f / S, LX0 = 0.5f / S;
-    extern __shared__ float smem[];
-    const int C = P2.C;
-    float* taps = smem;                                     // [C + CH][16 groups][4 taps]
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int tiles_per_img = P2.nty * P2.ntx;
-    const long long ntiles = (long long)P2.B * tiles_per_img;
-    const size_t plane = (size_t)P2.h * P2.w;
-    // warp tile w (0..3) of this CTA -> (image, tile row, tile column)
-    auto tile_of = [&](int w, int& n, int& GY0, int& GX0) -> bool {
-        const long long wt = (long long)blockIdx.x * 4 + w;
-        if (wt >= ntiles) { n = 0; GY0 = 0; GX0 = 0; return false; }
-        n = (int)(wt / tiles_per_img);
-        const int trem = (int)(wt - (long long)n * tiles_per_img);
-        const int tyi = trem / P2.ntx;
-        GY0 = tyi * 2; GX0 = (trem - tyi * P2.ntx) * 2;
-        return true;
-    };
-    // ---- stage (whole CTA): thread -> fixed (group, tap), 4 classes per sweep; index-clamped taps --------------
-    {
-        const int r = threadIdx.x % CSF, gq = r >> 2, tap = r & 3;
-        int n, GY0, GX0;
-        const bool act = tile_of(gq >> 2, n, GY0, GX0);
-        const int ky = GY0 + ((gq & 3) >> 1) - 1, kx = GX0 + (gq & 1) - 1;
-        const bool ok = act && ky < P2.h && kx < P2.w;
-        const int yy = clampi2(ky + (tap >> 1), 0, P2.h - 1), xx = clampi2(kx + (tap & 1), 0, P2.w - 1);
-        const float* src = P2.low + (size_t)n * C * plane + (size_t)yy * P2.w + xx;
-        float* dst = taps + r;
-        for (int c = threadIdx.x / CSF; c < C; c += 256 / CSF) {
-            if (ok) cp_async4(dst + c * CSF, src + (size_t)c * plane);
-            else dst[c * CSF] = 0.f;
-        }
-        for (int c = C + threadIdx.x / CSF; c < C + CH; c += 256 / CSF) dst[c * CSF] = -3.0e38f;   // never wins
-    }
-    if (warp >= 4) {
-        const int cw = warp - 4;
-        int n, GY0, GX0;
-        const bool act = tile_of(cw, n, GY0, GX0);
-        k2_strip_warp<S, true, CSF, true, K23_UNR>(P2, taps + cw * 16, act, n, GY0, GX0, lane);
-    } else {
-        const int aw = warp;
-#pragma unroll 1
-        for (int round = 0; round < 2; ++round) {
-            const int g = round * 8 + aw * 2 + lane / S, i = lane % S;     // group 0..15 of the CTA, row of the group
-            int n, GY0, GX0;
-            const bool act = tile_of(g >> 2, n, GY0, GX0);
-            const int ky = GY0 + ((g & 3) >> 1) - 1, kx = GX0 + (g & 1) - 1;
-            const bool group_in = act && ky < P2.h && kx < P2.w;
-            const float ly = ((float)i + 0.5f) * RS;
-            const float4* st4 = reinterpret_cast<const float4*>(taps) + g;
-            if (round == 0)
-                k3_strip_rows<S, true, CSF / 4, true, 2>(P3, st4, n, ky, kx, i, group_in, ly, LX0, RS);
-            else
-                k3_strip_rows<S, true, CSF / 4, true, 0>(P3, st4, n, ky, kx, i, group_in, ly, LX0, RS);
-        }
-    }
+    k3_strip_rows<S, PACKED, GPW>(P, reinterpret_cast<const float4*>(st) + gl, n, ky, kx, i, group_in, ly, lx0, rsx);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -878,7 +739,7 @@ static int launch_k3_strip(const float* d_low, int N, int C, int h, int w, int H
     K3SParams P;
     P.low = d_low; P.labels = labels; P.confmat = (unsigned long long*)d_confmat;
     P.per_image = (unsigned long long*)d_per_image; P.pred_out = (long long*)d_pred;
-    P.N = N; P.C = C; P.h = h; P.w = w; P.H = H; P.W = W; P.lh = lh; P.lw = lw; P.onehot_grad = nullptr;
+    P.N = N; P.C = C; P.h = h; P.w = w; P.H = H; P.W = W; P.lh = lh; P.lw = lw;
     const long long ngroups = (long long)N * (h + 1) * (w + 1);
     const long long warps = (ngroups + (32 / s) - 1) / (32 / s);
     const unsigned grid = (unsigned)((warps + wpc - 1) / wpc);
@@ -927,27 +788,8 @@ extern "C" int lc2is_ce_argmax_fused_packed(const float* d_low, const uint16_t* 
     if ((uintptr_t)d_labels_packed % 16) return fail(LC2IS_ERR_ARG, "packed labels must be 16-byte aligned%s");
     if (!lc2is_ce_argmax_fused_supported(C, h, w, H, W))
         return fail(LC2IS_ERR_UNSUPPORTED, "fused K2+K3 needs scale 16 and a class count whose job tiles fit one SM%s");
-    if (!getenv("LC2IS_FUSED_V1") || (size_t)(C + 8) * 64 * sizeof(float) > 72 * 1024)
-        return launch_k23_rc(d_low, d_labels_packed, B, C, h, w, H, W, d_loss_sum, d_grad_low, onehot, d_n_valid,
-                             d_confmat, d_per_image, d_pred, (cudaStream_t)stream);
-    K2SParams P2;
-    P2.low = d_low; P2.labels = nullptr; P2.labels16 = d_labels_packed; P2.grad_low = d_grad_low;
-    P2.n_valid = (unsigned long long*)d_n_valid;
-    P2.loss_sum = d_loss_sum; P2.grad_scale = nullptr; P2.ignore_index = 0;
-    P2.B = B; P2.C = C; P2.h = h; P2.w = w; P2.H = H; P2.W = W;
-    P2.nty = (h + 1 + 1) / 2; P2.ntx = (w + 1 + 1) / 2;
-    K3SParams P3;
-    P3.low = d_low; P3.labels = d_labels_packed; P3.confmat = (unsigned long long*)d_confmat;
-    P3.per_image = (unsigned long long*)d_per_image; P3.pred_out = (long long*)d_pred;
-    P3.N = B; P3.C = C; P3.h = h; P3.w = w; P3.H = H; P3.W = W; P3.lh = H; P3.lw = W;
-    P3.onehot_grad = onehot ? d_grad_low : nullptr;
-    const size_t smem = (size_t)(C + 8) * 64 * sizeof(float);
-    const long long tiles = (long long)B * P2.nty * P2.ntx;
-    const unsigned grid = (unsigned)((tiles + 3) / 4);
-    if (int e = set_smem(k23_fused_kernel<16>, smem)) return e;
-    k23_fused_kernel<16><<<grid, 256, smem, (cudaStream_t)stream>>>(P2, P3);
-    LC2IS_CHECK_LAUNCH("k23_fused_kernel");
-    return 0;
+    return launch_k23_rc(d_low, d_labels_packed, B, C, h, w, H, W, d_loss_sum, d_grad_low, onehot, d_n_valid,
+                         d_confmat, d_per_image, d_pred, (cudaStream_t)stream);
 }
 
 extern "C" int lc2is_argmax_confmat_lowres_packed(const float* d_low, int N, int C, int h, int w, int H, int W,

@@ -10,7 +10,6 @@ Used by bench.py and usable as the data-parallel engine shim (SURVEY 8f-4).
 """
 from __future__ import annotations
 
-import os
 from typing import Optional
 
 import torch
@@ -110,9 +109,9 @@ class HeadStep:
         self._pending = None           # block whose bucket has not been all-reduced yet (distributed only)
         # the exchange steps go through ncclAllReduce on a stream of their own, forked / joined with events: plain
         # stream-ordered launches that overlap the head kernels and can be captured into the step's CUDA graph
-        # (LC2IS_DP_TORCH_NCCL=1: torch.distributed's process group instead - not capturable on this stack)
+        # (a process group that is not NCCL: torch.distributed's collectives instead - not capturable on this stack)
         self.comm = None
-        if self.distributed and os.environ.get("LC2IS_DP_TORCH_NCCL") != "1":
+        if self.distributed:
             from . import nccl
             self.comm = nccl.default_comm(dev)
         self._xs = torch.cuda.Stream(device=dev) if self.comm is not None else None

@@ -196,7 +196,7 @@ def test_strip_kernel_non_finite_taps_and_ties():
 @pytest.mark.parametrize("N,C,h,ign,frac", [(3, 151, 6, 0, 0.1), (2, 150, 32, 0, 0.1), (1, 19, 3, 5, 0.3), (5, 37, 5, 0, 0.0),
                                                (3, 151, 8, 0, 0.1), (1, 19, 4, 5, 0.3), (2, 40, 12, 0, 0.2), (1, 200, 4, 0, 0.1)])
 def test_fused_ce_argmax_kernel_matches_separate_kernels_and_oracle(N, C, h, ign, frac):
-    """k23_fused_kernel (x16): the warp-specialised K2+K3 kernel gives the loss / gradient of the split K2 path and
+    """k23_rc_kernel (x16): the fused K2+K3 kernel gives the loss / gradient of the split K2 path and
     the bit-exact confusion matrix / per-image counts / masks of K3 (dyadic logits)."""
     s = 16
     H = s * h

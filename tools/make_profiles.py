@@ -46,7 +46,7 @@ def opmix(d, h2):
         st[s_[6:]] = sum(int(r[ix[s_]]) for r in d)
     t = sum(st.values()) or 1
     return "\n".join(lines + ["", "warp-state samples: " + ", ".join(f"{k} {v / t * 100:.1f}%" for k, v in sorted(st.items(), key=lambda kv: -kv[1])[:8])])
-names = {"k23_rc": "k23rc", "k1_logits": "k1", "k1b_dv": "k1bdv", "k1b_dt_kernel": "k1bdt", "k23_fused": "k23fused", "k2_strip": "k2", "k3_strip": "k3strip", "prepass": "prepass", "prep_f32": "k1bprep", "pack_labels": "packlabels"}
+names = {"k23_rc": "k23rc", "k1_logits": "k1", "k1b_dv": "k1bdv", "k1b_dt_kernel": "k1bdt", "k2_strip": "k2", "k3_strip": "k3strip", "prepass": "prepass", "prep_f32": "k1bprep", "pack_labels": "packlabels"}
 for blk in summ.split("-" * 60):
     m = re.search(r"Kernel Name = (.*)", blk)
     if not m: continue
@@ -61,7 +61,6 @@ except Exception: tj = {}
 tj["note"] = "dram__bytes_read.sum + dram__bytes_write.sum per launch, ncu --set full, cfg2 G-A B=16 C=150 (profiles/*_ncu_full.txt)"
 for k, v in traffic.items():
     if "k23_rc" in k: tj["k23_rc_kernel<16>"] = v
-    elif "k23_fused" in k: tj["k23_fused_kernel<16>"] = v
     elif "pack_labels" in k: tj["k2_pack_labels_kernel"] = v
     elif "prep_f32" in k: tj["k1b_prep_f32_kernel"] = v
 json.dump(tj, open("profiles/traffic.json", "w"), indent=1)
