@@ -1,10 +1,12 @@
 """Per-warp timeline of k23_rc_kernel from an instrumented build (csrc built with -DRC_STAMPS; development aid).
-build:  nvcc ... -DRC_STAMPS -c k23_rowclass.cu && relink;  usage: python tools/k23_timeline.py [B]"""
+build:  nvcc ... -DRC_STAMPS -c k23_rowclass.cu && relink;  usage: python tools/k23_timeline.py [B]
+Per warp RC_STAMP_SLOTS = 32 stamps: [0] start, then (class phase starts, job ends) per job, [31] = stamps taken."""
 import ctypes, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from lc2is_b200 import synthetic, _lib
 from lc2is_b200.step import HeadStep
+SLOTS = 32
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 16
 h, H, C, D = 32, 512, 150, 512
 V = synthetic.make_patch_embeddings(B, h * h, D).cuda(); L = synthetic.make_labels(B, H, H, C, ignore_frac=0.1).cuda()
@@ -12,10 +14,10 @@ t = synthetic.make_prototypes(C, D).cuda()
 hs = HeadStep(B, h, h, H, H, C, ignore_index=0)
 for _ in range(5): hs(V, t, L)
 torch.cuda.synchronize()
-buf = np.zeros(148 * 16 * 16, dtype=np.uint64)
+buf = np.zeros(148 * 16 * SLOTS, dtype=np.uint64)
 rc = _lib.lib.lc2is_debug_stamps(buf.ctypes.data_as(ctypes.c_void_p)); assert rc == 0, rc
-S = buf.reshape(148 * 16, 16).astype(np.int64)
-n = S[:, 15]; ok = n >= 3
+S = buf.reshape(148 * 16, SLOTS).astype(np.int64)
+n = S[:, SLOTS - 1]; ok = n >= 3
 t0 = S[ok, 0].min()
 start = S[ok, 0] - t0
 ends = np.array([S[i, n[i] - 1] - t0 for i in np.nonzero(ok)[0]])
