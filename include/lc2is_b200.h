@@ -189,6 +189,29 @@ int lc2is_upsample_ce_fwd_bwd(const float* d_low, const int64_t* d_labels,
                               double* d_loss_sum, float* d_grad_low, void* d_grad_low_bf16,
                               lc2is_stream_t stream);
 
+/* ---------------------------------------------------------------------------------------
+ * K2, weighted form: the same fused pass for a criterion configured with class weights and / or label smoothing,
+ *       nn.CrossEntropyLoss(weight=w, ignore_index=ii, label_smoothing=eps) applied to
+ *       F.interpolate(input, mode="bilinear", size=(H, W))     (engine.py:94 on final.py:44; loss.py:19-20).
+ * lc2is_ce_weight_sum: *d_wsum += sum over counted labels (in [0,C) and != ignore_index) of w[label], in double
+ *            (d_weight = NULL counts them): the 'mean' denominator of the weighted cross-entropy.  ACCUMULATED.
+ * lc2is_upsample_ce_fwd_bwd_ex: lc2is_upsample_ce_fwd_bwd with
+ *   d_weight         [C] fp32 class weights on the device, or NULL (all 1); the host never reads them.
+ *   label_smoothing  eps in [0, 1] (else LC2IS_ERR_ARG).
+ *   With W = sum_c w_c and a = (1-eps) w_t + (eps/C) W, a counted pixel adds
+ *       a * logsumexp_c x_c - (1-eps) w_t x_t - (eps/C) sum_c w_c x_c          to *d_loss_sum, and
+ *       g * (a * softmax_c - (1-eps) w_t [c == t] - (eps/C) w_c)              to dL/dx_c,
+ *   scattered through the bilinear taps.  reduction='mean' is d_grad_scale = 1 / wsum and loss = loss_sum / wsum
+ *   (wsum from lc2is_ce_weight_sum).  d_weight == NULL with eps == 0 runs exactly lc2is_upsample_ce_fwd_bwd.
+ */
+int lc2is_ce_weight_sum(const int64_t* d_labels, int64_t n, int C, int64_t ignore_index,
+                        const float* d_weight, double* d_wsum, lc2is_stream_t stream);
+int lc2is_upsample_ce_fwd_bwd_ex(const float* d_low, const int64_t* d_labels,
+                                 int B, int C, int h, int w, int H, int W,
+                                 int64_t ignore_index, const float* d_weight, float label_smoothing,
+                                 const float* d_grad_scale, double* d_loss_sum, float* d_grad_low,
+                                 void* d_grad_low_bf16, lc2is_stream_t stream);
+
 /* Split form of K2 for power-of-two scales 8 / 16 (what the whole-step entries run): the same
  * reference lines (model/loss.py:19-20 + autograd), cut so that everything that depends on the
  * labels only happens once, in one pass over the int64 map.

@@ -60,6 +60,9 @@ SIGNATURES = {
     "lc2is_mean_scale_finalize": (c_int, [_p, c_float, _p, _p, _p, _p]),
     "lc2is_upsample_ce_fwd_bwd": (c_int, [_p, _p, c_int, c_int, c_int, c_int, c_int, c_int, c_int64, _p, _p,
                                           _p, _p, _p]),
+    "lc2is_ce_weight_sum": (c_int, [_p, c_int64, c_int, c_int64, _p, _p, _p]),
+    "lc2is_upsample_ce_fwd_bwd_ex": (c_int, [_p, _p, c_int, c_int, c_int, c_int, c_int, c_int, c_int64, _p, c_float,
+                                             _p, _p, _p, _p, _p]),
     "lc2is_ce_split_supported": (c_int, [c_int, c_int, c_int, c_int]),
     "lc2is_ce_labels_prepass": (c_int, [_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int64, _p, _p, _p, _p]),
     "lc2is_upsample_ce_packed": (c_int, [_p, _p, c_int, c_int, c_int, c_int, c_int, c_int, _p, _p, _p]),

@@ -105,6 +105,19 @@ struct K2SParams {
     int nty, ntx;                 // warp tiles per image
     unsigned long long* n_valid;  // SPLIT: += number of counted pixels (null = the caller counted them already)
 };
+// The weighted form's parameters (a separate type: K2SParams is copied to the stack for k2_strip_slow, and the unweighted
+// kernels keep their frame): class weights w[C] (null = all 1), 1 - eps and eps / C of the label smoothing eps.
+struct K2SParamsW : K2SParams {
+    const float* weight;
+    float one_m_eps, eps_c;
+};
+template <bool WT>
+using K2SP = typename std::conditional<WT, K2SParamsW, K2SParams>::type;
+
+// Weighted / label-smoothed cross-entropy (nn.CrossEntropyLoss(weight=w, label_smoothing=eps)); with W = sum_c w_c and
+// a = (1-eps) w_t + (eps/C) W, a counted pixel adds  a*lse - (1-eps) w_t x_t - (eps/C) sum_c w_c x_c  to the loss and
+//   g * (a * softmax_c - (1-eps) w_t [c == t] - (eps/C) w_c)  to d/dx_c.
+__device__ __forceinline__ float k2_class_weight(const float* w, int c) { return w ? __ldg(w + c) : 1.f; }
 
 // Where a group's four taps (a b / c d) of class c come from.  TapsSmem: the staged tile, one LDS.128.  TapsGlobal: the
 // class-plane-major map itself (L1 / L2) - for class counts whose staged tile would leave a handful of warps per SM
@@ -125,9 +138,9 @@ struct TapsGlobal {
     }
 };
 
-template <int S, bool SPLIT, class TQ>
+template <int S, bool SPLIT, class TQ, bool WT = false>
 __device__ __noinline__ float k2_strip_slow(const TQ tq, unsigned vm, int n, int y0, int x0,
-                                            int u, const K2SParams& P, float gs, float* gA, float* gB,
+                                            int u, const K2SP<WT>& P, float gs, float* gA, float* gB,
                                             float* gC, float* gD) {
     const int C = P.C;
     const size_t plane = (size_t)P.h * P.w;
@@ -145,21 +158,35 @@ __device__ __noinline__ float k2_strip_slow(const TQ tq, unsigned vm, int n, int
                 m = fmaxf(m, fmaf(lx, R - L, L));
             }
             float sum = 0.f, lt = 0.f;
+            float wl = 0.f, wsum = 0.f;                     // WT: sum_c w_c x_c, sum_c w_c
             for (int c = 0; c < C; ++c) {
                 const float4 q = tq.get(c);
                 const float L = fmaf(ly, q.z - q.x, q.x), R = fmaf(ly, q.w - q.y, q.y);
                 const float l = fmaf(lx, R - L, L);
                 sum += ex2f((l - m) * LOG2E);
                 if (c == t) lt = l;
+                if constexpr (WT) {
+                    const float wc = k2_class_weight(P.weight, c);
+                    wl = fmaf(wc, l, wl);
+                    wsum += wc;
+                }
             }
-            loss += logf(sum) + m - lt;
+            float a = 1.f, wt = 1.f;
+            if constexpr (WT) {
+                wt = P.one_m_eps * k2_class_weight(P.weight, t);
+                a = fmaf(P.eps_c, wsum, wt);
+                loss += a * (logf(sum) + m) - wt * lt - P.eps_c * wl;
+            } else {
+                loss += logf(sum) + m - lt;
+            }
             if (gA) {
-                const float uu = gs / sum;
+                const float uu = WT ? gs * a / sum : gs / sum;
                 const float wa = (1.f - ly) * (1.f - lx), wb = (1.f - ly) * lx, wc = ly * (1.f - lx), wd = ly * lx;
                 for (int c = 0; c < C; ++c) {
                     const float4 q = tq.get(c);
                     const float L = fmaf(ly, q.z - q.x, q.x), R = fmaf(ly, q.w - q.y, q.y);
-                    const float gg = ex2f((fmaf(lx, R - L, L) - m) * LOG2E) * uu - (c == t ? gs : 0.f);
+                    float gg = ex2f((fmaf(lx, R - L, L) - m) * LOG2E) * uu - (c == t ? (WT ? gs * wt : gs) : 0.f);
+                    if constexpr (WT) gg -= gs * P.eps_c * k2_class_weight(P.weight, c);
                     atomicAdd(gA + (size_t)c * plane, gg * wa); atomicAdd(gB + (size_t)c * plane, gg * wb);
                     atomicAdd(gC + (size_t)c * plane, gg * wc); atomicAdd(gD + (size_t)c * plane, gg * wd);
                 }
@@ -169,9 +196,14 @@ __device__ __noinline__ float k2_strip_slow(const TQ tq, unsigned vm, int n, int
 }
 
 // CSF = floats per class of the warp's tile of quads; st = the warp's first tap quad of class 0.
-template <int S, bool SPLIT, int CSF, bool GTAPS = false>
-__device__ __forceinline__ void k2_strip_warp(const K2SParams& P, float* st, bool active, int n, int GY0,
+// WT: the weighted / label-smoothed form (one-call path only).  Besides a*lse and the (1-eps) w_t scale of the -onehot
+// runs, the smoothing terms are linear in the logits: the loss takes (eps/C) V.Q per thread, with Q = sum_c w_c * taps
+// (accumulated in the max-tap sweep) and V = the thread's summed bilinear tap weights of its counted pixels; the
+// gradient takes -g (eps/C) w_c V_cell on the lane that issues the cell's reduction (V merged like the gradients).
+template <int S, bool SPLIT, int CSF, bool GTAPS = false, bool WT = false>
+__device__ __forceinline__ void k2_strip_warp(const K2SP<WT>& P, float* st, bool active, int n, int GY0,
                                               int GX0, int lane) {
+    static_assert(!(WT && SPLIT), "the weighted form is one-call only");
     constexpr int TPG = S / 2;                              // threads (lanes) per group
     constexpr int GPW = 32 / TPG;                           // groups per warp: 4 (S=16) / 8 (S=8)
     constexpr int WGX = GPW / 2;                            // warp tile = 2 x WGX groups
@@ -265,15 +297,28 @@ __device__ __forceinline__ void k2_strip_warp(const K2SParams& P, float* st, boo
 
     // ---- softmax shift: M = max over classes of the group's taps --------------------------------------------
     float mx = -INFINITY, mn = INFINITY;
+    float4 wq = make_float4(0.f, 0.f, 0.f, 0.f);            // WT: sum_c w_c * taps
+    float wsum = 0.f;                                       // WT: W = sum_c w_c
     for (int c = u; c < C; c += TPG) {
         const float4 q = tq.get(c);
         mx = fmaxf(mx, fmaxf(fmaxf(q.x, q.y), fmaxf(q.z, q.w)));
         mn = fminf(mn, fminf(fminf(q.x, q.y), fminf(q.z, q.w)));
+        if constexpr (WT) {
+            const float wc = k2_class_weight(P.weight, c);
+            wq.x = fmaf(wc, q.x, wq.x); wq.y = fmaf(wc, q.y, wq.y);
+            wq.z = fmaf(wc, q.z, wq.z); wq.w = fmaf(wc, q.w, wq.w);
+            wsum += wc;
+        }
     }
 #pragma unroll
     for (int o = TPG / 2; o > 0; o >>= 1) {
         mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
         mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+        if constexpr (WT) {
+            wq.x += __shfl_xor_sync(0xffffffffu, wq.x, o); wq.y += __shfl_xor_sync(0xffffffffu, wq.y, o);
+            wq.z += __shfl_xor_sync(0xffffffffu, wq.z, o); wq.w += __shfl_xor_sync(0xffffffffu, wq.w, o);
+            wsum += __shfl_xor_sync(0xffffffffu, wsum, o);
+        }
     }
     const float M = mx;
     const unsigned bal = __ballot_sync(0xffffffffu, vm != 0);
@@ -339,7 +384,66 @@ __device__ __forceinline__ void k2_strip_warp(const K2SParams& P, float* st, boo
         }
         // ---- loss: log-sum-exp part, and U = g / S --------------------------------------------------------------
         // (lg2.approx / rcp.approx: 2^-22 relative; S is in [exp(-K2_FAST_RANGE), C], never denormal)
-        {
+        int va4[4] = {0, 0, 0, 0};                          // WT: V of the four taps, in units of 1 / (4 S^2)
+        if constexpr (WT) {
+            // per counted pixel: a*(M + ln S), U = g*a / S, the target logit and the -(1-eps) w_t onehot runs
+#pragma unroll
+            for (int j = 0; j < S; ++j) {
+                if (!((vm >> j) & 1u)) U2[j].x = 0.f;
+                if (!((vm >> (16 + j)) & 1u)) U2[j].y = 0.f;
+            }
+            if (vm) {
+                const float wscale = -gs / (float)(4 * S * S);
+#pragma unroll
+                for (int r = 0; r < 2; ++r) {
+                    if (!((vm >> (r * 16)) & 0xffffu)) continue;
+                    const long long* row = P.labels + ((size_t)n * P.H + (y0 + r)) * P.W + x0;
+                    const float lyr = r ? ly2.y : ly2.x;
+                    const int lyi = 2 * (2 * u + r) + 1;    // lambda_y * 2S
+                    int cur = -1, sw0 = 0, sw1 = 0, tw0 = 0, tw1 = 0;
+                    float wcur = 0.f;
+                    auto flush = [&]() {
+                        if (cur >= 0 && gb) {
+                            const float ws = wscale * wcur;
+                            atomicAdd(gA + (size_t)cur * plane, ws * (float)((2 * S - lyi) * sw0));
+                            atomicAdd(gB + (size_t)cur * plane, ws * (float)((2 * S - lyi) * sw1));
+                            atomicAdd(gC + (size_t)cur * plane, ws * (float)(lyi * sw0));
+                            atomicAdd(gD + (size_t)cur * plane, ws * (float)(lyi * sw1));
+                        }
+                    };
+#pragma unroll
+                    for (int jj = 0; jj < S / 2; ++jj) {
+                        if (!((vm >> (r * 16 + 2 * jj)) & 3u)) continue;
+                        const longlong2 t2 = __ldg(reinterpret_cast<const longlong2*>(row + 2 * jj));
+#pragma unroll
+                        for (int e = 0; e < 2; ++e) {
+                            const int j = 2 * jj + e;
+                            if (!((vm >> (r * 16 + j)) & 1u)) continue;
+                            const int t = (int)(e ? t2.y : t2.x);
+                            const float wt = P.one_m_eps * k2_class_weight(P.weight, t);
+                            const float a = fmaf(P.eps_c, wsum, wt);
+                            float& sv = r ? U2[j].y : U2[j].x;
+                            loss = fmaf(a, fmaf(lg2f(sv), LN2, M), loss);
+                            sv = gs * a * rcpf(sv);
+                            const float4 q = tq.get(t);
+                            const float L = fmaf(lyr, q.z - q.x, q.x), R = fmaf(lyr, q.w - q.y, q.y);
+                            loss = fmaf(-wt, fmaf(((float)j + 0.5f) * RS, R - L, L), loss);
+                            if (t != cur) { flush(); cur = t; wcur = wt; sw0 = 0; sw1 = 0; }
+                            sw0 += 2 * S - (2 * j + 1);
+                            sw1 += 2 * j + 1;
+                            tw0 += 2 * S - (2 * j + 1);
+                            tw1 += 2 * j + 1;
+                        }
+                    }
+                    flush();
+                    va4[0] += (2 * S - lyi) * tw0; va4[1] += (2 * S - lyi) * tw1;
+                    va4[2] += lyi * tw0;           va4[3] += lyi * tw1;
+                }
+                // smoothing: -(eps/C) sum over the counted pixels of the interpolated sum_c w_c x_c
+                const float vq = (float)va4[0] * wq.x + (float)va4[1] * wq.y + (float)va4[2] * wq.z + (float)va4[3] * wq.w;
+                loss = fmaf(-P.eps_c * (1.f / (float)(4 * S * S)), vq, loss);
+            }
+        } else {
             float lg = 0.f;
 #pragma unroll
             for (int j = 0; j < S; ++j) {
@@ -351,7 +455,7 @@ __device__ __forceinline__ void k2_strip_warp(const K2SParams& P, float* st, boo
             loss += fmaf((float)__popc(vm), M, lg * LN2);
         }
         // ---- target logits and the -g*onehot term (exact integer tap weights, run-length per row) ---------------
-        if (!SPLIT && vm) {
+        if (!SPLIT && !WT && vm) {
             const float wscale = -gs / (float)(4 * S * S);
 #pragma unroll
             for (int r = 0; r < 2; ++r) {
@@ -410,6 +514,16 @@ __device__ __forceinline__ void k2_strip_warp(const K2SParams& P, float* st, boo
             float* dst = (holder && uy <= P.h && ux <= P.w)
                              ? gb + (size_t)clampi2(uy, 0, P.h - 1) * P.w + clampi2(ux, 0, P.w - 1) : nullptr;
             const float2 omy = make_float2(1.f - ly2.x, 1.f - ly2.y);
+            float kv = 0.f;                                  // WT: -g (eps/C) V of this lane's source cell
+            if constexpr (WT) {
+                float V0 = (float)va4[0], V1 = (float)va4[1], V2 = (float)va4[2], V3 = (float)va4[3];
+                group_reduce4<TPG>(V0, V1, V2, V3, u);
+                const float hv = __shfl_sync(0xffffffffu, V0, h_src);
+                if (h_dst) V0 += hv;
+                const float vv = __shfl_sync(0xffffffffu, V0, v_src);
+                if (v_dst) V0 += vv;
+                kv = V0 != 0.f ? -gs * P.eps_c * (1.f / (float)(4 * S * S)) * V0 : 0.f;
+            }
             float2 eN, rN;
             row_exp(tq.get(0), eN, rN);
             float4 qn = tq.get(1);
@@ -437,11 +551,12 @@ __device__ __forceinline__ void k2_strip_warp(const K2SParams& P, float* st, boo
                 if (h_dst) A += hx;
                 const float vx = __shfl_sync(0xffffffffu, A, v_src);
                 if (v_dst) A += vx;
+                if constexpr (WT) A = fmaf(kv, k2_class_weight(P.weight, c), A);
                 if (dst) atomicAdd(dst + (size_t)c * plane, A);
             }
         }
     } else if (warp_any) {
-        loss += k2_strip_slow<S, SPLIT, TQ>(tq, vm, n, y0, x0, u, P, gs, gA, gB, gC, gD);
+        loss += k2_strip_slow<S, SPLIT, TQ, WT>(tq, vm, n, y0, x0, u, P, gs, gA, gB, gC, gD);
     }
     loss = warp_sum(loss);
     if (lane == 0 && loss != 0.f) atomicAdd(P.loss_sum, (double)loss);

@@ -56,6 +56,36 @@ __global__ void k2_count_valid_kernel(const long long* __restrict__ labels, long
     }
 }
 
+// sum of the class weights of the counted labels (the 'mean' denominator of the weighted cross-entropy); weight = null
+// counts them.  Accumulated in double.
+__global__ void k2_weight_sum_kernel(const long long* __restrict__ labels, long long n, long long C, long long ignore,
+                                     const float* __restrict__ weight, double* __restrict__ out) {
+    auto wl = [&](long long v) {
+        return (unsigned long long)v < (unsigned long long)C && v != ignore ? (double)k2_class_weight(weight, (int)v) : 0.0;
+    };
+    double acc = 0.0;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long n2 = n / 2;
+    const longlong2* l2 = reinterpret_cast<const longlong2*>(labels);
+    for (long long k = i; k < n2; k += stride) {
+        longlong2 v = __ldg(l2 + k);
+        acc += wl(v.x) + wl(v.y);
+    }
+    if (i == 0 && (n & 1)) acc += wl(labels[n - 1]);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    __shared__ double ws[32];
+    if ((threadIdx.x & 31) == 0) ws[threadIdx.x >> 5] = acc;
+    __syncthreads();
+    if (threadIdx.x < 32) {
+        double v = threadIdx.x < (blockDim.x >> 5) ? ws[threadIdx.x] : 0.0;
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+        if (threadIdx.x == 0 && v != 0.0) atomicAdd(out, v);
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
 // Geometry of the fast path.  A GROUP is the set of bps x bps 4x4-pixel blocks (bps = s/4) that
 // interpolate between the same 2x2 source cells: group (gy,gx) has taps (ky,kx) = (gy-1, gx-1)
@@ -73,6 +103,8 @@ struct K2Params {
     int s, off, q;                // scale, pixel offset of the block grid, block offset of group 0
     int tgy, tgx;                 // groups per CTA
     float rs;
+    const float* weight;          // WT: class weights [C] (null = all 1); 1 - eps, eps / C (k2_strip.cuh: k2_class_weight)
+    float one_m_eps, eps_c;
 };
 
 // exp-polynomial of one class inside a 4x4 block: exp(l(i,j) - M) = E * p^i * q^j * t^(i*j)
@@ -91,11 +123,15 @@ __device__ __forceinline__ Poly k2_poly(float a, float b, float cc, float d, flo
     return P;
 }
 
-template <int BPS>
+// WT: the weighted / label-smoothed form (k2_strip.cuh: k2_class_weight): U = g*a / S, a*lse, a (1-eps) w_t scale on the
+// -onehot runs, and the smoothing terms through V = the thread's summed tap weights (loss: V.Q with Q = sum_c w_c * taps
+// from the max-tap sweep; gradient: -g (eps/C) w_c V per tap and class).
+template <int BPS, bool WT = false>
 __global__ void __launch_bounds__(128)
 k2_fast_kernel(const K2Params P) {
     constexpr int LPG = BPS * BPS;                          // lanes (threads) per group
     constexpr bool QUAD = LPG >= 4;                         // tile layout: per-group tap quads vs cells
+    static_assert(!WT || LPG == 1, "the weighted form is instantiated for one thread per group");
     extern __shared__ float smem[];
     const int C = P.C;
     const int ngr = P.tgy * P.tgx;
@@ -197,11 +233,18 @@ k2_fast_kernel(const K2Params P) {
 
     // ---- softmax shift: M = max over classes of the group's taps (>= every pixel's max) -----------
     float mx = -INFINITY, mn = INFINITY;
+    float4 wq = make_float4(0.f, 0.f, 0.f, 0.f);            // WT: sum_c w_c * taps
+    float wsum = 0.f;                                       // WT: W = sum_c w_c
     for (int c = u; c < C; c += LPG) {                      // the group's lanes split the classes
         float a, b, cc, d;
         taps(c, a, b, cc, d);
         mx = fmaxf(mx, fmaxf(fmaxf(a, b), fmaxf(cc, d)));
         mn = fminf(mn, fminf(fminf(a, b), fminf(cc, d)));
+        if constexpr (WT) {
+            const float wc = k2_class_weight(P.weight, c);
+            wq.x = fmaf(wc, a, wq.x); wq.y = fmaf(wc, b, wq.y); wq.z = fmaf(wc, cc, wq.z); wq.w = fmaf(wc, d, wq.w);
+            wsum += wc;
+        }
     }
 #pragma unroll
     for (int o = LPG / 2; o > 0; o >>= 1) {
@@ -278,7 +321,11 @@ k2_fast_kernel(const K2Params P) {
         }
     }
     // ---- loss and per-pixel gradient scale U = g / S ----------------------------------------------------
+    const int S2 = 2 * P.s;
+    const int lyi0 = 2 * y0 + 1 - P.s - S2 * ky, lxi0 = 2 * x0 + 1 - P.s - S2 * kx;   // lambda * 2s of pixel (0,0)
+    float4 kv = make_float4(0.f, 0.f, 0.f, 0.f);            // WT: -g (eps/C) V of the four taps
     if (any) {
+        int va = 0, vb = 0, vc = 0, vd = 0;                 // WT: V in units of 1 / (2s)^2
 #pragma unroll
         for (int i = 0; i < 4; ++i)
 #pragma unroll
@@ -290,11 +337,29 @@ k2_fast_kernel(const K2Params P) {
                     float a, b, cc, d;
                     taps(t, a, b, cc, d);
                     const float L = fmaf(ly, cc - a, a), R = fmaf(ly, d - b, b);
-                    loss += logf(U[i * 4 + j]) + Mp[i * 4 + j] - fmaf(lx, R - L, L);
-                    uu = gs / U[i * 4 + j];
+                    if constexpr (WT) {
+                        const float wt = P.one_m_eps * k2_class_weight(P.weight, t);
+                        const float aw = fmaf(P.eps_c, wsum, wt);
+                        loss += aw * (logf(U[i * 4 + j]) + Mp[i * 4 + j]) - wt * fmaf(lx, R - L, L);
+                        uu = gs * aw / U[i * 4 + j];
+                        const int lyi = lyi0 + 2 * i, lxi = lxi0 + 2 * j;
+                        va += (S2 - lyi) * (S2 - lxi); vb += (S2 - lyi) * lxi;
+                        vc += lyi * (S2 - lxi);        vd += lyi * lxi;
+                    } else {
+                        loss += logf(U[i * 4 + j]) + Mp[i * 4 + j] - fmaf(lx, R - L, L);
+                        uu = gs / U[i * 4 + j];
+                    }
                 }
                 U[i * 4 + j] = uu;
             }
+        if constexpr (WT) {
+            // smoothing: -(eps/C) sum over the counted pixels of the interpolated sum_c w_c x_c
+            const float rn = 1.f / (float)(S2 * S2);
+            loss = fmaf(-P.eps_c * rn, (float)va * wq.x + (float)vb * wq.y + (float)vc * wq.z + (float)vd * wq.w, loss);
+            const float k = -gs * P.eps_c * rn;
+            kv = make_float4(va ? k * (float)va : 0.f, vb ? k * (float)vb : 0.f, vc ? k * (float)vc : 0.f,
+                             vd ? k * (float)vd : 0.f);
+        }
     } else {
 #pragma unroll
         for (int i = 0; i < 16; ++i) U[i] = 0.f;
@@ -316,6 +381,10 @@ k2_fast_kernel(const K2Params P) {
             const float Y = fmaf(rs, Gy, ly0 * G);                        // sum lambda_y g
             const float XY = fmaf(ly0, X, rs * fmaf(rs, Gxy, lx0 * Gy));  // sum lambda_x lambda_y g
             float A = (G - X) - (Y - XY), Bv = X - XY, Cv = Y - XY, Dv = XY;
+            if constexpr (WT) {
+                const float wc = k2_class_weight(P.weight, c);
+                A = fmaf(kv.x, wc, A); Bv = fmaf(kv.y, wc, Bv); Cv = fmaf(kv.z, wc, Cv); Dv = fmaf(kv.w, wc, Dv);
+            }
             group_reduce4<LPG>(A, Bv, Cv, Dv, u);
             if (QUAD) {
                 if (writer) atomicAdd(gcell + (size_t)c * plane, A);
@@ -382,9 +451,7 @@ k2_fast_kernel(const K2Params P) {
         }
         // ---- - g * onehot: exact integer tap weights (lambda * 2s are odd integers), aggregated per
         //      distinct label of this thread's 16 pixels (blocky label maps: usually one), 4 reductions each
-        const int S2 = 2 * P.s;
         const float wscale = -gs / (float)(S2 * S2);
-        const int lyi0 = 2 * y0 + 1 - P.s - S2 * ky, lxi0 = 2 * x0 + 1 - P.s - S2 * kx;
         int cur = 0x7fffffff;
 #pragma unroll
         for (int i = 0; i < 16; ++i)
@@ -404,10 +471,11 @@ k2_fast_kernel(const K2Params P) {
                         nxt = min(nxt, t);
                     }
                 }
-            atomicAdd(gA + (size_t)cur * plane, wscale * (float)wa);
-            atomicAdd(gB + (size_t)cur * plane, wscale * (float)wb);
-            atomicAdd(gC + (size_t)cur * plane, wscale * (float)wc);
-            atomicAdd(gD + (size_t)cur * plane, wscale * (float)wd);
+            const float ws = WT ? wscale * (P.one_m_eps * k2_class_weight(P.weight, cur)) : wscale;
+            atomicAdd(gA + (size_t)cur * plane, ws * (float)wa);
+            atomicAdd(gB + (size_t)cur * plane, ws * (float)wb);
+            atomicAdd(gC + (size_t)cur * plane, ws * (float)wc);
+            atomicAdd(gD + (size_t)cur * plane, ws * (float)wd);
             cur = nxt;
         }
     }
@@ -421,9 +489,10 @@ k2_fast_kernel(const K2Params P) {
 // SPLIT = false: the one-call path (int64 labels; loss, -g*onehot and g*softmax all here).
 // SPLIT = true : the label-only work (valid count, packing, -onehot term) was done by k2_labels_prepass_kernel;
 //                this kernel adds sum(log-sum-exp - target logit) and the softmax term only.
-template <int S, bool SPLIT>
+// WT: the weighted / label-smoothed form (SPLIT = false only).
+template <int S, bool SPLIT, bool WT = false>
 __global__ void __launch_bounds__(128)
-k2_strip_kernel(const K2SParams P) {
+k2_strip_kernel(const K2SP<WT> P) {
     constexpr int TPG = S / 2, GPW = 32 / TPG, WGX = GPW / 2, CS = GPW * 4;
     extern __shared__ float smem[];
     const int C = P.C;
@@ -453,14 +522,14 @@ k2_strip_kernel(const K2SParams P) {
             else dst[c * CS] = 0.f;
         }
     }
-    k2_strip_warp<S, SPLIT, CS>(P, st, true, n, GY0, GX0, lane);
+    k2_strip_warp<S, SPLIT, CS, false, WT>(P, st, true, n, GY0, GX0, lane);
 }
 
 // The same strips with the taps read from the class-plane-major map itself (no staged tile): for class counts whose
 // tile would not leave enough warps per SM (BASELINE config 5: C = 847 -> 54 KB per warp, four warps per SM).
-template <int S, bool SPLIT>
+template <int S, bool SPLIT, bool WT = false>
 __global__ void __launch_bounds__(128)
-k2_strip_gtaps_kernel(const K2SParams P) {
+k2_strip_gtaps_kernel(const K2SP<WT> P) {
     constexpr int TPG = S / 2, GPW = 32 / TPG, WGX = GPW / 2, CS = GPW * 4;
     const int lane = threadIdx.x & 31;
     const long long wt = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -469,7 +538,7 @@ k2_strip_gtaps_kernel(const K2SParams P) {
     const int n = (int)(wt / tiles_per_img);
     const int trem = (int)(wt - (long long)n * tiles_per_img);
     const int tyi = trem / P.ntx, txi = trem - tyi * P.ntx;
-    k2_strip_warp<S, SPLIT, CS, true>(P, nullptr, true, n, tyi * 2, txi * WGX, lane);
+    k2_strip_warp<S, SPLIT, CS, true, WT>(P, nullptr, true, n, tyi * 2, txi * WGX, lane);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -641,11 +710,14 @@ k2_pack_labels_kernel(const long long* __restrict__ labels, long long n8, int C,
 
 // ---------------------------------------------------------------------------------------------
 // generic path: any (h,w)->(H,W); one pixel per thread; exact 3-pass softmax; global atomics.
+// WT: the weighted / label-smoothed form (k2_strip.cuh: k2_class_weight), every term per pixel and class.
+template <bool WT = false>
 __global__ void __launch_bounds__(256)
 k2_generic_kernel(const float* __restrict__ low, const long long* __restrict__ labels,
                   float* __restrict__ grad_low, double* __restrict__ loss_sum,
                   const float* __restrict__ grad_scale, long long ignore_index,
-                  int B, int C, int h, int w, int H, int W, float scale_y, float scale_x) {
+                  int B, int C, int h, int w, int H, int W, float scale_y, float scale_x,
+                  const float* __restrict__ weight, float one_m_eps, float eps_c) {
     const long long HW = (long long)H * W;
     const long long total = (long long)B * HW;
     const float gs = grad_scale ? __ldg(grad_scale) : 1.f;
@@ -675,22 +747,36 @@ k2_generic_kernel(const float* __restrict__ low, const long long* __restrict__ l
             m = fmaxf(m, l);
         }
         float S = 0.f, lt = 0.f;
+        float wl = 0.f, wsum = 0.f;                         // WT: sum_c w_c x_c, sum_c w_c
         for (int c = 0; c < C; ++c) {
             const float* q = base + (size_t)c * h * w;
             float l = (1.f - ly) * ((1.f - lx) * __ldg(q + oa) + lx * __ldg(q + ob)) +
                       ly * ((1.f - lx) * __ldg(q + oc) + lx * __ldg(q + od));
             S += ex2f((l - m) * LOG2E);
             if (c == t) lt = l;
+            if constexpr (WT) {
+                const float wc = k2_class_weight(weight, c);
+                wl = fmaf(wc, l, wl);
+                wsum += wc;
+            }
         }
-        loss += lg2f(S) * LN2 + m - lt;
+        float a = 1.f, wt = 1.f;
+        if constexpr (WT) {
+            wt = one_m_eps * k2_class_weight(weight, t);
+            a = fmaf(eps_c, wsum, wt);
+            loss += a * (lg2f(S) * LN2 + m) - wt * lt - eps_c * wl;
+        } else {
+            loss += lg2f(S) * LN2 + m - lt;
+        }
         if (grad_low) {
-            const float u = gs / S;
+            const float u = WT ? gs * a / S : gs / S;
             float* gb = grad_low + (size_t)n * C * h * w;
             for (int c = 0; c < C; ++c) {
                 const float* q = base + (size_t)c * h * w;
                 float l = (1.f - ly) * ((1.f - lx) * __ldg(q + oa) + lx * __ldg(q + ob)) +
                           ly * ((1.f - lx) * __ldg(q + oc) + lx * __ldg(q + od));
-                float g = ex2f((l - m) * LOG2E) * u - (c == t ? gs : 0.f);
+                float g = ex2f((l - m) * LOG2E) * u - (c == t ? (WT ? gs * wt : gs) : 0.f);
+                if constexpr (WT) g -= gs * eps_c * k2_class_weight(weight, c);
                 float* gp = gb + (size_t)c * h * w;
                 atomicAdd(gp + oa, g * wa); atomicAdd(gp + ob, g * wb);
                 atomicAdd(gp + oc, g * wc); atomicAdd(gp + od, g * wd);
@@ -743,6 +829,23 @@ extern "C" int lc2is_count_valid(const int64_t* d_labels, int64_t n, int C, int6
     return 0;
 }
 
+extern "C" int lc2is_ce_weight_sum(const int64_t* d_labels, int64_t n, int C, int64_t ignore_index,
+                                   const float* d_weight, double* d_wsum, lc2is_stream_t stream) {
+    if (int e = ensure_device()) return e;
+    if (n < 0) return fail(LC2IS_ERR_SHAPE, "negative n%s");
+    if (n == 0) return 0;
+    if (!d_labels || !d_wsum) return fail(LC2IS_ERR_ARG, "null pointer%s");
+    if ((uintptr_t)d_labels % 16) return fail(LC2IS_ERR_ARG, "labels must be 16-byte aligned%s");
+    long long blocks = (n / 2 + 255) / 256;
+    long long cap = (long long)sm_count() * 8;
+    if (blocks > cap) blocks = cap;
+    if (blocks < 1) blocks = 1;
+    k2_weight_sum_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+        (const long long*)d_labels, n, (long long)C, ignore_index, d_weight, d_wsum);
+    LC2IS_CHECK_LAUNCH("k2_weight_sum_kernel");
+    return 0;
+}
+
 extern "C" int lc2is_grad_to_bf16(const float* d_grad, int B, int C, int hw, void* d_grad_bf16,
                                   lc2is_stream_t stream) {
     if (int e = ensure_device()) return e;
@@ -764,8 +867,22 @@ extern "C" int lc2is_upsample_ce_fwd_bwd(const float* d_low, const int64_t* d_la
                                          int64_t ignore_index, const float* d_grad_scale,
                                          double* d_loss_sum, float* d_grad_low, void* d_grad_low_bf16,
                                          lc2is_stream_t stream) {
+    return lc2is_upsample_ce_fwd_bwd_ex(d_low, d_labels, B, C, h, w, H, W, ignore_index, nullptr, 0.f, d_grad_scale,
+                                        d_loss_sum, d_grad_low, d_grad_low_bf16, stream);
+}
+
+extern "C" int lc2is_upsample_ce_fwd_bwd_ex(const float* d_low, const int64_t* d_labels,
+                                            int B, int C, int h, int w, int H, int W,
+                                            int64_t ignore_index, const float* d_weight, float label_smoothing,
+                                            const float* d_grad_scale, double* d_loss_sum, float* d_grad_low,
+                                            void* d_grad_low_bf16, lc2is_stream_t stream) {
     if (int e = ensure_device()) return e;
     if (B < 0 || C <= 0 || h <= 0 || w <= 0 || H <= 0 || W <= 0) return fail(LC2IS_ERR_SHAPE, "bad shape%s");
+    if (!(label_smoothing >= 0.f && label_smoothing <= 1.f))
+        return fail(LC2IS_ERR_ARG, "label_smoothing must be in [0, 1]%s");
+    // the unweighted instantiations unless a weight or a smoothing is asked for
+    const bool wt = d_weight != nullptr || label_smoothing != 0.f;
+    const float one_m_eps = 1.f - label_smoothing, eps_c = label_smoothing / (float)C;
     if (B == 0) return 0;
     if (!d_low || !d_labels || !d_loss_sum) return fail(LC2IS_ERR_ARG, "null pointer%s");
     if (d_grad_low_bf16 && !d_grad_low)
@@ -778,10 +895,12 @@ extern "C" int lc2is_upsample_ce_fwd_bwd(const float* d_low, const int64_t* d_la
     bool fast = fast_scale(h, w, H, W, &s) && s <= 16;
     // ---- strip path: s = 8 / 16 -----------------------------------------------------------------------
     if (fast && s >= 8 && ((uintptr_t)d_labels % 16) == 0) {
-        K2SParams P;
+        K2SParamsW PW;
+        K2SParams& P = PW;
         P.low = d_low; P.labels = (const long long*)d_labels; P.labels16 = nullptr; P.n_valid = nullptr; P.grad_low = d_grad_low;
         P.loss_sum = d_loss_sum; P.grad_scale = d_grad_scale; P.ignore_index = ignore_index;
         P.B = B; P.C = C; P.h = h; P.w = w; P.H = H; P.W = W;
+        PW.weight = d_weight; PW.one_m_eps = one_m_eps; PW.eps_c = eps_c;
         // warps are independent; a warp's tile of taps takes C * (32 / (s/2)) * 16 bytes of shared memory
         const size_t smem_warp = (size_t)(C + 2) * (64 / s) * 16;
         int wpc = 4;
@@ -796,15 +915,18 @@ extern "C" int lc2is_upsample_ce_fwd_bwd(const float* d_low, const int64_t* d_la
             const unsigned grid = (unsigned)((tiles + wpc - 1) / wpc);
             auto launch = [&](auto kernel) -> int {
                 LC2IS_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                kernel<<<grid, wpc * 32, smem, st>>>(P);
+                kernel<<<grid, wpc * 32, smem, st>>>(PW);          // (sliced to K2SParams for the unweighted kernels)
                 return 0;
             };
             auto launch_g = [&](auto kernel) -> int {
-                kernel<<<(unsigned)((tiles + 3) / 4), 128, 0, st>>>(P);
+                kernel<<<(unsigned)((tiles + 3) / 4), 128, 0, st>>>(PW);
                 return 0;
             };
-            int e = gtaps ? (s == 8 ? launch_g(k2_strip_gtaps_kernel<8, false>) : launch_g(k2_strip_gtaps_kernel<16, false>))
-                          : (s == 8 ? launch(k2_strip_kernel<8, false>) : launch(k2_strip_kernel<16, false>));
+            int e = wt ? (gtaps ? (s == 8 ? launch_g(k2_strip_gtaps_kernel<8, false, true>)
+                                          : launch_g(k2_strip_gtaps_kernel<16, false, true>))
+                                : (s == 8 ? launch(k2_strip_kernel<8, false, true>) : launch(k2_strip_kernel<16, false, true>)))
+                       : (gtaps ? (s == 8 ? launch_g(k2_strip_gtaps_kernel<8, false>) : launch_g(k2_strip_gtaps_kernel<16, false>))
+                                : (s == 8 ? launch(k2_strip_kernel<8, false>) : launch(k2_strip_kernel<16, false>)));
             if (e) return e;
             LC2IS_CHECK_LAUNCH("k2_strip_kernel");
             if (d_grad_low_bf16) return lc2is_grad_to_bf16(d_grad_low, B, C, h * w, d_grad_low_bf16, stream);
@@ -820,6 +942,7 @@ extern "C" int lc2is_upsample_ce_fwd_bwd(const float* d_low, const int64_t* d_la
         P.loss_sum = d_loss_sum; P.grad_scale = d_grad_scale; P.ignore_index = ignore_index;
         P.B = B; P.C = C; P.h = h; P.w = w; P.H = H; P.W = W;
         P.s = s; P.off = g.off; P.rs = g.rs;
+        P.weight = d_weight; P.one_m_eps = one_m_eps; P.eps_c = eps_c;
         const int bps = s / 4;
         P.q = (g.off + s / 2) / 4;
         // 128 threads = tgy*tgx groups of bps*bps threads; tile = 32 x 64 pixels
@@ -834,7 +957,7 @@ extern "C" int lc2is_upsample_ce_fwd_bwd(const float* d_low, const int64_t* d_la
             kernel<<<grid, 128, smem, st>>>(P);
             return 0;
         };
-        int e = launch(k2_fast_kernel<1>);
+        int e = wt ? launch(k2_fast_kernel<1, true>) : launch(k2_fast_kernel<1>);
         if (e) return e;
         LC2IS_CHECK_LAUNCH("k2_fast_kernel");
     } else {
@@ -843,9 +966,9 @@ extern "C" int lc2is_upsample_ce_fwd_bwd(const float* d_low, const int64_t* d_la
         long long blocks = (total + 255) / 256;
         long long cap = (long long)sm_count() * 8;
         if (blocks > cap) blocks = cap;
-        k2_generic_kernel<<<(unsigned)blocks, 256, 0, st>>>(d_low, (const long long*)d_labels, d_grad_low,
-                                                             d_loss_sum, d_grad_scale, ignore_index,
-                                                             B, C, h, w, H, W, sy, sx);
+        auto kernel = wt ? k2_generic_kernel<true> : k2_generic_kernel<false>;
+        kernel<<<(unsigned)blocks, 256, 0, st>>>(d_low, (const long long*)d_labels, d_grad_low, d_loss_sum, d_grad_scale,
+                                                 ignore_index, B, C, h, w, H, W, sy, sx, d_weight, one_m_eps, eps_c);
         LC2IS_CHECK_LAUNCH("k2_generic_kernel");
     }
     if (d_grad_low_bf16) return lc2is_grad_to_bf16(d_grad_low, B, C, h * w, d_grad_low_bf16, stream);

@@ -5,6 +5,8 @@
       ``v = F.normalize(v, dim=1); t = F.normalize(t, dim=2); einsum('bchw,bkc->bkhw', v, t)``
 * :class:`SegHeadLoss`    - K0 -> K1 -> K2 -> (K1b) fused: logits, upsampled softmax-CE and all
       gradients with no [B,C,H,W] tensor and no autograd graph in between.
+* :class:`UpsampledCrossEntropyLoss` - K2 for a configured criterion (engine.py:94 on final.py:44):
+      ``nn.CrossEntropyLoss(weight, ignore_index, reduction, label_smoothing)`` of the bilinearly upsampled score map.
 """
 from __future__ import annotations
 
@@ -14,6 +16,7 @@ import torch
 from torch import Tensor, nn
 
 from . import ops
+from .model.loss import _UpsampleCE
 
 
 def _hw_shape(P: int, hw_shape) -> Tuple[int, int]:
@@ -87,16 +90,24 @@ def upsample_tokens_bicubic4(x: Tensor, hw_shape: Optional[Tuple[int, int]] = No
 class _SegHeadLoss(torch.autograd.Function):
 
     @staticmethod
-    def forward(ctx, v, t, labels, ignore_index, normalize, logit_scale, hw_shape, reduction):
+    def forward(ctx, v, t, labels, ignore_index, normalize, logit_scale, hw_shape, reduction, weight=None,
+                label_smoothing=0.0):
         t_hat, inv_t = ops.proto_normalize(t.float(), normalize)
         C = t.shape[-2]
         logits, v_hat, inv_v = ops.cosine_logits_fwd(v, t_hat, C, hw_shape, normalize, logit_scale)
         need_grad = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
         n_valid = ops.count_valid(labels, C, ignore_index)
-        gscale = ops.mean_scale(n_valid) if reduction == "mean" else None
-        loss_sum, _, gbf = ops.upsample_ce(logits, labels, ignore_index, gscale, want_grad=need_grad,
-                                           want_bf16=need_grad)
-        loss = ops.finalize_loss(loss_sum, n_valid) if reduction == "mean" else loss_sum.float()
+        if weight is None and label_smoothing == 0:
+            gscale = ops.mean_scale(n_valid) if reduction == "mean" else None
+            loss_sum, _, gbf = ops.upsample_ce(logits, labels, ignore_index, gscale, want_grad=need_grad,
+                                               want_bf16=need_grad)
+            loss = ops.finalize_loss(loss_sum, n_valid) if reduction == "mean" else loss_sum.float()
+        else:
+            den = ops.ce_weight_sum(labels, C, ignore_index, weight) if reduction == "mean" else None
+            gscale = torch.reciprocal(den).float() if reduction == "mean" else None
+            loss_sum, _, gbf = ops.upsample_ce(logits, labels, ignore_index, gscale, want_grad=need_grad,
+                                               want_bf16=need_grad, weight=weight, label_smoothing=label_smoothing)
+            loss = ops.weighted_mean_loss(loss_sum, den) if reduction == "mean" else loss_sum.float()
         if need_grad:
             ctx.save_for_backward(gbf, logits, v_hat, inv_v, t_hat, inv_t)
         ctx.meta = (C, normalize, logit_scale, v.dtype, t.dtype, t.dim())
@@ -113,7 +124,53 @@ class _SegHeadLoss(torch.autograd.Function):
                                                grad_scale=gs, grad_v_dtype=gv_dtype)
         if t_dim == 2:
             grad_t = grad_t[0]
-        return grad_v.to(v_dtype), grad_t.to(t_dtype), None, None, None, None, None, None
+        return grad_v.to(v_dtype), grad_t.to(t_dtype), None, None, None, None, None, None, None, None
+
+
+def _check_ce_options(C: int, weight: Optional[Tensor], label_smoothing: float, reduction: str) -> None:
+    """The argument errors nn.CrossEntropyLoss raises, before any device work."""
+    if reduction not in ("mean", "sum"):
+        raise NotImplementedError(
+            "reduction='none' needs a backward that takes a per-pixel upstream gradient; the fused forward+backward "
+            "kernels support reduction='mean' | 'sum'")
+    if not 0.0 <= label_smoothing <= 1.0:
+        raise RuntimeError(f"label_smoothing must be between 0.0 and 1.0. Got: {label_smoothing}")
+    if weight is not None and (weight.dim() != 1 or weight.numel() != C):
+        raise RuntimeError(f"weight tensor should be defined either for all {C} classes or no classes but got weight "
+                           f"tensor of shape: {list(weight.shape)}")
+
+
+class UpsampledCrossEntropyLoss(nn.CrossEntropyLoss):
+    """``nn.CrossEntropyLoss(weight, ignore_index=..., reduction=..., label_smoothing=...)`` applied to
+    ``F.interpolate(input, size=target.shape[-2:], mode="bilinear", align_corners=False)`` - the criterion of
+    engine.py:94 on the score map of final.py:44 - without the upsampled [B,C,H,W] tensor: one fused K2 pass computes the
+    loss and d loss / d input.
+
+    forward(input [B,C,h,w] low-resolution scores (fp32 / bf16 / fp16), target [B,H,W] int64) -> scalar.  Any (H, W):
+    power-of-two scales 4 / 8 / 16 take the fast kernels, the rest the generic one.  ``weight`` is a buffer (follows
+    ``.to()`` and ``state_dict``); 'mean' divides by the summed weights of the counted pixels, like torch.  Labels outside
+    [0, C) that are not ignore_index are skipped.  reduction='none' is not supported.  CUDA tensors only; no host
+    synchronisation (CUDA-graph capturable)."""
+
+    def __init__(self, weight: Optional[Tensor] = None, size_average=None, ignore_index: int = -100, reduce=None,
+                 reduction: str = "mean", label_smoothing: float = 0.0) -> None:
+        super().__init__(weight, size_average, ignore_index, reduce, reduction, label_smoothing)
+        if self.reduction not in ("mean", "sum"):
+            _check_ce_options(0, None, 0.0, self.reduction)
+
+    def forward(self, input: Tensor, target: Tensor) -> Tensor:
+        if input.dim() != 4 or target.dim() != 3 or target.shape[0] != input.shape[0]:
+            raise ValueError(f"UpsampledCrossEntropyLoss: input must be [B,C,h,w] and target [B,H,W], got "
+                             f"{tuple(input.shape)} / {tuple(target.shape)}")
+        weight = self.weight
+        _check_ce_options(input.shape[1], weight, float(self.label_smoothing), self.reduction)
+        if target.device != input.device or (weight is not None and weight.device != input.device):
+            raise RuntimeError("Expected all tensors to be on the same device, but found input on "
+                               f"{input.device}, target on {target.device}"
+                               + ("" if weight is None else f", weight on {weight.device}"))
+        if weight is not None:
+            weight = weight.detach().float().contiguous()
+        return _UpsampleCE.apply(input, target, self.ignore_index, self.reduction, weight, float(self.label_smoothing))
 
 
 class SegHeadLoss(nn.Module):
@@ -121,10 +178,13 @@ class SegHeadLoss(nn.Module):
     (final.py:41-44 + engine.py:94, or final.py:266-268 + loss.py:17-21 for the aux head).
 
     forward(v [B,P,D], t [K,D]|[B,K,D], labels [B,H,W] int64) -> (loss, low_logits [B,K,h,w], n_valid)
+
+    ``weight`` (fp32 [K], a buffer) and ``label_smoothing`` are those of ``nn.CrossEntropyLoss`` (see
+    :class:`UpsampledCrossEntropyLoss`); n_valid stays the number of counted pixels.
     """
 
     def __init__(self, ignore_index: int = -100, normalize: bool = True, logit_scale: float = 1.0,
-                 reduction: str = "mean") -> None:
+                 reduction: str = "mean", weight: Optional[Tensor] = None, label_smoothing: float = 0.0) -> None:
         super().__init__()
         if reduction not in ("mean", "sum"):
             raise NotImplementedError("SegHeadLoss supports reduction='mean' | 'sum'")
@@ -132,8 +192,14 @@ class SegHeadLoss(nn.Module):
         self.normalize = normalize
         self.logit_scale = logit_scale
         self.reduction = reduction
+        self.register_buffer("weight", weight)
+        self.label_smoothing = label_smoothing
 
     def forward(self, v: Tensor, t: Tensor, labels: Tensor, hw_shape=None):
         h, w = _hw_shape(v.shape[1], hw_shape)
+        weight = self.weight
+        _check_ce_options(t.shape[-2], weight, float(self.label_smoothing), self.reduction)
+        if weight is not None:
+            weight = weight.detach().float().contiguous()
         return _SegHeadLoss.apply(v, t, labels, self.ignore_index, self.normalize, self.logit_scale, (h, w),
-                                  self.reduction)
+                                  self.reduction, weight, float(self.label_smoothing))

@@ -17,15 +17,26 @@ from .. import ops
 
 
 class _UpsampleCE(torch.autograd.Function):
+    """weight (fp32 [C]) / label_smoothing select the weighted kernels; 'mean' then divides by sum_i w[t_i] over the
+    counted pixels (ops.ce_weight_sum), all on the device."""
 
     @staticmethod
-    def forward(ctx, low: Tensor, target: Tensor, ignore_index: int, reduction: str):
+    def forward(ctx, low: Tensor, target: Tensor, ignore_index: int, reduction: str,
+                weight: Optional[Tensor] = None, label_smoothing: float = 0.0):
         need_grad = ctx.needs_input_grad[0]
         low32 = low.float()
-        n_valid = ops.count_valid(target, low.shape[1], ignore_index)
-        gscale = ops.mean_scale(n_valid) if reduction == "mean" else None
-        loss_sum, grad, _ = ops.upsample_ce(low32, target, ignore_index, gscale, want_grad=need_grad)
-        loss = ops.finalize_loss(loss_sum, n_valid) if reduction == "mean" else loss_sum.float()
+        if weight is None and label_smoothing == 0:
+            n_valid = ops.count_valid(target, low.shape[1], ignore_index)
+            gscale = ops.mean_scale(n_valid) if reduction == "mean" else None
+            loss_sum, grad, _ = ops.upsample_ce(low32, target, ignore_index, gscale, want_grad=need_grad)
+            loss = ops.finalize_loss(loss_sum, n_valid) if reduction == "mean" else loss_sum.float()
+        else:
+            den = ops.ce_weight_sum(target, low.shape[1], ignore_index, weight) if reduction == "mean" else None
+            # 1 / 0 = inf when nothing is counted: every gradient term of an uncounted pixel is a select, not a product
+            gscale = torch.reciprocal(den).float() if reduction == "mean" else None
+            loss_sum, grad, _ = ops.upsample_ce(low32, target, ignore_index, gscale, want_grad=need_grad, weight=weight,
+                                                label_smoothing=label_smoothing)
+            loss = ops.weighted_mean_loss(loss_sum, den) if reduction == "mean" else loss_sum.float()
         if need_grad:
             ctx.save_for_backward(grad)
         ctx.in_dtype = low.dtype
@@ -34,7 +45,7 @@ class _UpsampleCE(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_out: Tensor):
         (grad,) = ctx.saved_tensors
-        return (grad * grad_out).to(ctx.in_dtype), None, None, None
+        return (grad * grad_out).to(ctx.in_dtype), None, None, None, None, None
 
 
 class AuxiliaryLoss(nn.CrossEntropyLoss):
@@ -46,7 +57,8 @@ class AuxiliaryLoss(nn.CrossEntropyLoss):
         if weight is not None or label_smoothing != 0 or self.reduction not in ("mean", "sum"):
             raise NotImplementedError(
                 "the B200 AuxiliaryLoss kernel covers the reference's usage (no class weights, no label "
-                "smoothing, reduction 'mean'|'sum'); there is deliberately no silent PyTorch fallback")
+                "smoothing, reduction 'mean'|'sum'); there is deliberately no silent PyTorch fallback.  "
+                "lc2is_b200.head.UpsampledCrossEntropyLoss takes class weights and label smoothing")
 
     def forward(self, input: Tensor, target: Tensor) -> Tensor:
         B, H, W = target.shape

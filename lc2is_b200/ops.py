@@ -193,23 +193,56 @@ def finalize_loss(loss_sum: Tensor, n_valid: Tensor) -> Tensor:
     return out
 
 
+def ce_weight_sum(labels: Tensor, n_classes: int, ignore_index: int, weight: Optional[Tensor] = None,
+                  out: Optional[Tensor] = None) -> Tensor:
+    """sum of weight[label] over the counted labels (in [0, n_classes), != ignore_index), double[1] on the device: the
+    'mean' denominator of the weighted cross-entropy.  weight=None counts them."""
+    labels = _req(labels, torch.int64, "labels")
+    if weight is not None:
+        weight = _class_weight(weight, n_classes)
+    if out is None:
+        out = torch.zeros(1, dtype=torch.float64, device=labels.device)
+    check(lib.lc2is_ce_weight_sum(ptr(labels), labels.numel(), int(n_classes), int(ignore_index), ptr(weight), ptr(out),
+                                  stream_ptr()), "lc2is_ce_weight_sum")
+    return out
+
+
+def weighted_mean_loss(loss_sum: Tensor, wsum: Tensor) -> Tensor:
+    """loss_sum / wsum as fp32 [1] on the device; NaN when wsum == 0 - torch divides the target and the smoothing parts
+    separately, so counted pixels that all have weight 0 give 0/0 even when the smoothing sum is not 0."""
+    return torch.where(wsum != 0, loss_sum / wsum, torch.full_like(wsum, float("nan"))).float()
+
+
+def _class_weight(weight: Tensor, n_classes: int) -> Tensor:
+    weight = _req(weight, torch.float32, "weight")
+    if weight.dim() != 1 or weight.numel() != n_classes:
+        raise _lib.Lc2isError(f"weight must have shape [{n_classes}], got {list(weight.shape)}")
+    return weight
+
+
 def upsample_ce(low: Tensor, labels: Tensor, ignore_index: int = -100, grad_scale: Optional[Tensor] = None,
                 want_grad: bool = True, want_bf16: bool = False,
-                loss_sum: Optional[Tensor] = None) -> Tuple[Tensor, Optional[Tensor], Optional[Tensor]]:
-    """low [B,C,h,w] fp32, labels [B,H,W] int64 -> (loss_sum double[1], grad_low fp32, grad_low_bf16)."""
+                loss_sum: Optional[Tensor] = None, weight: Optional[Tensor] = None,
+                label_smoothing: float = 0.0) -> Tuple[Tensor, Optional[Tensor], Optional[Tensor]]:
+    """low [B,C,h,w] fp32, labels [B,H,W] int64 -> (loss_sum double[1], grad_low fp32, grad_low_bf16).
+    weight (fp32 [C] on the device) / label_smoothing: the weighted form (lc2is_upsample_ce_fwd_bwd_ex); loss_sum is then
+    the sum of the per-pixel losses, to be divided by ce_weight_sum for reduction='mean'."""
     low = _req(low, torch.float32, "low")
     labels = _req(labels, torch.int64, "labels")
     B, C, h, w = low.shape
     Bl, H, W = labels.shape
     if Bl != B:
         raise _lib.Lc2isError("batch mismatch between logits and labels")
+    if weight is not None:
+        weight = _class_weight(weight, C)
     if loss_sum is None:
         loss_sum = torch.zeros(1, dtype=torch.float64, device=low.device)
     grad = torch.empty_like(low) if (want_grad or want_bf16) else None
     gbf = torch.empty(B, _lib.class_pad(C), h * w, dtype=torch.bfloat16, device=low.device) if want_bf16 else None
-    check(lib.lc2is_upsample_ce_fwd_bwd(ptr(low), ptr(labels), B, C, h, w, H, W, int(ignore_index),
-                                        ptr(grad_scale), ptr(loss_sum), ptr(grad), ptr(gbf), stream_ptr()),
-          "lc2is_upsample_ce_fwd_bwd")
+    check(lib.lc2is_upsample_ce_fwd_bwd_ex(ptr(low), ptr(labels), B, C, h, w, H, W, int(ignore_index), ptr(weight),
+                                           float(label_smoothing), ptr(grad_scale), ptr(loss_sum), ptr(grad), ptr(gbf),
+                                           stream_ptr()),
+          "lc2is_upsample_ce_fwd_bwd_ex")
     return loss_sum, grad, gbf
 
 
