@@ -19,13 +19,20 @@ sum evaluated with n roundings of unit round-off u).  The tests compare per elem
 
 Everything runs in float64 on the device of the given tensors, one image at a time (so that the 16 x 16384-pixel case
 needs a few GB on a GPU, and small shapes can run on the CPU).  A float64 G skips the bf16 rounding of the operand: the
-exact algebra, which the host tests compare with torch.autograd."""
+exact algebra, which the host tests compare with torch.autograd.
+
+``check_bound`` asserts a kernel's result against a reference and its A; test_gpu_k1b_exact.py and
+test_gpu_step_routes.py share it."""
 from __future__ import annotations
 
 from typing import NamedTuple, Optional
 
 import torch
 from torch import Tensor
+
+# check_bound's per-element bound |got - ref| <= TAU * A: 2^7 x the fp32 unit round-off (test_gpu_k1b_exact.py says why)
+TAU = 2.0 ** -16
+BF16_OUT = 2.0 ** -8            # output rounding of a bf16 grad_v: the bf16 unit round-off (half an ulp <= 2^-8 |x|)
 
 
 class K1bReference(NamedTuple):
@@ -117,3 +124,28 @@ def k1b_reference(G: Tensor, logits: Tensor, v: Tensor, inv_v: Tensor, t_hat: Te
     else:
         gt, gt_A = sg * st, sg_abs * st_abs
     return K1bReference(gv, gv_A, gt, gt_A)
+
+
+def check_bound(name, got, ref, A, bf16_out=False, base=None, tau=TAU):
+    """|got - (base + ref)| <= tau * A (+ BF16_OUT |ref|) per element, asserted on the maxima of [128 rows x 64 channels]
+    blocks of the [images | sets, rows, D] tensors.  -> (worst |got - ref| / A, worst share of the bound used)."""
+    got = got.to(ref.device).double().reshape(ref.shape)
+    if base is not None:
+        got = got - base.to(ref.device).double().reshape(ref.shape)
+    err = (got - ref).abs()
+    bound = tau * A + (BF16_OUT * ref.abs() if bf16_out else 0.0)
+    if base is not None:                           # one fp32 rounding of base + result
+        bound = bound + 2.0 ** -24 * (base.to(ref.device).double().reshape(ref.shape) + ref).abs()
+    use = torch.where(err == 0, torch.zeros_like(err), err / bound)          # NaN (unwritten) stays NaN
+    X, R, D = use.shape
+    Rp = -(-R // 128) * 128
+    blocks = torch.nn.functional.pad(use, (0, 0, 0, Rp - R)).view(X, Rp // 128, 128, D // 64, 64).amax(dim=(2, 4))
+    bad = ~(blocks <= 1)
+    if bool(bad.any()):
+        worst = torch.nan_to_num(blocks, nan=float("inf")).flatten().argmax()
+        x, rt, cb = (int(i) for i in torch.unravel_index(worst, blocks.shape))
+        raise AssertionError(f"{name}: {int(bad.sum())} of {blocks.numel()} [128 x 64] blocks exceed the bound; worst: "
+                             f"image/set {x}, rows {128 * rt}.., channels {64 * cb}.. at {float(blocks[x, rt, cb]):.3g} "
+                             f"x the bound (worst |got-ref|/A overall {float((err / A).nan_to_num(float('inf')).max()):.3g})")
+    pos = A > 0
+    return float((err[pos] / A[pos]).max()), float(blocks.max())

@@ -29,14 +29,12 @@ import itertools
 import pytest
 import torch
 
-from k1b_reference import k1b_reference
+from k1b_reference import check_bound as _check, k1b_reference
 from lc2is_b200 import _lib, head, ops
 from lc2is_b200._lib import BF16, BWD_RAW_V, BWD_REUSE_PREP, F32, lib, ptr, stream_ptr
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
-TAU = 2.0 ** -16
-BF16_OUT = 2.0 ** -8            # output rounding of a bf16 grad_v: the bf16 unit round-off (half an ulp <= 2^-8 |x|)
 ERR_ARG, ERR_SHAPE = -1, -2
 
 
@@ -99,31 +97,6 @@ def _bwd(G, logits, V, inv_v, t_hat, inv_t, C, *, normalize=True, scale=1.0, gsc
                                           ptr(inv_v), ptr(t_hat), ptr(inv_t), B, hw, D, n_sets, C, int(normalize),
                                           float(scale), ptr(gscale), ptr(gv), ops._dt(gv) if gv is not None else F32,
                                           ptr(gt), ptr(ws), stream_ptr(), flags)
-
-
-def _check(name, got, ref, A, bf16_out=False, base=None):
-    """|got - (base + ref)| <= TAU * A (+ BF16_OUT |ref|) per element, asserted on the maxima of [128 rows x 64 channels]
-    blocks of the [images | sets, rows, D] tensors.  -> (worst |got - ref| / A, worst share of the bound used)."""
-    got = got.to(ref.device).double().reshape(ref.shape)
-    if base is not None:
-        got = got - base.to(ref.device).double().reshape(ref.shape)
-    err = (got - ref).abs()
-    bound = TAU * A + (BF16_OUT * ref.abs() if bf16_out else 0.0)
-    if base is not None:                           # one fp32 rounding of base + result
-        bound = bound + 2.0 ** -24 * (base.to(ref.device).double().reshape(ref.shape) + ref).abs()
-    use = torch.where(err == 0, torch.zeros_like(err), err / bound)          # NaN (unwritten) stays NaN
-    X, R, D = use.shape
-    Rp = -(-R // 128) * 128
-    blocks = torch.nn.functional.pad(use, (0, 0, 0, Rp - R)).view(X, Rp // 128, 128, D // 64, 64).amax(dim=(2, 4))
-    bad = ~(blocks <= 1)
-    if bool(bad.any()):
-        worst = torch.nan_to_num(blocks, nan=float("inf")).flatten().argmax()
-        x, rt, cb = (int(i) for i in torch.unravel_index(worst, blocks.shape))
-        raise AssertionError(f"{name}: {int(bad.sum())} of {blocks.numel()} [128 x 64] blocks exceed the bound; worst: "
-                             f"image/set {x}, rows {128 * rt}.., channels {64 * cb}.. at {float(blocks[x, rt, cb]):.3g} "
-                             f"x the bound (worst |got-ref|/A overall {float((err / A).nan_to_num(float('inf')).max()):.3g})")
-    pos = A > 0
-    return float((err[pos] / A[pos]).max()), float(blocks.max())
 
 
 def _report(case, gv, gt):
