@@ -318,6 +318,31 @@ int lc2is_pack_labels(const int64_t* d_labels, int64_t n, int C, int64_t ignore_
                       uint16_t* d_labels_packed, int64_t* d_n_valid, lc2is_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------
+ * The cross-entropy stages of a whole step (K2 + K3 on the logits of K1; what HeadStep and
+ * lc2is_head_step_host run), each picking its kernels from the geometry:
+ *   route     labels stage              CE stage                                argmax stage
+ *   fused     lc2is_pack_labels         lc2is_ce_argmax_fused_packed, onehot=1  nothing
+ *             (packs, counts)           (loss, softmax - onehot, confmat)
+ *   split     lc2is_ce_labels_prepass   lc2is_upsample_ce_packed                lc2is_argmax_confmat_lowres_packed
+ *             (packs, counts, -onehot)
+ *   one-call  lc2is_count_valid         lc2is_upsample_ce_fwd_bwd               lc2is_argmax_confmat_lowres
+ *                                       (d_grad_scale NULL)                     (LC2IS_BILINEAR, labels at H x W)
+ * fused where lc2is_ce_argmax_fused_supported, else split where lc2is_ce_split_supported, else one-call.
+ * The CE and argmax stages read the packed labels the labels stage wrote.  d_n_valid, d_loss_sum, d_confmat ACCUMULATE.
+ * d_labels [B,H,W] int64 (read by the labels stage, and by the other two on the one-call route).
+ * d_labels_packed [B,H,W] uint16, written by the labels stage; NULL only on the one-call route (else LC2IS_ERR_ARG).
+ * d_grad_low [B,C,h,w] fp32, un-scaled (1/n_valid is K1b's d_grad_scale), or NULL = forward only: on the split and fused
+ *   routes the labels and CE stages ACCUMULATE into it (zero it first), on the one-call route the CE stage overwrites it.
+ */
+int lc2is_step_ce_labels(const int64_t* d_labels, int B, int C, int h, int w, int H, int W, int64_t ignore_index,
+                         uint16_t* d_labels_packed, int64_t* d_n_valid, float* d_grad_low, lc2is_stream_t stream);
+int lc2is_step_ce(const float* d_low, const int64_t* d_labels, const uint16_t* d_labels_packed,
+                  int B, int C, int h, int w, int H, int W, int64_t ignore_index,
+                  double* d_loss_sum, float* d_grad_low, int64_t* d_confmat, lc2is_stream_t stream);
+int lc2is_step_argmax(const float* d_low, const int64_t* d_labels, const uint16_t* d_labels_packed,
+                      int B, int C, int h, int w, int H, int W, int64_t* d_confmat, lc2is_stream_t stream);
+
+/* ---------------------------------------------------------------------------------------
  * K4  ContrastiveLoss on the low-resolution logits.  Replaces model/loss.py:39-64
  *       loss_visual  = CrossEntropyLoss(out [B,C,h,w], labels [B,h,w])            (class axis, ignore_index)
  *       loss_textual = CrossEntropyLoss(out [B,h,w,C], one_hot(labels,151).float()) (torch takes dim 1 = the image-row

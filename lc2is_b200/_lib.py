@@ -75,6 +75,9 @@ SIGNATURES = {
     "lc2is_ce_argmax_fused_supported": (c_int, [c_int, c_int, c_int, c_int, c_int]),
     "lc2is_ce_argmax_fused_packed": (c_int, [_p, _p, c_int, c_int, c_int, c_int, c_int, c_int, _p, _p, c_int, _p, _p, _p, _p, _p]),
     "lc2is_pack_labels": (c_int, [_p, c_int64, c_int, c_int64, _p, _p, _p]),
+    "lc2is_step_ce_labels": (c_int, [_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int64, _p, _p, _p, _p]),
+    "lc2is_step_ce": (c_int, [_p, _p, _p, c_int, c_int, c_int, c_int, c_int, c_int, c_int64, _p, _p, _p, _p]),
+    "lc2is_step_argmax": (c_int, [_p, _p, _p, c_int, c_int, c_int, c_int, c_int, c_int, _p, _p]),
     "lc2is_head_step_workspace": (c_int64, [c_int, c_int, c_int, c_int, c_int, c_int]),
     "lc2is_head_step_host": (c_int, [_p, _p, _p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int64,
                                      c_float, c_int, _p, _p, _p, _p, _p, _p, _p, c_int, c_int]),

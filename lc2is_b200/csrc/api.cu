@@ -381,6 +381,102 @@ extern "C" int64_t lc2is_head_step_workspace(int B, int hw, int D, int C, int H,
     return (int64_t)step_layout(B, hw, D, C, H, W).total;
 }
 
+// ---------------------------------------------------------------------------------------------
+// The cross-entropy stages of a whole step (HeadStep through the lc2is_step_* entries, and head_step_enqueue).  The
+// route follows from the geometry: power-of-two scales 8 / 16 run the split form of K2 (labels packed ahead, packed-label
+// K2 / K3), x16 with a class count that fits it runs K2 and K3 as one kernel, other geometries the one-call K2 and the
+// int64-label K3.  The split and fused routes accumulate into a zeroed d_grad_low; the one-call K2 overwrites it.
+namespace {
+enum CeRoute { CE_ONE_CALL, CE_SPLIT, CE_FUSED };
+CeRoute ce_route(int C, int h, int w, int H, int W) {
+    if (!lc2is_ce_split_supported(h, w, H, W)) return CE_ONE_CALL;
+    return lc2is_ce_argmax_fused_supported(C, h, w, H, W) ? CE_FUSED : CE_SPLIT;
+}
+
+// Labels of nb images.  lb = 0: all of them int64 at d_labels.  lb = 1 / 2 (the host step's host-form labels, split
+// routes only): the first np are on the device in the host form - one byte per label at d_lab8 (lb = 1) or already
+// packed in d_packed (lb = 2) - and the other nb - np are int64 at d_labels + np * H * W.  n_valid += the counted
+// labels, except for two-byte host labels on the fused route (the CE stage counts those: ce_stage's d_count).
+int ce_labels_stage(CeRoute r, const int64_t* d_labels, const uint8_t* d_lab8, int lb, int np, int nb, int C, int h,
+                    int w, int H, int W, int64_t ign, uint16_t* d_packed, int64_t* d_nvalid, float* d_glow,
+                    lc2is_stream_t stream) {
+    const size_t HW = (size_t)H * W;
+    if (lb == 0) {
+        // the fused kernel only needs the labels packed and counted (it adds the -onehot term itself); the separate
+        // kernels need the label prepass (count, packing, -onehot)
+        if (r == CE_FUSED) return lc2is_pack_labels(d_labels, (int64_t)nb * HW, C, ign, d_packed, d_nvalid, stream);
+        if (r == CE_SPLIT)
+            return lc2is_ce_labels_prepass(d_labels, nb, C, h, w, H, W, ign, d_packed, d_nvalid, d_glow, stream);
+        return lc2is_count_valid(d_labels, (int64_t)nb * HW, C, ign, d_nvalid, stream);
+    }
+    // one-byte host labels are widened to the packed form, int64 ones packed; both count the valid pixels when nothing
+    // downstream does (the fused kernel counts for two-byte host labels, the prepass otherwise)
+    int64_t* cnt = (r == CE_FUSED && lb == 1) ? d_nvalid : nullptr;
+    if (lb == 1 && np > 0)
+        if (int e = lc2is_expand_labels(d_lab8, (int64_t)np * HW, C, ign, d_packed, cnt, stream)) return e;
+    if (np < nb)
+        if (int e = lc2is_pack_labels(d_labels + np * HW, (int64_t)(nb - np) * HW, C, ign, d_packed + np * HW, cnt,
+                                      stream))
+            return e;
+    if (r == CE_SPLIT) return lc2is_ce_labels_prepass_packed(d_packed, nb, C, h, w, H, W, d_nvalid, d_glow, stream);
+    return 0;
+}
+
+// K2 (+ K3 on the fused route).  d_count: n_valid for the fused kernel to add to (labels that arrived un-counted), or NULL.
+int ce_stage(CeRoute r, const float* d_low, const int64_t* d_labels, const uint16_t* d_packed, int B, int C, int h,
+             int w, int H, int W, int64_t ign, double* d_loss_sum, float* d_glow, int64_t* d_cm, int64_t* d_count,
+             lc2is_stream_t stream) {
+    if (r == CE_FUSED)
+        return lc2is_ce_argmax_fused_packed(d_low, d_packed, B, C, h, w, H, W, d_loss_sum, d_glow, 1, d_count, d_cm,
+                                            nullptr, nullptr, stream);
+    if (r == CE_SPLIT) return lc2is_upsample_ce_packed(d_low, d_packed, B, C, h, w, H, W, d_loss_sum, d_glow, stream);
+    return lc2is_upsample_ce_fwd_bwd(d_low, d_labels, B, C, h, w, H, W, ign, nullptr, d_loss_sum, d_glow, nullptr, stream);
+}
+
+// K3 where it is a kernel of its own
+int argmax_stage(CeRoute r, const float* d_low, const int64_t* d_labels, const uint16_t* d_packed, int B, int C, int h,
+                 int w, int H, int W, int64_t* d_cm, lc2is_stream_t stream) {
+    if (r == CE_FUSED) return 0;
+    if (r == CE_SPLIT)
+        return lc2is_argmax_confmat_lowres_packed(d_low, B, C, h, w, H, W, d_packed, d_cm, nullptr, nullptr, stream);
+    return lc2is_argmax_confmat_lowres(d_low, B, C, h, w, H, W, LC2IS_BILINEAR, d_labels, H, W, d_cm, nullptr, nullptr,
+                                       stream);
+}
+
+int step_route(int C, int h, int w, int H, int W, const uint16_t* d_labels_packed, CeRoute* r) {
+    if (int e = ensure_device()) return e;
+    *r = ce_route(C, h, w, H, W);
+    if (*r != CE_ONE_CALL && !d_labels_packed)
+        return fail(LC2IS_ERR_ARG, "d_labels_packed is NULL on a split geometry (scale 8 / 16)%s");
+    return 0;
+}
+}  // namespace
+
+extern "C" int lc2is_step_ce_labels(const int64_t* d_labels, int B, int C, int h, int w, int H, int W,
+                                    int64_t ignore_index, uint16_t* d_labels_packed, int64_t* d_n_valid,
+                                    float* d_grad_low, lc2is_stream_t stream) {
+    CeRoute r;
+    if (int e = step_route(C, h, w, H, W, d_labels_packed, &r)) return e;
+    return ce_labels_stage(r, d_labels, nullptr, 0, 0, B, C, h, w, H, W, ignore_index, d_labels_packed, d_n_valid,
+                           d_grad_low, stream);
+}
+
+extern "C" int lc2is_step_ce(const float* d_low, const int64_t* d_labels, const uint16_t* d_labels_packed,
+                             int B, int C, int h, int w, int H, int W, int64_t ignore_index,
+                             double* d_loss_sum, float* d_grad_low, int64_t* d_confmat, lc2is_stream_t stream) {
+    CeRoute r;
+    if (int e = step_route(C, h, w, H, W, d_labels_packed, &r)) return e;
+    return ce_stage(r, d_low, d_labels, d_labels_packed, B, C, h, w, H, W, ignore_index, d_loss_sum, d_grad_low,
+                    d_confmat, nullptr, stream);
+}
+
+extern "C" int lc2is_step_argmax(const float* d_low, const int64_t* d_labels, const uint16_t* d_labels_packed,
+                                 int B, int C, int h, int w, int H, int W, int64_t* d_confmat, lc2is_stream_t stream) {
+    CeRoute r;
+    if (int e = step_route(C, h, w, H, W, d_labels_packed, &r)) return e;
+    return argmax_stage(r, d_low, d_labels, d_labels_packed, B, C, h, w, H, W, d_confmat, stream);
+}
+
 static int head_step_enqueue(const void* h_v, const float* h_t, const int64_t* h_labels,
                              int B, int h, int w, int D, int C, int H, int W,
                              int64_t ignore_index, float logit_scale, int do_backward,
@@ -413,10 +509,8 @@ static int head_step_enqueue(const void* h_v, const float* h_t, const int64_t* h
     float* d_gscale = (float*)(ws + L.scalars + 16);
     float* d_loss = (float*)(ws + L.scalars + 20);
     int64_t* d_cm = (int64_t*)(ws + L.confmat);
-    // Power-of-two scales 8 / 16 run the split form of K2 (label prepass + packed-label kernels); other
-    // geometries the one-call K2 and the int64-label K3.
-    const bool split = lc2is_ce_split_supported(h, w, H, W) != 0;
-    const bool fused = split && lc2is_ce_argmax_fused_supported(C, h, w, H, W) != 0;   // one K2+K3 kernel (x16)
+    const CeRoute route = ce_route(C, h, w, H, W);
+    const bool split = route != CE_ONE_CALL;
 
     // The batch is cut into chunks: chunk i+1 is copied host->device on `copy_stream` while the
     // kernels of chunk i run on `stream` (engine.py:75 / :145 copy the whole batch up front).
@@ -434,8 +528,8 @@ static int head_step_enqueue(const void* h_v, const float* h_t, const int64_t* h
     if (n_raw > 0 && !h_labels) return fail(LC2IS_ERR_ARG, "n_raw > 0 needs h_labels%s");
     const int Bp = hpack ? B - n_raw : 0;                   // images whose labels are packed on the host
     // host form of the packed labels: one byte per label for C <= 254 (expanded to uint16 on the device, next to the
-    // copy: lc2is_expand_labels), else the uint16 form itself
-    const int lb = hpack ? host_label_bytes(C) : 2;
+    // copy: lc2is_expand_labels), else the uint16 form itself; 0 = no host form, every label crosses as int64
+    const int lb = hpack ? host_label_bytes(C) : 0;
     uint8_t* d_lab8 = (uint8_t*)d_labels;                   // the int64 area of the workspace is free when hpack
     if (prepacked && !hpack) return fail(LC2IS_ERR_UNSUPPORTED, "pre-packed labels need a split-path geometry (scale 8 / 16)%s");
     constexpr int MAXCH = 8;
@@ -510,46 +604,16 @@ static int head_step_enqueue(const void* h_v, const float* h_t, const int64_t* h
         }
         float* lg = d_logits + (size_t)b0 * C * hw;
         float* gl = do_backward ? d_glow + (size_t)b0 * C * hw : nullptr;
-        // labels: the fused K2+K3 kernel only needs them packed and counted (it adds the -onehot term itself);
-        // the separate kernels need the label prepass (count, packing, -onehot)
-        if (hpack) {
-            // one-byte host labels are widened to the packed form here, int64 ones packed; both count the valid pixels
-            // when nothing downstream does (the fused kernel counts for two-byte host labels, the prepass otherwise)
-            int64_t* cnt = (fused && lb == 1) ? d_nvalid : nullptr;
-            if (lb == 1 && np > 0)
-                STEP_RC(lc2is_expand_labels(d_lab8 + lab_off, (int64_t)np * H * W, C, ignore_index, d_packed + lab_off,
-                                            cnt, stream));
-            if (nr > 0)
-                STEP_RC(lc2is_pack_labels(d_labels + raw_off, (int64_t)nr * H * W, C, ignore_index, d_packed + raw_off,
-                                          cnt, stream));
-            if (!fused)
-                STEP_RC(lc2is_ce_labels_prepass_packed(d_packed + lab_off, nb, C, h, w, H, W, d_nvalid, gl, stream));
-        } else if (fused)
-            STEP_RC(lc2is_pack_labels(d_labels + lab_off, (int64_t)nb * H * W, C, ignore_index, d_packed + lab_off,
-                                      d_nvalid, stream));
-        else if (split)
-            STEP_RC(lc2is_ce_labels_prepass(d_labels + lab_off, nb, C, h, w, H, W, ignore_index, d_packed + lab_off,
-                                            d_nvalid, gl, stream));
-        else
-            STEP_RC(lc2is_count_valid(d_labels + lab_off, (int64_t)nb * H * W, C, ignore_index, d_nvalid, stream));
+        STEP_RC(ce_labels_stage(route, d_labels + lab_off, d_lab8 + lab_off, lb, np, nb, C, h, w, H, W, ignore_index,
+                                d_packed + lab_off, d_nvalid, gl, stream));
         if (i == 0) STEP_RC(lc2is_proto_normalize(d_t, 1, C, D, 1, d_that, d_invt, stream));
         // (row normalisation inside the GEMM: no v_hat; the backward takes the raw V)
         STEP_RC(lc2is_cosine_logits_fwd(d_v + v_off, LC2IS_BF16, nb, hw, D, d_that, 1, C, 1, logit_scale,
                                         nullptr, d_invv + (size_t)b0 * hw, lg, stream));
-        if (fused) {
-            // (two-byte labels packed on the host arrive un-counted: the kernel counts them)
-            STEP_RC(lc2is_ce_argmax_fused_packed(lg, d_packed + lab_off, nb, C, h, w, H, W, d_loss_sum, gl, 1,
-                                                 (hpack && lb == 2) ? d_nvalid : nullptr, d_cm, nullptr, nullptr, stream));
-        } else if (split) {
-            STEP_RC(lc2is_upsample_ce_packed(lg, d_packed + lab_off, nb, C, h, w, H, W, d_loss_sum, gl, stream));
-            STEP_RC(lc2is_argmax_confmat_lowres_packed(lg, nb, C, h, w, H, W, d_packed + lab_off, d_cm, nullptr,
-                                                       nullptr, stream));
-        } else {
-            STEP_RC(lc2is_upsample_ce_fwd_bwd(lg, d_labels + lab_off, nb, C, h, w, H, W, ignore_index, nullptr,
-                                              d_loss_sum, gl, nullptr, stream));
-            STEP_RC(lc2is_argmax_confmat_lowres(lg, nb, C, h, w, H, W, LC2IS_BILINEAR, d_labels + lab_off, H, W,
-                                                d_cm, nullptr, nullptr, stream));
-        }
+        // (two-byte labels packed on the host arrive un-counted: the fused kernel counts them)
+        STEP_RC(ce_stage(route, lg, d_labels + lab_off, d_packed + lab_off, nb, C, h, w, H, W, ignore_index, d_loss_sum,
+                         gl, d_cm, lb == 2 ? d_nvalid : nullptr, stream));
+        STEP_RC(argmax_stage(route, lg, d_labels + lab_off, d_packed + lab_off, nb, C, h, w, H, W, d_cm, stream));
     }
     STEP_RC(lc2is_mean_scale(d_nvalid, 1.0f, d_gscale, stream));
     if (do_backward) {

@@ -15,7 +15,7 @@ from typing import Optional
 import torch
 
 from . import _lib, dp
-from ._lib import BF16, BILINEAR, F32, check, lib, ptr, stream_ptr
+from ._lib import BF16, F32, check, lib, ptr, stream_ptr
 
 
 class _Block:
@@ -95,9 +95,10 @@ class HeadStep:
         self.v_hat = None if self.fuse_norm else e(M, D, dt=torch.bfloat16)
         self.inv_v = e(M)
         self.logits = e(B, C, h, w)
-        self.split = bool(lib.lc2is_ce_split_supported(h, w, H, W))     # label prepass + packed-label K2 / K3
+        # the route the lc2is_step_* stages take for this geometry: packed labels + packed-label K2 / K3 (split), at x16
+        # K2 and K3 as ONE kernel (fused, k23_rc_kernel)
+        self.split = bool(lib.lc2is_ce_split_supported(h, w, H, W))
         self.labels_packed = e(B, H, W, dt=torch.uint16) if self.split else None
-        # x16: K2 and K3 run as ONE kernel (k23_rc_kernel)
         self.fused = bool(self.split and lib.lc2is_ce_argmax_fused_supported(C, h, w, H, W))
         self.grad_v = e(B, self.hw, D, dt=torch.bfloat16)
         self._blocks = [_Block(B, C, D, h, w, dev), _Block(B, C, D, h, w, dev)]
@@ -274,25 +275,16 @@ class HeadStep:
 
     def _part_labels(self, labels, k: int) -> None:
         """zero-fill of block k + everything that depends on the labels only (packing, valid count)."""
-        st = stream_ptr()
         B, C, h, w, H, W = self.B, self.C, self.h, self.w, self.H, self.W
         blk = self._blocks[k]
         self._mark("zero-fill")
         blk.acc32.zero_()                                        # bucket, grad_low, scalars: one fill
         glow = ptr(blk.grad_low) if self.backward else None
         self._mark("label prepass / count")
-        if self.fused:
-            # the fused K2+K3 kernel only needs the labels packed and counted (its row phase adds the -onehot term)
-            check(lib.lc2is_pack_labels(ptr(labels), labels.numel(), C, self.ignore_index, ptr(self.labels_packed),
-                                        ptr(blk.n_valid), st), "pack_labels")
-        elif self.split:
-            # un-scaled gradients accumulate into grad_low (prepass: -onehot, K2: +softmax); 1/N_valid is applied
-            # by K1b, so the valid-count all-reduce hides behind K0 / K1 / K2
-            check(lib.lc2is_ce_labels_prepass(ptr(labels), B, C, h, w, H, W, self.ignore_index,
-                                              ptr(self.labels_packed), ptr(blk.n_valid), glow, st), "ce_labels_prepass")
-        else:
-            check(lib.lc2is_count_valid(ptr(labels), labels.numel(), C, self.ignore_index, ptr(blk.n_valid), st),
-                  "count_valid")
+        # un-scaled gradients accumulate into grad_low on the split routes; 1/N_valid is applied by K1b, so the
+        # valid-count all-reduce hides behind K0 / K1 / K2
+        check(lib.lc2is_step_ce_labels(ptr(labels), B, C, h, w, H, W, self.ignore_index, ptr(self.labels_packed),
+                                       ptr(blk.n_valid), glow, stream_ptr()), "step_ce_labels")
 
     def _fuse(self, v) -> bool:
         return self.fuse_norm and v.dtype == torch.bfloat16
@@ -316,16 +308,8 @@ class HeadStep:
         self._mark("K2 upsample+CE")
         if self.k2_events is not None:
             self.k2_events[0].record()
-        if self.fused:
-            check(lib.lc2is_ce_argmax_fused_packed(ptr(self.logits), ptr(self.labels_packed), B, C, h, w, H, W,
-                                                   ptr(blk.loss_sum), glow, 1, None, ptr(self.confmat), None, None, st),
-                  "ce_argmax_fused_packed")
-        elif self.split:
-            check(lib.lc2is_upsample_ce_packed(ptr(self.logits), ptr(self.labels_packed), B, C, h, w, H, W,
-                                               ptr(blk.loss_sum), glow, st), "upsample_ce_packed")
-        else:
-            check(lib.lc2is_upsample_ce_fwd_bwd(ptr(self.logits), ptr(labels), B, C, h, w, H, W, self.ignore_index,
-                                                None, ptr(blk.loss_sum), glow, None, st), "upsample_ce_fwd_bwd")
+        check(lib.lc2is_step_ce(ptr(self.logits), ptr(labels), ptr(self.labels_packed), B, C, h, w, H, W,
+                                self.ignore_index, ptr(blk.loss_sum), glow, ptr(self.confmat), st), "step_ce")
         if self.k2_events is not None:
             self.k2_events[1].record()
 
@@ -350,14 +334,8 @@ class HeadStep:
                                                  _lib.BWD_RAW_V if fuse else 0),
                   "cosine_logits_bwd")
         self._mark("K3 argmax+confmat")
-        if self.fused:
-            pass                                                  # done inside the fused kernel
-        elif self.split:
-            check(lib.lc2is_argmax_confmat_lowres_packed(ptr(self.logits), B, C, h, w, H, W, ptr(self.labels_packed),
-                                                         ptr(self.confmat), None, None, st), "argmax_confmat_packed")
-        else:
-            check(lib.lc2is_argmax_confmat_lowres(ptr(self.logits), B, C, h, w, H, W, BILINEAR, ptr(labels), H, W,
-                                                  ptr(self.confmat), None, None, st), "argmax_confmat_lowres")
+        check(lib.lc2is_step_argmax(ptr(self.logits), ptr(labels), ptr(self.labels_packed), B, C, h, w, H, W,
+                                    ptr(self.confmat), st), "step_argmax")       # (nothing on the fused route)
         self._mark("finalize")
         if self.distributed:
             blk.bucket.views[1].copy_(blk.loss_sum)              # fp32 copy of the loss sum rides in the bucket
