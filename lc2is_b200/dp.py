@@ -82,7 +82,8 @@ def allreduce_confmat_(confmat: Tensor) -> Tensor:
 
 
 def gather_per_image(per_image: Tensor, counts: Sequence[int]) -> Tensor:
-    """All-gather ragged per-image stats [n_local,3,C] -> [N,3,C] in rank order."""
+    """All-gather ragged per-image stats [n_local,3,C] -> [N,3,C] in rank order (any tensor ragged in dim 0;
+    `counts` are every rank's first dimensions)."""
     if not is_dist():
         return per_image
     world = dist.get_world_size()
@@ -94,17 +95,35 @@ def gather_per_image(per_image: Tensor, counts: Sequence[int]) -> Tensor:
     return torch.cat([o[:c] for o, c in zip(out, counts)], dim=0)
 
 
-class GradBucket:
-    """One flat fp32 buffer holding views of every head gradient, all-reduced with a single call."""
+def gather_ragged(t: Optional[Tensor], device) -> Optional[Tensor]:
+    """All-gather tensors that differ in their first dimension -> their concatenation in rank order, on every rank.
+    A rank may hold nothing (`t=None`, e.g. an empty evaluation shard): it still enters every collective, learning the
+    trailing shape and dtype from the others.  Returns None when no rank holds a tensor.  `device` is where the
+    collective runs (CUDA for NCCL)."""
+    world = dist.get_world_size()
+    metas = [None] * world
+    dist.all_gather_object(metas, None if t is None else (t.shape[0], tuple(t.shape[1:]), t.dtype))
+    known = [m for m in metas if m is not None]
+    if not known:
+        return None
+    _, tail, dtype = known[0]
+    local = t.to(device) if t is not None else torch.empty((0,) + tail, dtype=dtype, device=device)
+    return gather_per_image(local, [m[0] if m is not None else 0 for m in metas])
 
-    def __init__(self, shapes: Iterable[Sequence[int]], device, flat: Optional[Tensor] = None) -> None:
+
+class GradBucket:
+    """One flat buffer (fp32 unless `dtype` says otherwise) holding views of every head gradient, all-reduced with a
+    single call."""
+
+    def __init__(self, shapes: Iterable[Sequence[int]], device, flat: Optional[Tensor] = None,
+                 dtype: torch.dtype = torch.float32) -> None:
         self.shapes = [tuple(s) for s in shapes]
         self.sizes = [int(torch.Size(s).numel()) for s in self.shapes]
-        # `flat`: optional caller-owned fp32 storage of exactly the bucket's size (e.g. a slice of a larger
+        # `flat`: optional caller-owned storage of exactly the bucket's size (e.g. a slice of a larger
         # buffer that is zeroed in one go)
         if flat is not None:
-            assert flat.dtype == torch.float32 and flat.numel() == sum(self.sizes) and flat.is_contiguous()
-        self.flat = flat if flat is not None else torch.zeros(sum(self.sizes), dtype=torch.float32, device=device)
+            assert flat.dtype == dtype and flat.numel() == sum(self.sizes) and flat.is_contiguous()
+        self.flat = flat if flat is not None else torch.zeros(sum(self.sizes), dtype=dtype, device=device)
         self.views: List[Tensor] = []
         o = 0
         for s, n in zip(self.shapes, self.sizes):

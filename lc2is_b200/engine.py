@@ -2,19 +2,28 @@
 loop shape: ``train`` / ``train_loop`` / ``evaluate`` / ``eval_loop`` / ``log`` / ``save`` / ``should_*``,
 engine.py:14-208) - SURVEY 8f-4.  What changes, and only this:
 
-* **one process per GPU** (torchrun): every rank iterates its own shard of the loaders; after ``loss.backward()``
-  (engine.py:100) the gradients - which live as views of ONE flat fp32 bucket, so there is nothing to pack - are summed
-  with a single NCCL all-reduce and divided by the world size (engine.py has no such step: single device,
-  engine.py:17,29-31); progress bars, wandb and checkpoints are rank 0's business only.
+* **one process per GPU** (torchrun): the constructor broadcasts rank 0's parameters and buffers; every rank iterates
+  its own shard of the loaders, and the ranks' j-th batches together are the j-th batch of the single-process run.  Each
+  loss term is scaled by local / global denominator before ``loss.backward()`` (engine.py:100): the denominator of a
+  term is what its ``'mean'`` divides by (the targets that are not ``ignore_index``; the summed ``weight[target]`` of
+  those when the criterion has class weights; 1 for ``reduction='sum'``, whose term is not scaled; the batch size for a
+  criterion without ``reduction`` / ``ignore_index`` attributes), all-reduced in one small collective.  The gradients -
+  views of ONE flat bucket, so there is nothing to pack - are then summed with a single all-reduce, which gives the
+  gradient of the global-batch loss however the shards differ in size or in ignored pixels (engine.py has no such step:
+  single device, engine.py:17,29-31).  Logged losses are global-batch values; progress bars, wandb and checkpoints are
+  rank 0's business only.  Every rank must run the same number of training steps (checked when ``train`` starts);
+  evaluation shards may differ, down to empty ones.
 * **online evaluation**: the reference concatenates every batch's ``outputs`` on the CPU (``torch.concat`` inside the
   loop, O(n^2) copies, engine.py:162-163) and hands the tensor to ``compute_metrics``.  Here each batch goes through K3
   on the device (bicubic x4 + argmax + confusion matrix + per-image counts, metrics.py:84-101) and only integers
   accumulate; at the end of the pass ONE int64 all-reduce sums the confusion matrix over the ranks and the per-image
-  statistics are all-gathered.  ``online_metrics=False`` keeps the reference behaviour (lists, one concat at the end)
-  for a user-supplied ``compute_metrics(outputs=..., labels=...)``.
+  statistics are all-gathered.  ``online_metrics=False`` keeps the reference behaviour (lists, one concat at the end,
+  gathered from every rank) for a user-supplied ``compute_metrics(outputs=..., labels=...)``; it is the default when
+  ``compute_metrics`` is given.
 * **CUDA-graph step** (``cuda_graph=True``, static shapes): forward + criterion + backward of a training step are
   captured once after three eager warm-up steps and replayed from static input buffers; the bucket all-reduce and the
-  optimizer step stay outside the graph.
+  optimizer step stay outside the graph, and the loss-term scales are static inputs of it.  A batch whose shapes differ
+  from the first batch's (a short last batch) runs eagerly.
 
 PyTorch is plumbing here (modules, autograd, optimizers, ``torch.distributed``); the head kernels are the mirrors in
 ``lc2is_b200.model`` / ``lc2is_b200.metrics`` that the model and the criteria are built from.
@@ -30,6 +39,25 @@ import torch.distributed as dist
 from torch import nn
 
 from . import dp
+
+_TERMS = ("loss", "aux_loss")          # the logged loss terms: criterion on "outputs", aux_criterion on "low_score_map"
+
+
+def _local_denominator(crit, labels: torch.Tensor) -> torch.Tensor:
+    """float64 scalar: what `crit`'s 'mean' divides the summed losses of this batch by (see the module docstring)."""
+    reduction, ii = getattr(crit, "reduction", None), getattr(crit, "ignore_index", None)
+    if reduction == "sum":
+        return torch.ones((), dtype=torch.float64, device=labels.device)
+    if reduction is None or ii is None:
+        return torch.full((), float(labels.shape[0]), dtype=torch.float64, device=labels.device)
+    counted = labels != ii
+    weight = getattr(crit, "weight", None)
+    if weight is None:
+        return counted.sum().double()
+    C = weight.numel()
+    counted &= (labels >= 0) & (labels < C)
+    w = weight.detach().double()[labels.clamp(0, C - 1)]
+    return torch.where(counted, w, torch.zeros_like(w)).sum()
 
 
 class _NoBar:
@@ -57,7 +85,7 @@ class Engine:
                  max_epoch: int = 1, max_steps: Optional[int] = None, eval_step: Optional[int] = None,
                  log_step: Optional[int] = None, save_step: Optional[int] = None,
                  out_dir: str = "./", logger: Optional[str] = "wandb", logger_args: Optional[dict] = None,
-                 *, online_metrics: bool = True, n_cls: Optional[int] = None, ignore_index: Optional[int] = 0,
+                 *, online_metrics: Optional[bool] = None, n_cls: Optional[int] = None, ignore_index: Optional[int] = 0,
                  cuda_graph: bool = False) -> None:
         self.name = name
         self.model, self.optimizer, self.criterion, self.lr_scheduler = model, optimizer, criterion, lr_scheduler
@@ -80,6 +108,11 @@ class Engine:
         self.rank = dist.get_rank() if self.distributed else 0
         self.world = dist.get_world_size() if self.distributed else 1
         self.is_main = self.rank == 0
+        if self.distributed:
+            for t in [*self.model.parameters(), *self.model.buffers()]:
+                dist.broadcast(t.data, src=0)                       # replicas start from rank 0's state
+        if online_metrics is None:
+            online_metrics = compute_metrics is None                # a compute_metrics passed in is called
         self.online_metrics, self.n_cls, self.ignore_index = online_metrics, n_cls, ignore_index
         self.cuda_graph = cuda_graph
         self._graph = None
@@ -93,11 +126,11 @@ class Engine:
         params = [p for p in self.model.parameters() if p.requires_grad]
         if not params:
             return
-        dev = params[0].device
-        self._bucket = dp.GradBucket([tuple(p.shape) for p in params], dev)
+        dev, dtype = params[0].device, params[0].dtype
+        if dtype not in (torch.float32, torch.float64) or any(p.dtype != dtype for p in params):
+            raise TypeError("the gradient bucket holds one dtype, fp32 or fp64: keep fp32 master parameters")
+        self._bucket = dp.GradBucket([tuple(p.shape) for p in params], dev, dtype=dtype)
         for p, v in zip(params, self._bucket.views):
-            if p.dtype != torch.float32:
-                raise TypeError("the gradient bucket is fp32: keep fp32 master parameters")
             p.grad = v                                              # autograd accumulates in place into the bucket
 
     def _zero_grad(self) -> None:
@@ -108,8 +141,31 @@ class Engine:
 
     def _allreduce_grads(self) -> None:
         if self.distributed and self._bucket is not None:
-            self._bucket.allreduce_()
-            self._bucket.flat.div_(self.world)
+            self._bucket.allreduce_()                               # a plain sum: the terms carry their scales
+
+    def _crit(self, key: str):
+        return self.aux_criterion if key.endswith("aux_loss") else self.criterion
+
+    def _summed(self, key: str) -> bool:
+        return getattr(self._crit(key), "reduction", None) == "sum"
+
+    def _local_denominators(self, keys, labels: torch.Tensor) -> torch.Tensor:
+        return torch.stack([_local_denominator(self._crit(k), labels) for k in keys])
+
+    def _denominators(self, keys, labels: torch.Tensor):
+        """Distributed only: (float64 [n] this rank's denominator of each term, float64 [n] the scale local / global of
+        each term's loss - 1 for a summed term).  The one collective of a step before backward."""
+        den = self._local_denominators(keys, labels)
+        tot = den.clone()
+        dist.all_reduce(tot)
+        scale = den / torch.where(tot > 0, tot, torch.ones_like(tot))
+        summed = torch.tensor([self._summed(k) for k in keys], device=den.device)
+        return den, torch.where(summed, torch.ones_like(scale), scale)
+
+    @staticmethod
+    def _total(losses: dict, scales: Optional[torch.Tensor]) -> torch.Tensor:
+        terms = torch.stack([v for v in losses.values()])
+        return (terms if scales is None else terms * scales.to(terms.dtype)).sum()
 
     # ---- one training step (engine.py:83-101) ----------------------------------------------------------------
     def _forward_losses(self, inputs: dict, labels: torch.Tensor) -> dict:
@@ -119,60 +175,73 @@ class Engine:
             losses.update(dict(train_aux_loss=self.aux_criterion(outputs_dict["low_score_map"], labels) * 0.4))
         return losses
 
-    def _step_eager(self, inputs: dict, labels: torch.Tensor) -> dict:
+    def _step_eager(self, inputs: dict, labels: torch.Tensor):
+        """-> (losses, local denominators or None)"""
         self._zero_grad()
+        den = scales = None
         if self.fp16:
             with torch.autocast(device_type=str(self.device).split(":")[0], dtype=torch.float16):
                 losses = self._forward_losses(inputs, labels)
-                loss = torch.stack([v for v in losses.values()]).sum()
+                if self.distributed:
+                    den, scales = self._denominators(losses, labels)
+                loss = self._total(losses, scales)
             self.scaler.scale(loss).backward()
             self._allreduce_grads()
             self.scaler.step(self.optimizer)
             self.scaler.update()
         else:
             losses = self._forward_losses(inputs, labels)
-            loss = torch.stack([v for v in losses.values()]).sum()
-            loss.backward()
+            if self.distributed:
+                den, scales = self._denominators(losses, labels)
+            self._total(losses, scales).backward()
             self._allreduce_grads()
             self.optimizer.step()
-        return losses
+        return losses, den
 
-    def _step_graphed(self, inputs: dict, labels: torch.Tensor) -> dict:
-        """Static-shape step: three eager steps, then forward + criteria + backward replayed from one CUDA graph."""
+    def _step_graphed(self, inputs: dict, labels: torch.Tensor):
+        """Static-shape step: three eager steps, then forward + criteria + backward replayed from one CUDA graph.
+        Batches whose shapes differ from the first batch's run eagerly."""
         g = self._graph
+        shapes = (sorted((k, v.shape, v.dtype) for k, v in inputs.items()), labels.shape, labels.dtype)
         if g is None:
             # warm-up AND capture run on one side stream: autograd's AccumulateGrad nodes remember the stream they
             # were created on, and a node created on the default stream breaks the capture
-            self._graph = g = dict(warm=0, stream=torch.cuda.Stream())
+            self._graph = g = dict(warm=0, stream=torch.cuda.Stream(), shapes=shapes)
         if self.fp16:
             return self._step_eager(inputs, labels)
         side, cur = g["stream"], torch.cuda.current_stream()
-        if g["warm"] < 3:
-            g["warm"] += 1
+        if g["warm"] < 3 or shapes != g["shapes"]:
+            g["warm"] += shapes == g["shapes"]
             side.wait_stream(cur)
             with torch.cuda.stream(side):
-                losses = self._step_eager(inputs, labels)
+                out = self._step_eager(inputs, labels)
             cur.wait_stream(side)
-            return losses
+            g["keys"] = list(out[0])
+            return out
         if "graph" not in g:
             g["inputs"] = {k: v.clone() for k, v in inputs.items()}
             g["labels"] = labels.clone()
+            g["scales"] = torch.ones(len(g["keys"]), dtype=torch.float64, device=labels.device)
             side.wait_stream(cur)
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.stream(side):
                 with torch.cuda.graph(graph, stream=side, capture_error_mode="thread_local"):
                     self._bucket.zero_()
                     losses = self._forward_losses(g["inputs"], g["labels"])
-                    torch.stack([v for v in losses.values()]).sum().backward()
+                    self._total(losses, g["scales"]).backward()
             cur.wait_stream(side)
             g["graph"], g["losses"] = graph, losses
+        den = None
+        if self.distributed:
+            den, scales = self._denominators(g["keys"], labels)
+            g["scales"].copy_(scales)
         for k, v in inputs.items():
             g["inputs"][k].copy_(v, non_blocking=True)
         g["labels"].copy_(labels, non_blocking=True)
         g["graph"].replay()
         self._allreduce_grads()
         self.optimizer.step()
-        return {k: v.detach().clone() for k, v in g["losses"].items()}
+        return {k: v.detach().clone() for k, v in g["losses"].items()}, den
 
     # ---- reference loop shape ----------------------------------------------------------------------------------
     def train(self):
@@ -185,10 +254,20 @@ class Engine:
                 self._wandb = wandb
             except Exception:  # noqa: BLE001  (no wandb offline: keep training, log to the progress bar only)
                 self._wandb = None
+        if self.distributed:
+            # every training step all-reduces: ranks that disagree on the step count would wait on each other forever
+            n = torch.tensor([self.steps_in_epoch, self.train_steps], device=self._comm_device())
+            ext = torch.cat([n, -n])
+            dist.all_reduce(ext, op=dist.ReduceOp.MAX)
+            hi, lo = ext[:2], -ext[2:]
+            if not torch.equal(lo, hi):
+                raise RuntimeError(f"rank {self.rank}: the ranks disagree on the number of training steps (batches per "
+                                   f"epoch {int(-lo[0])}..{int(hi[0])}, steps {int(-lo[1])}..{int(hi[1])}); every rank "
+                                   f"must get a train_loader of the same length")
         self.train_progress = _bar(self.train_steps, "Training", self.is_main)
         self.stop_train, self.train_step = False, 0
         self.train_metrics, self.eval_metrics = {}, {}
-        self.all_train_metrics = {}
+        self.all_train_metrics = []
         if self.fp16:
             self.scaler = torch.amp.GradScaler("cuda")
         metrics, save_path = {}, None
@@ -206,13 +285,12 @@ class Engine:
             inputs, metas = data
             inputs = {k: v.to(self.device, non_blocking=True) for k, v in inputs.items()}
             labels = inputs.pop("label")
-            losses_dict = self._step_graphed(inputs, labels) if self.cuda_graph else self._step_eager(inputs, labels)
+            losses_dict, den = (self._step_graphed if self.cuda_graph else self._step_eager)(inputs, labels)
             if self.lr_scheduler is not None:
                 self.lr_scheduler.step()
             self.train_progress.update()
-            # (device scalars: converted to Python numbers when they are logged, not every step)
-            for k, v in losses_dict.items():
-                self.all_train_metrics.setdefault(k, []).append(v.detach())
+            # (device rows: converted to Python numbers when they are logged, not every step)
+            self.all_train_metrics.append(self._loss_row("train_", losses_dict, den))
             eval_metrics = self.should_eval()
             log_metrics = self.should_log()
             save_path = self.should_save()
@@ -234,7 +312,7 @@ class Engine:
         from . import ops
         self.model.eval()
         eval_progress = _bar(len(self.eval_loader), "Evaluation", self.is_main, leave=False)
-        self.all_eval_metrics = {}
+        self.all_eval_metrics = []
         outs, labs = [], []
         confmat, per_image = None, []
         for data in self.eval_loader:
@@ -246,9 +324,9 @@ class Engine:
                 losses_dict = dict(eval_loss=self.criterion(outputs_dict["outputs"], labels))
                 if "low_score_map" in outputs_dict.keys():
                     losses_dict.update(dict(eval_aux_loss=self.aux_criterion(outputs_dict["low_score_map"], labels) * 0.4))
+                den = self._local_denominators(losses_dict, labels) if self.distributed else None
             eval_progress.update()
-            for k, v in losses_dict.items():
-                self.all_eval_metrics.setdefault(k, []).append(v.detach())
+            self.all_eval_metrics.append(self._loss_row("eval_", losses_dict, den))
             out = outputs_dict["outputs"]
             if self.online_metrics:
                 # metrics.py:84-101 per batch on the device: only integers survive the batch
@@ -260,25 +338,67 @@ class Engine:
                 outs.append(out.cpu())
                 labs.append(labels.cpu())
         eval_progress.close()
-        eval_metrics = {k: self._mean_over_ranks(v) for k, v in self.all_eval_metrics.items()}
+        eval_metrics = self._global_losses("eval_", self.all_eval_metrics)
+        # every rank enters every collective below, whatever its shard held (an empty shard included)
         if self.online_metrics:
             pi = torch.cat(per_image) if per_image else None
-            if self.distributed and confmat is not None:
-                dp.allreduce_confmat_(confmat)                       # ONE int64 all-reduce for the pass
-                counts = [torch.zeros(1, dtype=torch.int64, device=confmat.device) for _ in range(self.world)]
-                dist.all_gather(counts, torch.tensor([pi.shape[0]], dtype=torch.int64, device=confmat.device))
-                pi = dp.gather_per_image(pi, [int(c) for c in counts])
+            if self.distributed:
+                pi = dp.gather_ragged(pi, self._comm_device())
+                if pi is not None:
+                    if confmat is None:
+                        C = pi.shape[-1]
+                        confmat = torch.zeros(C, C, dtype=torch.int64, device=pi.device)
+                    dp.allreduce_confmat_(confmat)                   # ONE int64 all-reduce for the pass
             eval_outputs = dict(confmat=confmat, per_image=pi)
         else:
-            eval_outputs = dict(outputs=torch.cat(outs), labels=torch.cat(labs))      # ONE concat, not one per batch
+            outputs = torch.cat(outs) if outs else None                # ONE concat, not one per batch
+            labels = torch.cat(labs) if labs else None
+            if self.distributed:
+                outputs, labels = (dp.gather_ragged(t, self._comm_device()) for t in (outputs, labels))
+                outputs, labels = (None if t is None else t.cpu() for t in (outputs, labels))
+            eval_outputs = dict(outputs=outputs, labels=labels)
         return eval_metrics, eval_outputs
 
-    def _mean_over_ranks(self, values) -> float:
-        t = torch.stack([v.float().reshape(()) for v in values])
-        s = torch.stack([t.sum(), torch.tensor(float(t.numel()), device=t.device)])
+    def _comm_device(self) -> torch.device:
+        return torch.device(self.device)
+
+    def _loss_row(self, prefix: str, losses: dict, den: Optional[torch.Tensor]) -> torch.Tensor:
+        """float64 [len(_TERMS), 3] of one batch: (numerator, denominator, present) of each term.  Single process:
+        (loss, 1).  Distributed: (loss * local denominator, local denominator), so that the sums over the ranks give the
+        global-batch value numerator / denominator; a summed term keeps (loss, 1) and its global value is the sum."""
+        rows, dev = [], next(iter(losses.values())).device
+        for name in _TERMS:
+            key = prefix + name
+            if key not in losses:
+                rows.append(torch.zeros(3, dtype=torch.float64, device=dev))
+                continue
+            v = losses[key].detach().double().reshape(())
+            d = torch.ones_like(v)
+            if den is not None and not self._summed(key):
+                d = den[list(losses).index(key)]
+                v = torch.where(d > 0, v * d, torch.zeros_like(v))  # a shard with nothing counted adds 0, not NaN
+            rows.append(torch.stack([v, d, torch.ones_like(v)]))
+        return torch.stack(rows)
+
+    def _global_losses(self, prefix: str, rows: list) -> dict:
+        """Mean over batches of the global-batch value of each term (the ranks' j-th batches together are batch j of
+        the single-process run).  Ranks may hold different numbers of batches, none included."""
+        n = len(rows)
+        t = torch.stack(rows) if rows else torch.zeros(0, len(_TERMS), 3, dtype=torch.float64,
+                                                        device=self._comm_device())
         if self.distributed:
-            dist.all_reduce(s)
-        return float(s[0] / s[1])
+            m = torch.tensor([n], device=t.device)
+            dist.all_reduce(m, op=dist.ReduceOp.MAX)
+            t = torch.cat([t, t.new_zeros(int(m) - n, len(_TERMS), 3)])
+            dist.all_reduce(t)
+        out = {}
+        for i, name in enumerate(_TERMS):
+            num, den, present = t[:, i].unbind(-1)
+            sel = present > 0
+            if bool(sel.any()):
+                key = prefix + name
+                out[key] = float((num[sel] if self._summed(key) else num[sel] / den[sel]).mean())
+        return out
 
     def _metrics_from_stats(self, stats: dict) -> dict:
         from . import metrics as M
@@ -292,7 +412,7 @@ class Engine:
 
     def log(self) -> dict:
         train_epoch = round(self.train_step / self.steps_in_epoch, 4) if self.steps_in_epoch else 0.0
-        train_metrics = {k: self._mean_over_ranks(v) for k, v in self.all_train_metrics.items()}
+        train_metrics = self._global_losses("train_", self.all_train_metrics)
         metrics = {**dict(train_step=self.train_step, train_epoch=train_epoch), **train_metrics, **self.eval_metrics}
         if self.is_main:
             self.train_progress.set_postfix(metrics)
@@ -317,7 +437,7 @@ class Engine:
     def should_log(self) -> dict:
         if self.log_step and (self.train_step % self.log_step) == 0:
             metrics = self.log()
-            self.all_train_metrics = {}
+            self.all_train_metrics = []
             return metrics
         return {}
 
