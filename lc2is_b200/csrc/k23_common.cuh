@@ -52,8 +52,8 @@ template <int S>
 __device__ __noinline__ float slow_ce_row(const SlowCtx P, int n, int ky, int kx, int i, unsigned vm) {
     const int C = P.C;
     const size_t plane = (size_t)P.h * P.w;
-    const int Ya = clampi2(ky, 0, P.h - 1), Yb = clampi2(ky + 1, 0, P.h - 1);
-    const int Xa = clampi2(kx, 0, P.w - 1), Xb = clampi2(kx + 1, 0, P.w - 1);
+    const int Ya = clampi(ky, 0, P.h - 1), Yb = clampi(ky + 1, 0, P.h - 1);
+    const int Xa = clampi(kx, 0, P.w - 1), Xb = clampi(kx + 1, 0, P.w - 1);
     const float* b = P.low + (size_t)n * C * plane;
     const int oA = Ya * P.w + Xa, oB = Ya * P.w + Xb, oC = Yb * P.w + Xa, oD = Yb * P.w + Xb;
     float* gb = P.grad ? P.grad + (size_t)n * C * plane : nullptr;

@@ -213,8 +213,8 @@ k23_rc_kernel(const __grid_constant__ CUtensorMap tm, const __grid_constant__ RC
         bool bad = false;
         {
             const int xs = rc_xs(J), ys = rc_ys(J);
-            const int ya = (clampi2(ky, 0, P.h - 1) - ys) * 8, yb = (clampi2(ky + 1, 0, P.h - 1) - ys) * 8;
-            const int xa = clampi2(kx, 0, P.w - 1) - xs, xb = clampi2(kx + 1, 0, P.w - 1) - xs;   // 0..4
+            const int ya = (clampi(ky, 0, P.h - 1) - ys) * 8, yb = (clampi(ky + 1, 0, P.h - 1) - ys) * 8;
+            const int xa = clampi(kx, 0, P.w - 1) - xs, xb = clampi(kx + 1, 0, P.w - 1) - xs;   // 0..4
             for (int k = lane; k < CP + 4; k += 32) {     // (+4: the rescan of a 4-class last chunk reads 8 classes)
                 const float* cp = cells + k * 16;
                 float4 q;
@@ -425,8 +425,8 @@ k23_rc_kernel(const __grid_constant__ CUtensorMap tm, const __grid_constant__ RC
 #pragma unroll
                 for (int jj = 0; jj < 8; ++jj) prow[jj] = bidx[jj];
             }
-            const int Ya = clampi2(ky, 0, P.h - 1), Yb = clampi2(ky + 1, 0, P.h - 1);
-            const int Xa = clampi2(kx, 0, P.w - 1), Xb = clampi2(kx + 1, 0, P.w - 1);
+            const int Ya = clampi(ky, 0, P.h - 1), Yb = clampi(ky + 1, 0, P.h - 1);
+            const int Xa = clampi(kx, 0, P.w - 1), Xb = clampi(kx + 1, 0, P.w - 1);
             const int oA = Ya * P.w + Xa, oB = Ya * P.w + Xb, oC = Yb * P.w + Xa, oD = Yb * P.w + Xb;
             const float* lbase = P.low + (size_t)n * C * plane;
             float* gbase = (P.grad && P.onehot) ? P.grad + (size_t)n * C * plane : nullptr;
@@ -516,8 +516,8 @@ k23_rc_kernel(const __grid_constant__ CUtensorMap tm, const __grid_constant__ RC
         // ================= class phase (lane = class): tap gradients by Horner sweeps ==============================
         if (!slow && P.grad != nullptr && any) {
             float* gimg = P.grad + (size_t)n * C * plane;
-            const int oA = clampi2(ky, 0, P.h - 1) * P.w, oC = clampi2(ky + 1, 0, P.h - 1) * P.w;
-            const int cxa = clampi2(kx, 0, P.w - 1), cxb = clampi2(kx + 1, 0, P.w - 1);
+            const int oA = clampi(ky, 0, P.h - 1) * P.w, oC = clampi(ky + 1, 0, P.h - 1) * P.w;
+            const int cxa = clampi(kx, 0, P.w - 1), cxb = clampi(kx + 1, 0, P.w - 1);
             const float Mk = mx * LOG2E;
             // NB blocks of 32 classes per sweep: one broadcast LDS.128 of U then feeds 4 * NB packed fma (with one block
             // the class phase leaned on the shared-memory pipe: 16 LDS.128 per 62 FFMA2, ncu mio_throttle / short

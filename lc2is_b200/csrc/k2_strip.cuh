@@ -20,8 +20,6 @@ __device__ __forceinline__ void cp_async_wait_all() {
 
 constexpr float K2_FAST_RANGE = 40.f;   // max logit range inside a group for the shared-shift fast path
 
-__device__ __forceinline__ int clampi2(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
-
 // ---- packed fp32x2 arithmetic (sm_100: FADD2 / FMUL2 / FFMA2 - two fp32 ops per issue slot) ------
 __device__ __forceinline__ unsigned long long pk2(float2 a) {
     unsigned long long r;
@@ -51,24 +49,23 @@ __device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
 __device__ __forceinline__ float2 bc2(float x) { return make_float2(x, x); }
 
 // Sum (a,b,c,d) over the LPG consecutive lanes of a group.  After the call lane u of the group
-// holds in `a` the total of value number (u * 4 / LPG) [LPG >= 4], i.e. the first quarter of the
-// lanes hold sum(a), the second sum(b), ... ; for LPG == 1 nothing happens.
+// holds in `a` the total of value number (u * 4 / LPG), i.e. the first quarter of the
+// lanes hold sum(a), the second sum(b), ...
 template <int LPG>
 __device__ __forceinline__ void group_reduce4(float& a, float& b, float& c, float& d, int u) {
-    if constexpr (LPG >= 4) {
-        const bool up = u & (LPG / 2);
-        float s0 = up ? a : c, s1 = up ? b : d;          // what this lane gives away
-        float k0 = up ? c : a, k1 = up ? d : b;          // what it keeps
-        k0 += __shfl_xor_sync(0xffffffffu, s0, LPG / 2);
-        k1 += __shfl_xor_sync(0xffffffffu, s1, LPG / 2);
-        const bool up2 = u & (LPG / 4);
-        float g = up2 ? k0 : k1;
-        float k = up2 ? k1 : k0;
-        k += __shfl_xor_sync(0xffffffffu, g, LPG / 4);
+    static_assert(LPG >= 4, "a group spans at least four lanes");
+    const bool up = u & (LPG / 2);
+    float s0 = up ? a : c, s1 = up ? b : d;          // what this lane gives away
+    float k0 = up ? c : a, k1 = up ? d : b;          // what it keeps
+    k0 += __shfl_xor_sync(0xffffffffu, s0, LPG / 2);
+    k1 += __shfl_xor_sync(0xffffffffu, s1, LPG / 2);
+    const bool up2 = u & (LPG / 4);
+    float g = up2 ? k0 : k1;
+    float k = up2 ? k1 : k0;
+    k += __shfl_xor_sync(0xffffffffu, g, LPG / 4);
 #pragma unroll
-        for (int o = LPG / 8; o > 0; o >>= 1) k += __shfl_xor_sync(0xffffffffu, k, o);
-        a = k;
-    }
+    for (int o = LPG / 8; o > 0; o >>= 1) k += __shfl_xor_sync(0xffffffffu, k, o);
+    a = k;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -103,7 +100,6 @@ struct K2SParams {
     long long ignore_index;
     int B, C, h, w, H, W;
     int nty, ntx;                 // warp tiles per image
-    unsigned long long* n_valid;  // SPLIT: += number of counted pixels (null = the caller counted them already)
 };
 // The weighted form's parameters (a separate type: K2SParams is copied to the stack for k2_strip_slow, and the unweighted
 // kernels keep their frame): class weights w[C] (null = all 1), 1 - eps and eps / C of the label smoothing eps.
@@ -201,8 +197,7 @@ __device__ __noinline__ float k2_strip_slow(const TQ tq, unsigned vm, int n, int
 // (accumulated in the max-tap sweep) and V = the thread's summed bilinear tap weights of its counted pixels; the
 // gradient takes -g (eps/C) w_c V_cell on the lane that issues the cell's reduction (V merged like the gradients).
 template <int S, bool SPLIT, int CSF, bool GTAPS = false, bool WT = false>
-__device__ __forceinline__ void k2_strip_warp(const K2SP<WT>& P, float* st, bool active, int n, int GY0,
-                                              int GX0, int lane) {
+__device__ __forceinline__ void k2_strip_warp(const K2SP<WT>& P, float* st, int n, int GY0, int GX0, int lane) {
     static_assert(!(WT && SPLIT), "the weighted form is one-call only");
     constexpr int TPG = S / 2;                              // threads (lanes) per group
     constexpr int GPW = 32 / TPG;                           // groups per warp: 4 (S=16) / 8 (S=8)
@@ -217,7 +212,7 @@ __device__ __forceinline__ void k2_strip_warp(const K2SP<WT>& P, float* st, bool
     // ---- this thread's strip ------------------------------------------------------------------------------
     const int gl = lane / TPG, u = lane % TPG;
     const int ky = GY0 + gl / WGX - 1, kx = GX0 + gl % WGX - 1;   // top-left tap of the group (-1 .. h-1)
-    const bool group_in = active && ky < P.h && kx < P.w;
+    const bool group_in = ky < P.h && kx < P.w;
     const int y0 = S * ky + S / 2 + 2 * u, x0 = S * kx + S / 2;
     const float gs = P.grad_scale ? __ldg(P.grad_scale) : 1.f;
 
@@ -271,18 +266,9 @@ __device__ __forceinline__ void k2_strip_warp(const K2SP<WT>& P, float* st, bool
     }
     cp_async_wait_all();
     __syncwarp();
-    if (!active) return;                                    // (after the barrier)
-    if constexpr (SPLIT) {
-        if (P.n_valid != nullptr) {                             // valid count of the warp's strips: one reduction per warp
-            int cnt = __popc(vm);
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-            if (lane == 0 && cnt) atomicAdd(P.n_valid, (unsigned long long)cnt);
-        }
-    }
 
-    const int Ya = clampi2(ky, 0, P.h - 1), Yb = clampi2(ky + 1, 0, P.h - 1);
-    const int Xa = clampi2(kx, 0, P.w - 1), Xb = clampi2(kx + 1, 0, P.w - 1);
+    const int Ya = clampi(ky, 0, P.h - 1), Yb = clampi(ky + 1, 0, P.h - 1);
+    const int Xa = clampi(kx, 0, P.w - 1), Xb = clampi(kx + 1, 0, P.w - 1);
     float* gb = P.grad_low ? P.grad_low + (size_t)n * C * plane : nullptr;
     float* gA = gb ? gb + (size_t)Ya * P.w + Xa : nullptr; float* gB = gb ? gb + (size_t)Ya * P.w + Xb : nullptr;
     float* gC = gb ? gb + (size_t)Yb * P.w + Xa : nullptr; float* gD = gb ? gb + (size_t)Yb * P.w + Xb : nullptr;
@@ -512,7 +498,7 @@ __device__ __forceinline__ void k2_strip_warp(const K2SP<WT>& P, float* st, bool
             const int cy = gy_ + ry, cx = gx_ + rx;                                // cell of the warp tile
             const int uy = GY0 - 1 + cy, ux = GX0 - 1 + cx;                        // unclamped source cell
             float* dst = (holder && uy <= P.h && ux <= P.w)
-                             ? gb + (size_t)clampi2(uy, 0, P.h - 1) * P.w + clampi2(ux, 0, P.w - 1) : nullptr;
+                             ? gb + (size_t)clampi(uy, 0, P.h - 1) * P.w + clampi(ux, 0, P.w - 1) : nullptr;
             const float2 omy = make_float2(1.f - ly2.x, 1.f - ly2.y);
             float kv = 0.f;                                  // WT: -g (eps/C) V of this lane's source cell
             if constexpr (WT) {

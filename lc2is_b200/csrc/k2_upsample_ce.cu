@@ -8,7 +8,7 @@
 // (softmax - onehot) * g back through the four bilinear taps into a shared-memory gradient
 // tile that is flushed once.
 //
-// Fast path (power-of-two scale s >= 4): one thread owns a 4x4 pixel block whose 16 pixels
+// Fast path (scale 4; 8 / 16 take the strip kernels): one thread owns a 4x4 pixel block whose 16 pixels
 // share the same 2x2 taps (common.cuh: BlockGeom).  Inside the block the upsampled logit is a
 // bilinear polynomial  l(i,j) = l00 + i*P + j*Q + i*j*T, so
 //     exp(l(i,j) - M) = E00 * p^i * q^j * t^(i*j)        (4 ex2 per class per 16 pixels,
@@ -87,11 +87,10 @@ __global__ void k2_weight_sum_kernel(const long long* __restrict__ labels, long 
 }
 
 // ---------------------------------------------------------------------------------------------
-// Geometry of the fast path.  A GROUP is the set of bps x bps 4x4-pixel blocks (bps = s/4) that
-// interpolate between the same 2x2 source cells: group (gy,gx) has taps (ky,kx) = (gy-1, gx-1)
-// .. (ky+1, kx+1), index-clamped to the image.  There are (h+1) x (w+1) groups per image.  The
-// bps*bps threads of a group are consecutive lanes of one warp, so their four tap contributions
-// are summed with a butterfly of warp shuffles and leave the SM as four L2 float reductions.
+// Geometry of the fast path (scale 4).  Thread (ty,tx) of a CTA owns the 4x4-pixel block that interpolates between
+// the source cells (ky,kx) = (GY0+ty-1, GX0+tx-1) .. (ky+1, kx+1), index-clamped to the image; there are (h+1) x (w+1)
+// blocks per image.  The CTA stages the (tgy+1) x (tgx+1) source cells its tgy x tgx blocks read, and each thread
+// sends its four tap gradients to L2 as four float reductions per class.
 struct K2Params {
     const float* low;            // [B,C,h,w]
     const long long* labels;     // [B,H,W]
@@ -100,8 +99,8 @@ struct K2Params {
     const float* grad_scale;     // device scalar or null
     long long ignore_index;
     int B, C, h, w, H, W;
-    int s, off, q;                // scale, pixel offset of the block grid, block offset of group 0
-    int tgy, tgx;                 // groups per CTA
+    int s, off, q;                // scale, pixel offset of the block grid, offset of block 0
+    int tgy, tgx;                 // blocks per CTA
     float rs;
     const float* weight;          // WT: class weights [C] (null = all 1); 1 - eps, eps / C (k2_strip.cuh: k2_class_weight)
     float one_m_eps, eps_c;
@@ -126,17 +125,13 @@ __device__ __forceinline__ Poly k2_poly(float a, float b, float cc, float d, flo
 // WT: the weighted / label-smoothed form (k2_strip.cuh: k2_class_weight): U = g*a / S, a*lse, a (1-eps) w_t scale on the
 // -onehot runs, and the smoothing terms through V = the thread's summed tap weights (loss: V.Q with Q = sum_c w_c * taps
 // from the max-tap sweep; gradient: -g (eps/C) w_c V per tap and class).
-template <int BPS, bool WT = false>
+template <bool WT = false>
 __global__ void __launch_bounds__(128)
 k2_fast_kernel(const K2Params P) {
-    constexpr int LPG = BPS * BPS;                          // lanes (threads) per group
-    constexpr bool QUAD = LPG >= 4;                         // tile layout: per-group tap quads vs cells
-    static_assert(!WT || LPG == 1, "the weighted form is instantiated for one thread per group");
     extern __shared__ float smem[];
     const int C = P.C;
-    const int ngr = P.tgy * P.tgx;
     const int ncx = P.tgx + 1, ncy = P.tgy + 1;
-    const int cs = QUAD ? ngr * 4 : ncy * ncx;              // class stride (floats) in the tile
+    const int cs = ncy * ncx;                               // class stride (floats) in the tile
     const int nthr = blockDim.x;
     float* st = smem;
 
@@ -145,26 +140,10 @@ k2_fast_kernel(const K2Params P) {
     const int cy0 = GY0 - 1, cx0 = GX0 - 1;                 // first cell of the tile (may be -1)
     const float* lowb = P.low + (size_t)n * C * P.h * P.w;
 
-    // ---- stage the source tile --------------------------------------------------------------------
-    // QUAD: st[c][group][4] = the group's four index-clamped taps (one LDS.128 per class later);
-    // cells: st[c][ncy][ncx].  Groups / cells outside the image hold 0.
-    if (QUAD) {
-        // cs = 4 * groups divides the 128 threads: thread -> fixed (group, tap), strided over classes
-        const int r = threadIdx.x % cs, cstep = nthr / cs;
-        const int gq = r >> 2, tap = r & 3;
-        const int ty = gq / P.tgx, tx = gq - ty * P.tgx;
-        const int kyy = GY0 + ty - 1, kxx = GX0 + tx - 1;
-        const bool ok = kyy < P.h && kxx < P.w;
-        const int gy = clampi2(kyy + (tap >> 1), 0, P.h - 1), gx = clampi2(kxx + (tap & 1), 0, P.w - 1);
-        const float* src = lowb + (size_t)gy * P.w + gx;
-        const size_t plane = (size_t)P.h * P.w;
-        for (int c = threadIdx.x / cs; c < C; c += cstep) {
-            if (ok) cp_async4(st + c * cs + r, src + (size_t)c * plane);
-            else st[c * cs + r] = 0.f;
-        }
-    } else {
-        // (a thread owns tile cells r, r + nthr, ... and walks the classes: no integer division per copied element - the
-        // staging loop was a third of this kernel's instructions)
+    // ---- stage the source tile st[c][ncy][ncx]; cells outside the image hold 0 ---------------------
+    // (a thread owns tile cells r, r + nthr, ... and walks the classes: no integer division per copied element - the
+    // staging loop was a third of this kernel's instructions)
+    {
         const size_t plane = (size_t)P.h * P.w;
         for (int r = threadIdx.x; r < cs; r += nthr) {
             const int i = r / ncx, j = r - i * ncx;
@@ -183,15 +162,14 @@ k2_fast_kernel(const K2Params P) {
     __syncthreads();
 
     // ---- per-thread block setup ---------------------------------------------------------------------
-    const int g = threadIdx.x / LPG, u = threadIdx.x % LPG;
+    const int g = threadIdx.x;
     const int tgy = g / P.tgx, tgx = g - tgy * P.tgx;
-    const int uy = u / BPS, ux = u % BPS;
-    const int ky = GY0 + tgy - 1, kx = GX0 + tgx - 1;       // top-left tap of the group (-1 .. h-1)
-    const int by = ky * BPS + P.q + uy, bx = kx * BPS + P.q + ux;
+    const int ky = GY0 + tgy - 1, kx = GX0 + tgx - 1;       // top-left tap of the block (-1 .. h-1)
+    const int by = ky + P.q, bx = kx + P.q;
     const int y0 = 4 * by - P.off, x0 = 4 * bx - P.off;
     const float gs = P.grad_scale ? __ldg(P.grad_scale) : 1.f;
     const float rs = P.rs;
-    const bool group_in = ky < P.h && kx < P.w;             // group exists in this image
+    const bool group_in = ky < P.h && kx < P.w;             // block exists in this image
     int lab[16];
     bool any = false;
 #pragma unroll
@@ -208,34 +186,25 @@ k2_fast_kernel(const K2Params P) {
             any |= l >= 0;
         }
     // clamped tap cells (global)
-    const int Ya = clampi2(ky, 0, P.h - 1), Yb = clampi2(ky + 1, 0, P.h - 1);
-    const int Xa = clampi2(kx, 0, P.w - 1), Xb = clampi2(kx + 1, 0, P.w - 1);
+    const int Ya = clampi(ky, 0, P.h - 1), Yb = clampi(ky + 1, 0, P.h - 1);
+    const int Xa = clampi(kx, 0, P.w - 1), Xb = clampi(kx + 1, 0, P.w - 1);
     // tile offsets of the four taps
-    int oa, ob, oc, od;
-    if (QUAD) { oa = g * 4; ob = oa + 1; oc = oa + 2; od = oa + 3; }
-    else {
-        oa = (Ya - cy0) * ncx + (Xa - cx0); ob = (Ya - cy0) * ncx + (Xb - cx0);
-        oc = (Yb - cy0) * ncx + (Xa - cx0); od = (Yb - cy0) * ncx + (Xb - cx0);
-        if (!group_in) oa = ob = oc = od = 0;
-    }
+    int oa = (Ya - cy0) * ncx + (Xa - cx0), ob = (Ya - cy0) * ncx + (Xb - cx0);
+    int oc = (Yb - cy0) * ncx + (Xa - cx0), od = (Yb - cy0) * ncx + (Xb - cx0);
+    if (!group_in) oa = ob = oc = od = 0;
     auto taps = [&](int c, float& a, float& b, float& cc, float& d) {
-        if (QUAD) {
-            const float4 v = *reinterpret_cast<const float4*>(st + (size_t)c * cs + oa);
-            a = v.x; b = v.y; cc = v.z; d = v.w;
-        } else {
-            const float* p = st + (size_t)c * cs;
-            a = p[oa]; b = p[ob]; cc = p[oc]; d = p[od];
-        }
+        const float* p = st + (size_t)c * cs;
+        a = p[oa]; b = p[ob]; cc = p[oc]; d = p[od];
     };
     // lambda of the block's first row / column ((y0+0.5)*rs-0.5-ky is exact for power-of-2 s)
     const float ly0 = ((float)y0 + 0.5f) * rs - 0.5f - (float)ky;
     const float lx0 = ((float)x0 + 0.5f) * rs - 0.5f - (float)kx;
 
-    // ---- softmax shift: M = max over classes of the group's taps (>= every pixel's max) -----------
+    // ---- softmax shift: M = max over classes of the block's taps (>= every pixel's max) -----------
     float mx = -INFINITY, mn = INFINITY;
     float4 wq = make_float4(0.f, 0.f, 0.f, 0.f);            // WT: sum_c w_c * taps
     float wsum = 0.f;                                       // WT: W = sum_c w_c
-    for (int c = u; c < C; c += LPG) {                      // the group's lanes split the classes
+    for (int c = 0; c < C; ++c) {
         float a, b, cc, d;
         taps(c, a, b, cc, d);
         mx = fmaxf(mx, fmaxf(fmaxf(a, b), fmaxf(cc, d)));
@@ -246,13 +215,8 @@ k2_fast_kernel(const K2Params P) {
             wsum += wc;
         }
     }
-#pragma unroll
-    for (int o = LPG / 2; o > 0; o >>= 1) {
-        mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-        mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
-    }
     const float M = mx;
-    // fast path needs a bounded logit range inside the group (no under/overflow of the shared-shift
+    // fast path needs a bounded logit range inside the block (no under/overflow of the shared-shift
     // polynomial); otherwise - or on inf/NaN - the whole warp takes the exact per-pixel path.
     bool slow = any && !((mx - mn) < K2_FAST_RANGE);
     slow = __any_sync(0xffffffffu, slow);
@@ -368,12 +332,7 @@ k2_fast_kernel(const K2Params P) {
     // ---- pass B: scatter softmax * U through the taps (warp-collective) ---------------------------------
     float* gb = P.grad_low ? P.grad_low + (size_t)n * C * P.h * P.w : nullptr;
     if (gb && warp_any) {
-        // which of the four totals this lane writes after the butterfly, and where
-        const int role = QUAD ? (u * 4) / LPG : 0;
-        const bool writer = QUAD ? (u % (LPG / 4)) == 0 : true;
-        const int cellY = (role & 2) ? Yb : Ya, cellX = (role & 1) ? Xb : Xa;
         const size_t plane = (size_t)P.h * P.w;
-        float* gcell = gb + (size_t)cellY * P.w + cellX;
         float* gA = gb + (size_t)Ya * P.w + Xa; float* gB = gb + (size_t)Ya * P.w + Xb;
         float* gC = gb + (size_t)Yb * P.w + Xa; float* gD = gb + (size_t)Yb * P.w + Xb;
         auto emit = [&](int c, float G, float Gx, float Gy, float Gxy) {
@@ -385,10 +344,7 @@ k2_fast_kernel(const K2Params P) {
                 const float wc = k2_class_weight(P.weight, c);
                 A = fmaf(kv.x, wc, A); Bv = fmaf(kv.y, wc, Bv); Cv = fmaf(kv.z, wc, Cv); Dv = fmaf(kv.w, wc, Dv);
             }
-            group_reduce4<LPG>(A, Bv, Cv, Dv, u);
-            if (QUAD) {
-                if (writer) atomicAdd(gcell + (size_t)c * plane, A);
-            } else if (any) {
+            if (any) {
                 atomicAdd(gA + (size_t)c * plane, A);  atomicAdd(gB + (size_t)c * plane, Bv);
                 atomicAdd(gC + (size_t)c * plane, Cv); atomicAdd(gD + (size_t)c * plane, Dv);
             }
@@ -514,7 +470,7 @@ k2_strip_kernel(const K2SP<WT> P) {
         const int gq = r >> 2, tap = r & 3;
         const int kyy = GY0 + gq / WGX - 1, kxx = GX0 + gq % WGX - 1;
         const bool ok = kyy < P.h && kxx < P.w;
-        const int yy = clampi2(kyy + (tap >> 1), 0, P.h - 1), xx = clampi2(kxx + (tap & 1), 0, P.w - 1);
+        const int yy = clampi(kyy + (tap >> 1), 0, P.h - 1), xx = clampi(kxx + (tap & 1), 0, P.w - 1);
         const float* src = lowb + (size_t)yy * P.w + xx;
         float* dst = st + r;
         for (int c = lane / CS; c < C; c += CSTEP) {
@@ -522,7 +478,7 @@ k2_strip_kernel(const K2SP<WT> P) {
             else dst[c * CS] = 0.f;
         }
     }
-    k2_strip_warp<S, SPLIT, CS, false, WT>(P, st, true, n, GY0, GX0, lane);
+    k2_strip_warp<S, SPLIT, CS, false, WT>(P, st, n, GY0, GX0, lane);
 }
 
 // The same strips with the taps read from the class-plane-major map itself (no staged tile): for class counts whose
@@ -538,7 +494,22 @@ k2_strip_gtaps_kernel(const K2SP<WT> P) {
     const int n = (int)(wt / tiles_per_img);
     const int trem = (int)(wt - (long long)n * tiles_per_img);
     const int tyi = trem / P.ntx, txi = trem - tyi * P.ntx;
-    k2_strip_warp<S, SPLIT, CS, true, WT>(P, nullptr, true, n, tyi * 2, txi * WGX, lane);
+    k2_strip_warp<S, SPLIT, CS, true, WT>(P, nullptr, n, tyi * 2, txi * WGX, lane);
+}
+
+// ---------------------------------------------------------------------------------------------
+// n_valid += the CTA's sum of cnt (nwarps <= 8 warps): one 64-bit reduction per CTA, none when n_valid is null.
+__device__ __forceinline__ void k2_block_count(int cnt, int nwarps, unsigned long long* n_valid) {
+    __shared__ int red_c[8];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+    if ((threadIdx.x & 31) == 0) red_c[threadIdx.x >> 5] = cnt;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        long long tc = 0;
+        for (int i = 0; i < nwarps; ++i) tc += red_c[i];
+        if (tc && n_valid) atomicAdd(n_valid, (unsigned long long)tc);
+    }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -570,8 +541,8 @@ k2_labels_prepass_kernel(const LT* __restrict__ labels,
         const int kx = gx - 1, x0 = S * kx + S / 2;
         const int ky = (y + S / 2) / S - 1;
         const int lyi = 2 * (y - (S * ky + S / 2)) + 1;                  // lambda_y * 2S
-        const int Ya = clampi2(ky, 0, h - 1), Yb = clampi2(ky + 1, 0, h - 1);
-        const int Xa = clampi2(kx, 0, w - 1), Xb = clampi2(kx + 1, 0, w - 1);
+        const int Ya = clampi(ky, 0, h - 1), Yb = clampi(ky + 1, 0, h - 1);
+        const int Xa = clampi(kx, 0, w - 1), Xb = clampi(kx + 1, 0, w - 1);
         const size_t oA = (size_t)Ya * w + Xa, oB = (size_t)Ya * w + Xb, oC = (size_t)Yb * w + Xa, oD = (size_t)Yb * w + Xb;
         const LT* row = labels + ((size_t)n * H + y) * W;
         unsigned short* prow = packed ? packed + ((size_t)n * H + y) * W : nullptr;
@@ -656,17 +627,7 @@ k2_labels_prepass_kernel(const LT* __restrict__ labels,
         }
         flush();
     }
-    // block reduction: one 64-bit count reduction per CTA
-    __shared__ int red_c[8];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-    if ((threadIdx.x & 31) == 0) red_c[threadIdx.x >> 5] = cnt;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        long long tc = 0;
-        for (int i = 0; i < (int)(blockDim.x >> 5); ++i) tc += red_c[i];
-        if (tc && n_valid) atomicAdd(n_valid, (unsigned long long)tc);
-    }
+    k2_block_count(cnt, (int)(blockDim.x >> 5), n_valid);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -696,16 +657,7 @@ k2_pack_labels_kernel(const long long* __restrict__ labels, long long n8, int C,
         }
         reinterpret_cast<uint4*>(packed)[i] = make_uint4(w[0], w[1], w[2], w[3]);
     }
-    __shared__ int red_c[8];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-    if ((threadIdx.x & 31) == 0) red_c[threadIdx.x >> 5] = cnt;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        long long tc = 0;
-        for (int i = 0; i < (int)(blockDim.x >> 5); ++i) tc += red_c[i];
-        if (tc && n_valid) atomicAdd(n_valid, (unsigned long long)tc);
-    }
+    k2_block_count(cnt, (int)(blockDim.x >> 5), n_valid);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -871,6 +823,36 @@ extern "C" int lc2is_upsample_ce_fwd_bwd(const float* d_low, const int64_t* d_la
                                         d_loss_sum, d_grad_low, d_grad_low_bf16, stream);
 }
 
+namespace lc2is {
+// The strip kernels (scale s = 8 / 16) over P.B images; sets P.nty / P.ntx.  Warps are independent; a warp's staged
+// tile of taps takes (C + 2) * (32 / (s/2)) * 16 bytes of shared memory, and above K2_GTAPS_SMEM the taps are read from
+// the map itself instead.
+template <bool SPLIT, bool WT>
+static int launch_k2_strip(K2SP<WT> P, int s, cudaStream_t st) {
+    const size_t smem_warp = (size_t)(P.C + 2) * (64 / s) * 16;
+    int wpc = 4;
+    while (wpc > 1 && smem_warp * wpc > 56 * 1024) wpc /= 2;
+    const size_t smem = smem_warp * wpc;
+    const bool gtaps = smem_warp > K2_GTAPS_SMEM;               // staged tile too large for a decent occupancy
+    const int wgx = (64 / s) / 2;
+    P.nty = (P.h + 1 + 1) / 2;
+    P.ntx = (P.w + 1 + wgx - 1) / wgx;
+    const long long tiles = (long long)P.B * P.nty * P.ntx;
+    auto launch = [&](auto kernel, auto kernel_gtaps) -> int {
+        if (gtaps) {
+            kernel_gtaps<<<(unsigned)((tiles + 3) / 4), 128, 0, st>>>(P);
+        } else {
+            LC2IS_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            kernel<<<(unsigned)((tiles + wpc - 1) / wpc), wpc * 32, smem, st>>>(P);
+        }
+        LC2IS_CHECK_LAUNCH(SPLIT ? "k2_strip_kernel(split)" : "k2_strip_kernel");
+        return 0;
+    };
+    return s == 8 ? launch(k2_strip_kernel<8, SPLIT, WT>, k2_strip_gtaps_kernel<8, SPLIT, WT>)
+                  : launch(k2_strip_kernel<16, SPLIT, WT>, k2_strip_gtaps_kernel<16, SPLIT, WT>);
+}
+}  // namespace lc2is
+
 extern "C" int lc2is_upsample_ce_fwd_bwd_ex(const float* d_low, const int64_t* d_labels,
                                             int B, int C, int h, int w, int H, int W,
                                             int64_t ignore_index, const float* d_weight, float label_smoothing,
@@ -887,51 +869,22 @@ extern "C" int lc2is_upsample_ce_fwd_bwd_ex(const float* d_low, const int64_t* d
     if (!d_low || !d_labels || !d_loss_sum) return fail(LC2IS_ERR_ARG, "null pointer%s");
     if (d_grad_low_bf16 && !d_grad_low)
         return fail(LC2IS_ERR_ARG, "grad_low_bf16 needs the fp32 grad_low buffer as well%s");
-    if (B == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
     if (d_grad_low) LC2IS_CUDA(cudaMemsetAsync(d_grad_low, 0, (size_t)B * C * h * w * sizeof(float), st));
 
     int s = 0;
     bool fast = fast_scale(h, w, H, W, &s) && s <= 16;
-    // ---- strip path: s = 8 / 16 -----------------------------------------------------------------------
     if (fast && s >= 8 && ((uintptr_t)d_labels % 16) == 0) {
+        // ---- strip path: s = 8 / 16 -----------------------------------------------------------------------
         K2SParamsW PW;
         K2SParams& P = PW;
-        P.low = d_low; P.labels = (const long long*)d_labels; P.labels16 = nullptr; P.n_valid = nullptr; P.grad_low = d_grad_low;
+        P.low = d_low; P.labels = (const long long*)d_labels; P.labels16 = nullptr; P.grad_low = d_grad_low;
         P.loss_sum = d_loss_sum; P.grad_scale = d_grad_scale; P.ignore_index = ignore_index;
         P.B = B; P.C = C; P.h = h; P.w = w; P.H = H; P.W = W;
         PW.weight = d_weight; PW.one_m_eps = one_m_eps; PW.eps_c = eps_c;
-        // warps are independent; a warp's tile of taps takes C * (32 / (s/2)) * 16 bytes of shared memory
-        const size_t smem_warp = (size_t)(C + 2) * (64 / s) * 16;
-        int wpc = 4;
-        while (wpc > 1 && smem_warp * wpc > 56 * 1024) wpc /= 2;
-        const size_t smem = smem_warp * wpc;
-        const bool gtaps = smem_warp > K2_GTAPS_SMEM;               // staged tile too large for a decent occupancy
-        if (smem <= 200 * 1024 || gtaps) {
-            const int wgx = (64 / s) / 2;
-            P.nty = (h + 1 + 1) / 2;
-            P.ntx = (w + 1 + wgx - 1) / wgx;
-            const long long tiles = (long long)B * P.nty * P.ntx;
-            const unsigned grid = (unsigned)((tiles + wpc - 1) / wpc);
-            auto launch = [&](auto kernel) -> int {
-                LC2IS_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                kernel<<<grid, wpc * 32, smem, st>>>(PW);          // (sliced to K2SParams for the unweighted kernels)
-                return 0;
-            };
-            auto launch_g = [&](auto kernel) -> int {
-                kernel<<<(unsigned)((tiles + 3) / 4), 128, 0, st>>>(PW);
-                return 0;
-            };
-            int e = wt ? (gtaps ? (s == 8 ? launch_g(k2_strip_gtaps_kernel<8, false, true>)
-                                          : launch_g(k2_strip_gtaps_kernel<16, false, true>))
-                                : (s == 8 ? launch(k2_strip_kernel<8, false, true>) : launch(k2_strip_kernel<16, false, true>)))
-                       : (gtaps ? (s == 8 ? launch_g(k2_strip_gtaps_kernel<8, false>) : launch_g(k2_strip_gtaps_kernel<16, false>))
-                                : (s == 8 ? launch(k2_strip_kernel<8, false>) : launch(k2_strip_kernel<16, false>)));
-            if (e) return e;
-            LC2IS_CHECK_LAUNCH("k2_strip_kernel");
-            if (d_grad_low_bf16) return lc2is_grad_to_bf16(d_grad_low, B, C, h * w, d_grad_low_bf16, stream);
-            return 0;
-        }
+        if (int e = wt ? launch_k2_strip<false, true>(PW, s, st) : launch_k2_strip<false, false>(P, s, st)) return e;
+        if (d_grad_low_bf16) return lc2is_grad_to_bf16(d_grad_low, B, C, h * w, d_grad_low_bf16, stream);
+        return 0;
     }
     fast = fast && s == 4;
     K2Params P;
@@ -943,11 +896,10 @@ extern "C" int lc2is_upsample_ce_fwd_bwd_ex(const float* d_low, const int64_t* d
         P.B = B; P.C = C; P.h = h; P.w = w; P.H = H; P.W = W;
         P.s = s; P.off = g.off; P.rs = g.rs;
         P.weight = d_weight; P.one_m_eps = one_m_eps; P.eps_c = eps_c;
-        const int bps = s / 4;
         P.q = (g.off + s / 2) / 4;
-        // 128 threads = tgy*tgx groups of bps*bps threads; tile = 32 x 64 pixels
-        P.tgy = 8 / bps; P.tgx = 16 / bps;
-        smem = (size_t)C * (bps > 1 ? P.tgy * P.tgx * 4 : (P.tgy + 1) * (P.tgx + 1)) * sizeof(float);
+        // 128 threads = 8 x 16 blocks of 4 x 4 pixels; the tile holds the 9 x 17 source cells they read
+        P.tgy = 8; P.tgx = 16;
+        smem = (size_t)C * (P.tgy + 1) * (P.tgx + 1) * sizeof(float);
         if (smem > 110 * 1024) fast = false;
     }
     if (fast) {
@@ -957,7 +909,7 @@ extern "C" int lc2is_upsample_ce_fwd_bwd_ex(const float* d_low, const int64_t* d
             kernel<<<grid, 128, smem, st>>>(P);
             return 0;
         };
-        int e = wt ? launch(k2_fast_kernel<1, true>) : launch(k2_fast_kernel<1>);
+        int e = wt ? launch(k2_fast_kernel<true>) : launch(k2_fast_kernel<false>);
         if (e) return e;
         LC2IS_CHECK_LAUNCH("k2_fast_kernel");
     } else {
@@ -982,6 +934,31 @@ extern "C" int lc2is_ce_split_supported(int h, int w, int H, int W) {
     return fast_scale(h, w, H, W, &s) && (s == 8 || s == 16) ? 1 : 0;
 }
 
+namespace lc2is {
+// Both prepass entries after their argument checks: k2_labels_prepass_kernel<s, LT> for the scale s = 4 / 8 / 16.
+template <typename LT>
+static int launch_labels_prepass(const LT* labels, int B, int C, int h, int w, int H, int W, long long ignore,
+                                 uint16_t* packed, int64_t* n_valid, float* grad_low, cudaStream_t st) {
+    int s = 0;
+    if (!fast_scale(h, w, H, W, &s) || s > 16)
+        return fail(LC2IS_ERR_UNSUPPORTED, "label prepass needs a power-of-two scale 4 / 8 / 16%s");
+    if (((uintptr_t)labels % 16) || ((uintptr_t)packed % 16)) return fail(LC2IS_ERR_ARG, "labels must be 16-byte aligned%s");
+    const long long total = (long long)B * H * (w + 1);
+    long long blocks = (total + 255) / 256;
+    const long long cap = (long long)sm_count() * 16;
+    if (blocks > cap) blocks = cap;
+    auto launch = [&](auto kernel) {
+        kernel<<<(unsigned)blocks, 256, 0, st>>>(labels, B, C, h, w, H, W, ignore, (unsigned short*)packed,
+                                                 (unsigned long long*)n_valid, grad_low);
+    };
+    if (s == 4) launch(k2_labels_prepass_kernel<4, LT>);
+    else if (s == 8) launch(k2_labels_prepass_kernel<8, LT>);
+    else launch(k2_labels_prepass_kernel<16, LT>);
+    LC2IS_CHECK_LAUNCH(sizeof(LT) == 2 ? "k2_labels_prepass_kernel(packed)" : "k2_labels_prepass_kernel");
+    return 0;
+}
+}  // namespace lc2is
+
 extern "C" int lc2is_ce_labels_prepass(const int64_t* d_labels,
                                        int B, int C, int h, int w, int H, int W, int64_t ignore_index,
                                        uint16_t* d_labels_packed, int64_t* d_n_valid,
@@ -991,25 +968,8 @@ extern "C" int lc2is_ce_labels_prepass(const int64_t* d_labels,
     if (C >= 0x7fff) return fail(LC2IS_ERR_UNSUPPORTED, "packed labels hold class ids < 32767%s");
     if (B == 0) return 0;
     if (!d_labels) return fail(LC2IS_ERR_ARG, "null pointer%s");
-    int s = 0;
-    if (!fast_scale(h, w, H, W, &s) || s > 16)
-        return fail(LC2IS_ERR_UNSUPPORTED, "label prepass needs a power-of-two scale 4 / 8 / 16%s");
-    if (((uintptr_t)d_labels % 16) || ((uintptr_t)d_labels_packed % 16))
-        return fail(LC2IS_ERR_ARG, "labels must be 16-byte aligned%s");
-    const long long total = (long long)B * H * (w + 1);
-    long long blocks = (total + 255) / 256;
-    const long long cap = (long long)sm_count() * 16;
-    if (blocks > cap) blocks = cap;
-    auto launch = [&](auto kernel) {
-        kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
-            (const long long*)d_labels, B, C, h, w, H, W, (long long)ignore_index,
-            (unsigned short*)d_labels_packed, (unsigned long long*)d_n_valid, d_grad_low);
-    };
-    if (s == 4) launch(k2_labels_prepass_kernel<4, long long>);
-    else if (s == 8) launch(k2_labels_prepass_kernel<8, long long>);
-    else launch(k2_labels_prepass_kernel<16, long long>);
-    LC2IS_CHECK_LAUNCH("k2_labels_prepass_kernel");
-    return 0;
+    return launch_labels_prepass((const long long*)d_labels, B, C, h, w, H, W, (long long)ignore_index, d_labels_packed,
+                                 d_n_valid, d_grad_low, (cudaStream_t)stream);
 }
 
 extern "C" int lc2is_pack_labels(const int64_t* d_labels, int64_t n, int C, int64_t ignore_index,
@@ -1093,24 +1053,8 @@ extern "C" int lc2is_ce_labels_prepass_packed(const uint16_t* d_labels_packed, i
     if (B < 0 || C <= 0 || h <= 0 || w <= 0 || H <= 0 || W <= 0) return fail(LC2IS_ERR_SHAPE, "bad shape%s");
     if (B == 0) return 0;
     if (!d_labels_packed) return fail(LC2IS_ERR_ARG, "null pointer%s");
-    int s = 0;
-    if (!fast_scale(h, w, H, W, &s) || s > 16)
-        return fail(LC2IS_ERR_UNSUPPORTED, "label prepass needs a power-of-two scale 4 / 8 / 16%s");
-    if ((uintptr_t)d_labels_packed % 16) return fail(LC2IS_ERR_ARG, "labels must be 16-byte aligned%s");
-    const long long total = (long long)B * H * (w + 1);
-    long long blocks = (total + 255) / 256;
-    const long long cap = (long long)sm_count() * 16;
-    if (blocks > cap) blocks = cap;
-    auto launch = [&](auto kernel) {
-        kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
-            (const unsigned short*)d_labels_packed, B, C, h, w, H, W, 0LL, (unsigned short*)nullptr,
-            (unsigned long long*)d_n_valid, d_grad_low);
-    };
-    if (s == 4) launch(k2_labels_prepass_kernel<4, unsigned short>);
-    else if (s == 8) launch(k2_labels_prepass_kernel<8, unsigned short>);
-    else launch(k2_labels_prepass_kernel<16, unsigned short>);
-    LC2IS_CHECK_LAUNCH("k2_labels_prepass_kernel(packed)");
-    return 0;
+    return launch_labels_prepass((const unsigned short*)d_labels_packed, B, C, h, w, H, W, 0LL, nullptr, d_n_valid,
+                                 d_grad_low, (cudaStream_t)stream);
 }
 
 extern "C" int lc2is_upsample_ce_packed(const float* d_low, const uint16_t* d_labels_packed,
@@ -1125,31 +1069,8 @@ extern "C" int lc2is_upsample_ce_packed(const float* d_low, const uint16_t* d_la
     if (!fast_scale(h, w, H, W, &s) || (s != 8 && s != 16))
         return fail(LC2IS_ERR_UNSUPPORTED, "split path needs scale 8 or 16 (see lc2is_ce_split_supported)%s");
     K2SParams P;
-    P.low = d_low; P.labels = nullptr; P.labels16 = d_labels_packed; P.n_valid = nullptr; P.grad_low = d_grad_low;
+    P.low = d_low; P.labels = nullptr; P.labels16 = d_labels_packed; P.grad_low = d_grad_low;
     P.loss_sum = d_loss_sum; P.grad_scale = nullptr; P.ignore_index = 0;
     P.B = B; P.C = C; P.h = h; P.w = w; P.H = H; P.W = W;
-    const size_t smem_warp = (size_t)(C + 2) * (64 / s) * 16;
-    int wpc = 4;
-    while (wpc > 1 && smem_warp * wpc > 56 * 1024) wpc /= 2;
-    const size_t smem = smem_warp * wpc;
-    const bool gtaps = smem_warp > K2_GTAPS_SMEM;                   // staged tile too large for a decent occupancy
-    const int wgx = (64 / s) / 2;
-    P.nty = (h + 1 + 1) / 2;
-    P.ntx = (w + 1 + wgx - 1) / wgx;
-    const long long tiles = (long long)B * P.nty * P.ntx;
-    const unsigned grid = (unsigned)((tiles + wpc - 1) / wpc);
-    auto launch = [&](auto kernel) -> int {
-        LC2IS_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        kernel<<<grid, wpc * 32, smem, (cudaStream_t)stream>>>(P);
-        return 0;
-    };
-    auto launch_g = [&](auto kernel) -> int {
-        kernel<<<(unsigned)((tiles + 3) / 4), 128, 0, (cudaStream_t)stream>>>(P);
-        return 0;
-    };
-    int e = gtaps ? (s == 8 ? launch_g(k2_strip_gtaps_kernel<8, true>) : launch_g(k2_strip_gtaps_kernel<16, true>))
-                  : (s == 8 ? launch(k2_strip_kernel<8, true>) : launch(k2_strip_kernel<16, true>));
-    if (e) return e;
-    LC2IS_CHECK_LAUNCH("k2_strip_kernel(split)");
-    return 0;
+    return launch_k2_strip<true, false>(P, s, (cudaStream_t)stream);
 }

@@ -16,7 +16,7 @@ import torch
 from torch import Tensor, nn
 
 from . import ops
-from .model.loss import _UpsampleCE
+from .model.loss import _UpsampleCE, _upsample_ce_loss
 
 
 def _hw_shape(P: int, hw_shape) -> Tuple[int, int]:
@@ -97,17 +97,8 @@ class _SegHeadLoss(torch.autograd.Function):
         logits, v_hat, inv_v = ops.cosine_logits_fwd(v, t_hat, C, hw_shape, normalize, logit_scale)
         need_grad = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
         n_valid = ops.count_valid(labels, C, ignore_index)
-        if weight is None and label_smoothing == 0:
-            gscale = ops.mean_scale(n_valid) if reduction == "mean" else None
-            loss_sum, _, gbf = ops.upsample_ce(logits, labels, ignore_index, gscale, want_grad=need_grad,
-                                               want_bf16=need_grad)
-            loss = ops.finalize_loss(loss_sum, n_valid) if reduction == "mean" else loss_sum.float()
-        else:
-            den = ops.ce_weight_sum(labels, C, ignore_index, weight) if reduction == "mean" else None
-            gscale = torch.reciprocal(den).float() if reduction == "mean" else None
-            loss_sum, _, gbf = ops.upsample_ce(logits, labels, ignore_index, gscale, want_grad=need_grad,
-                                               want_bf16=need_grad, weight=weight, label_smoothing=label_smoothing)
-            loss = ops.weighted_mean_loss(loss_sum, den) if reduction == "mean" else loss_sum.float()
+        loss, _, gbf = _upsample_ce_loss(logits, labels, ignore_index, reduction, weight, label_smoothing,
+                                        want_grad=need_grad, want_bf16=need_grad, n_valid=n_valid)
         if need_grad:
             ctx.save_for_backward(gbf, logits, v_hat, inv_v, t_hat, inv_t)
         ctx.meta = (C, normalize, logit_scale, v.dtype, t.dtype, t.dim())

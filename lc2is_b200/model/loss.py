@@ -16,27 +16,35 @@ from torch import Tensor, nn
 from .. import ops
 
 
+def _upsample_ce_loss(low32, labels, ignore_index, reduction, weight, label_smoothing, want_grad, want_bf16=False,
+                      n_valid=None):
+    """K2 with the 'mean' denominator of nn.CrossEntropyLoss -> (loss fp32 [1], grad_low, grad_low_bf16), the gradients
+    scaled by 1 / denominator: the number of counted pixels (n_valid, counted here unless given), or with a weight or a
+    smoothing the summed class weights of the counted pixels (ops.ce_weight_sum).  All on the device."""
+    mean = reduction == "mean"
+    if weight is None and label_smoothing == 0:
+        if n_valid is None:
+            n_valid = ops.count_valid(labels, low32.shape[1], ignore_index)
+        gscale = ops.mean_scale(n_valid) if mean else None
+        loss_sum, grad, gbf = ops.upsample_ce(low32, labels, ignore_index, gscale, want_grad=want_grad,
+                                              want_bf16=want_bf16)
+        return (ops.finalize_loss(loss_sum, n_valid) if mean else loss_sum.float()), grad, gbf
+    den = ops.ce_weight_sum(labels, low32.shape[1], ignore_index, weight) if mean else None
+    # 1 / 0 = inf when nothing is counted: every gradient term of an uncounted pixel is a select, not a product
+    gscale = torch.reciprocal(den).float() if mean else None
+    loss_sum, grad, gbf = ops.upsample_ce(low32, labels, ignore_index, gscale, want_grad=want_grad, want_bf16=want_bf16,
+                                          weight=weight, label_smoothing=label_smoothing)
+    return (ops.weighted_mean_loss(loss_sum, den) if mean else loss_sum.float()), grad, gbf
+
+
 class _UpsampleCE(torch.autograd.Function):
-    """weight (fp32 [C]) / label_smoothing select the weighted kernels; 'mean' then divides by sum_i w[t_i] over the
-    counted pixels (ops.ce_weight_sum), all on the device."""
 
     @staticmethod
     def forward(ctx, low: Tensor, target: Tensor, ignore_index: int, reduction: str,
                 weight: Optional[Tensor] = None, label_smoothing: float = 0.0):
         need_grad = ctx.needs_input_grad[0]
-        low32 = low.float()
-        if weight is None and label_smoothing == 0:
-            n_valid = ops.count_valid(target, low.shape[1], ignore_index)
-            gscale = ops.mean_scale(n_valid) if reduction == "mean" else None
-            loss_sum, grad, _ = ops.upsample_ce(low32, target, ignore_index, gscale, want_grad=need_grad)
-            loss = ops.finalize_loss(loss_sum, n_valid) if reduction == "mean" else loss_sum.float()
-        else:
-            den = ops.ce_weight_sum(target, low.shape[1], ignore_index, weight) if reduction == "mean" else None
-            # 1 / 0 = inf when nothing is counted: every gradient term of an uncounted pixel is a select, not a product
-            gscale = torch.reciprocal(den).float() if reduction == "mean" else None
-            loss_sum, grad, _ = ops.upsample_ce(low32, target, ignore_index, gscale, want_grad=need_grad, weight=weight,
-                                                label_smoothing=label_smoothing)
-            loss = ops.weighted_mean_loss(loss_sum, den) if reduction == "mean" else loss_sum.float()
+        loss, grad, _ = _upsample_ce_loss(low.float(), target, ignore_index, reduction, weight, label_smoothing,
+                                         want_grad=need_grad)
         if need_grad:
             ctx.save_for_backward(grad)
         ctx.in_dtype = low.dtype

@@ -27,7 +27,7 @@ ROUNDS, ITERS, TORCH_ITERS = 5, 50, 10
 SHAPES = [
     ("x16 G-A", 16, 150, 32, 512, "k2_strip_kernel<16>"),
     ("x8", 16, 150, 64, 512, "k2_strip_kernel<8>"),
-    ("x4 G-B", 16, 150, 128, 512, "k2_fast_kernel<1>"),
+    ("x4 G-B", 16, 150, 128, 512, "k2_fast_kernel"),
     ("x16 C=847", 8, 847, 64, 1024, "k2_strip_gtaps_kernel<16>"),
     ("generic 24->120", 4, 150, 24, 120, "k2_generic_kernel"),          # scale 5: not a power of two
 ]
