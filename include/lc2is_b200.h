@@ -83,8 +83,9 @@ int lc2is_cosine_logits_fwd(const void* d_v, int v_dtype, int B, int hw, int D,
 
 /* TextToPatch.visual / .textual forward (model/text_patch.py:11-12,16-17): y[M,N] = x[M,K] W[N,K]^T + b[N] on the
  * logits GEMM's tcgen05 / TMEM / TMA pipeline.  x, W bf16 (W in nn.Linear's own [out,in] layout), b fp32 or NULL,
- * y bf16 or fp32 row major.  K % 64 == 0, N % 16 == 0.  Shapes with M % 256 == 0, N % 256 == 0 and at least two
- * waves of 256 x 256 tiles run the 2-SM (cta_group::2) form of the kernel, everything else the 1-SM form. */
+ * y bf16 or fp32 row major.  K % 64 == 0, N % 16 == 0.  d_x, d_w, d_y and d_bias 16-byte aligned (LC2IS_ERR_ARG
+ * otherwise).  Shapes with M % 256 == 0, N % 256 == 0 and at least two 256 x 256 tiles per CTA pair (2 * (SMs / 2)
+ * tiles) run the 2-SM (cta_group::2) form of the kernel, everything else the 1-SM form. */
 int lc2is_linear_fwd(const void* d_x_bf16, const void* d_w_bf16, const float* d_bias,
                      long long M, int N, int K, void* d_y, int y_dtype, lc2is_stream_t stream);
 
@@ -103,10 +104,13 @@ int lc2is_bicubic4_tokens_bwd(const void* d_gy, int gy_dtype, int B, int h, int 
 
 /* Backward of the same projection (autograd of model/text_patch.py:12,17; y = x W^T + b), all on tcgen05:
  *   d_gx [M,K] (gx_dtype) = gy . W      lc2is_linear_fwd's pipeline on the transposed weight (built in d_ws)
- *   d_gw [N,K] fp32      += gy^T . x    split-K over the rows, both operands MN-major, fp32 L2 reductions (ACCUMULATES:
- *                                       zero it, or let several micro-batches add up like autograd does)
+ *   d_gw [N,K] fp32      += gy^T . x    split-K over the rows, both operands MN-major: each slice stores its fp32 partial
+ *                                       sum in d_ws, one pass adds the slices to d_gw (ACCUMULATES: zero it, or let
+ *                                       several micro-batches add up like autograd does)
  *   d_gb [N]   fp32      += column sums of gy
  * gy [M,N], x [M,K], W [N,K] bf16; N and K multiples of 64.  Any of d_gx / d_gw / d_gb may be NULL.
+ * d_gy, d_x, d_gx, d_gw and d_ws 16-byte aligned (LC2IS_ERR_ARG otherwise).  Pointers, shapes and gx_dtype are checked
+ * before the first launch: a call rejected for them has written no output.
  * d_ws: lc2is_linear_bwd_workspace(N, K) bytes (the transposed weight for d_gx, the split-K partial sums for d_gw). */
 int64_t lc2is_linear_bwd_workspace(int N, int K);
 int lc2is_linear_bwd(const void* d_gy_bf16, const void* d_x_bf16, const void* d_w_bf16, long long M, int N, int K,

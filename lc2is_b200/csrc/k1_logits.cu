@@ -737,7 +737,9 @@ extern "C" int lc2is_linear_fwd(const void* d_x_bf16, const void* d_w_bf16, cons
     if (N % 16) return fail(LC2IS_ERR_SHAPE, "N must be a multiple of 16 (got %s%lld)", "", N);
     if (M > 0x7fffffffLL / 2) return fail(LC2IS_ERR_SHAPE, "M too large%s");
     if (y_dtype != LC2IS_F32 && y_dtype != LC2IS_BF16) return fail(LC2IS_ERR_ARG, "y_dtype%s");
-    if (((uintptr_t)d_x_bf16 | (uintptr_t)d_w_bf16 | (uintptr_t)d_y) % 16) return fail(LC2IS_ERR_ARG, "pointers must be 16-byte aligned%s");
+    // x and W are TMA bases, y is written and the bias read with 16-byte vectors by the epilogue
+    if (((uintptr_t)d_x_bf16 | (uintptr_t)d_w_bf16 | (uintptr_t)d_y | (uintptr_t)d_bias) % 16)
+        return fail(LC2IS_ERR_ARG, "x, W, y and the bias must be 16-byte aligned%s");
     if (M == 0) return 0;
     K1Params P;
     P.out = nullptr; P.out_rm = d_y; P.bias = d_bias; P.out_f32 = y_dtype == LC2IS_F32;

@@ -780,7 +780,8 @@ extern "C" int lc2is_cosine_logits_bwd(const void* d_grad_logits, int g_dtype, c
 // ---------------------------------------------------------------------------------------------
 // TextToPatch.visual backward (autograd of model/text_patch.py:12,17; y = x W^T + b):
 //   gx [M,K]  = gy [M,N] . W [N,K]       lc2is_linear_fwd's tcgen05 pipeline on the transposed weight (workspace)
-//   gw [N,K] += gy^T . x                  tcgen05 split-K over the rows, both operands MN-major, fp32 L2 reductions
+//   gw [N,K] += gy^T . x                  tcgen05 split-K over the rows, both operands MN-major; each slice stored to the
+//                                         workspace, reduce_partials_kernel adds the slices to gw
 //   gb [N]   += column sums of gy
 constexpr int LINEAR_BWD_MAX_COLSUM_CTAS = 1024;            // per-CTA partial column sums of gy (workspace bound)
 constexpr int LINEAR_BWD_MAX_SLICES = 32;                  // split-K slices of the weight gradient (workspace bound)
@@ -798,10 +799,18 @@ extern "C" int lc2is_linear_bwd(const void* d_gy_bf16, const void* d_x_bf16, con
     if (N % 64 || K % 64) return fail(LC2IS_ERR_SHAPE, "N and K must be multiples of 64%s");
     if (M > 0x7fffffffLL / 2) return fail(LC2IS_ERR_SHAPE, "M too large%s");
     if (!d_gy_bf16) return fail(LC2IS_ERR_ARG, "null pointer%s");
+    // every argument is checked before the first launch, so that a rejected call leaves all outputs untouched
+    if (d_gx && (!d_w_bf16 || !d_ws)) return fail(LC2IS_ERR_ARG, "gx needs the weight and the workspace%s");
+    if (d_gx && gx_dtype != LC2IS_F32 && gx_dtype != LC2IS_BF16) return fail(LC2IS_ERR_ARG, "gx_dtype%s");
+    if (d_gw && (!d_x_bf16 || !d_ws)) return fail(LC2IS_ERR_ARG, "gw needs x and the workspace%s");
+    if (d_gb && !d_ws) return fail(LC2IS_ERR_ARG, "gb needs the workspace%s");
+    // gy, x and the workspace are TMA bases and read with 16-byte vectors (colsum_bf16_kernel, reduce_partials_kernel),
+    // gx is written by lc2is_linear_fwd's vector epilogue and gw read and written as float4; gb is accessed per element
+    if (((uintptr_t)d_gy_bf16 | (uintptr_t)d_x_bf16 | (uintptr_t)d_gx | (uintptr_t)d_gw | (uintptr_t)d_ws) % 16)
+        return fail(LC2IS_ERR_ARG, "gy, x, gx, gw and the workspace must be 16-byte aligned%s");
     if (M == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
     if (d_gx) {
-        if (!d_w_bf16 || !d_ws) return fail(LC2IS_ERR_ARG, "gx needs the weight and the workspace%s");
         dim3 grid((K + 31) / 32, (N + 31) / 32);
         transpose_bf16_kernel<<<grid, 256, 0, st>>>((const __nv_bfloat16*)d_w_bf16, N, K, (__nv_bfloat16*)d_ws);
         LC2IS_CHECK_LAUNCH("transpose_bf16_kernel");
@@ -809,7 +818,6 @@ extern "C" int lc2is_linear_bwd(const void* d_gy_bf16, const void* d_x_bf16, con
         if (int e = lc2is_linear_fwd(d_gy_bf16, d_ws, nullptr, M, K, N, d_gx, gx_dtype, stream)) return e;
     }
     if (d_gw) {
-        if (!d_x_bf16 || !d_ws) return fail(LC2IS_ERR_ARG, "gw needs x and the workspace%s");
         // out[n][k] += sum_m gy[m][n] x[m][k]: A = x (M side = the K input features, 256 per CTA), B = gy (N side);
         // every CTA stores its partial tile into slice ks of the workspace, reduce_partials_kernel adds the slices to gw
         DtParams P;
@@ -845,8 +853,6 @@ extern "C" int lc2is_linear_bwd(const void* d_gy_bf16, const void* d_x_bf16, con
         LC2IS_CHECK_LAUNCH("reduce_partials_kernel");
     }
     if (d_gb) {
-        if (!d_ws) return fail(LC2IS_ERR_ARG, "gb needs the workspace%s");
-        if (N % 8) return fail(LC2IS_ERR_SHAPE, "N must be a multiple of 8%s");
         float* cpart = reinterpret_cast<float*>(static_cast<uint8_t*>(d_ws) + ((size_t)N * K * 2 + 255) / 256 * 256 +
                                                 (size_t)LINEAR_BWD_MAX_SLICES * N * K * 4);
         long long blocks = (M + 255) / 256;

@@ -29,6 +29,13 @@ def _dt(t: Tensor) -> int:
     raise _lib.Lc2isError(f"unsupported dtype {t.dtype} (float32 / bfloat16 only)")
 
 
+def _aligned(t: Tensor) -> Tensor:
+    """t, or a copy of it when it does not start on a 16-byte boundary: the projection entries read and write their
+    tensors with 16-byte vectors and TMA, and a view into a larger buffer (a bias sliced out of a flat parameter
+    buffer, say) may start anywhere."""
+    return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
 # ---- K0 -----------------------------------------------------------------------------------
 def proto_normalize(t: Tensor, normalize: bool = True) -> Tuple[Tensor, Tensor]:
     """t [C,D] or [n_sets,C,D] fp32 -> (t_hat bf16 [n_sets,C_pad,D], inv_norm fp32 [n_sets,C])."""
@@ -47,12 +54,12 @@ def proto_normalize(t: Tensor, normalize: bool = True) -> Tuple[Tensor, Tensor]:
 # ---- TextToPatch projection ------------------------------------------------------------------
 def linear_fwd(x: Tensor, weight: Tensor, bias: Optional[Tensor] = None, out_dtype=torch.bfloat16) -> Tensor:
     """y = x W^T + b on the tcgen05 pipeline.  x [M,K] bf16, weight [N,K] bf16 (nn.Linear layout), bias fp32 [N]."""
-    x = _req(x, torch.bfloat16, "x")
-    weight = _req(weight, torch.bfloat16, "weight")
+    x = _aligned(_req(x, torch.bfloat16, "x"))
+    weight = _aligned(_req(weight, torch.bfloat16, "weight"))
     M, K = x.shape
     N = weight.shape[0]
     if bias is not None:
-        bias = _req(bias, torch.float32, "bias")
+        bias = _aligned(_req(bias, torch.float32, "bias"))
     y = torch.empty(M, N, dtype=out_dtype, device=x.device)
     check(lib.lc2is_linear_fwd(ptr(x), ptr(weight), ptr(bias), M, N, K, ptr(y), _dt(y), stream_ptr()), "lc2is_linear_fwd")
     return y
@@ -91,22 +98,28 @@ def bicubic4_tokens_bwd(gy: Tensor, hw_shape: Tuple[int, int], out_dtype=torch.f
 def linear_bwd(gy: Tensor, x: Tensor, weight: Tensor, need_gx: bool = True, need_gw: bool = True, need_gb: bool = True,
                gx_dtype=torch.bfloat16, gw: Optional[Tensor] = None, gb: Optional[Tensor] = None):
     """Backward of y = x W^T + b on tcgen05 (lc2is_linear_bwd).  gy [M,N], x [M,K], weight [N,K]: bf16.
-    -> (gx [M,K] gx_dtype | None, gw fp32 [N,K] | None, gb fp32 [N] | None); `gw` / `gb` given: accumulated into."""
-    gy = _req(gy, torch.bfloat16, "gy")
-    x = _req(x, torch.bfloat16, "x")
+    -> (gx [M,K] gx_dtype | None, gw fp32 [N,K] | None, gb fp32 [N] | None); `gw` / `gb` given: accumulated into
+    (a `gw` that is not contiguous or not 16-byte aligned through an aligned copy, written back)."""
+    gy = _aligned(_req(gy, torch.bfloat16, "gy"))
+    x = _aligned(_req(x, torch.bfloat16, "x"))
     weight = _req(weight, torch.bfloat16, "weight")
     M, N = gy.shape
     K = x.shape[1]
     dev = gy.device
     gx = torch.empty(M, K, dtype=gx_dtype, device=dev) if need_gx else None
+    gw_caller = None
     if need_gw and gw is None:
         gw = torch.zeros(N, K, dtype=torch.float32, device=dev)
+    elif need_gw and (gw.data_ptr() % 16 or not gw.is_contiguous()):
+        gw_caller, gw = gw, gw.clone(memory_format=torch.contiguous_format)
     if need_gb and gb is None:
         gb = torch.zeros(N, dtype=torch.float32, device=dev)
     ws = torch.empty(int(lib.lc2is_linear_bwd_workspace(N, K)), dtype=torch.uint8, device=dev)
     check(lib.lc2is_linear_bwd(ptr(gy), ptr(x), ptr(weight), M, N, K, ptr(gx), _dt(gx) if need_gx else 0,
                                ptr(gw) if need_gw else None, ptr(gb) if need_gb else None, ptr(ws), stream_ptr()),
           "lc2is_linear_bwd")
+    if gw_caller is not None:
+        gw = gw_caller.copy_(gw)
     return gx, (gw if need_gw else None), (gb if need_gb else None)
 
 

@@ -128,7 +128,8 @@ def k1b_reference(G: Tensor, logits: Tensor, v: Tensor, inv_v: Tensor, t_hat: Te
 
 def check_bound(name, got, ref, A, bf16_out=False, base=None, tau=TAU):
     """|got - (base + ref)| <= tau * A (+ BF16_OUT |ref|) per element, asserted on the maxima of [128 rows x 64 channels]
-    blocks of the [images | sets, rows, D] tensors.  -> (worst |got - ref| / A, worst share of the bound used)."""
+    blocks of the [images | sets, rows, D] (or [rows, D]) tensors; the last blocks may be partial.
+    -> (worst |got - ref| / A, worst share of the bound used)."""
     got = got.to(ref.device).double().reshape(ref.shape)
     if base is not None:
         got = got - base.to(ref.device).double().reshape(ref.shape)
@@ -137,9 +138,11 @@ def check_bound(name, got, ref, A, bf16_out=False, base=None, tau=TAU):
     if base is not None:                           # one fp32 rounding of base + result
         bound = bound + 2.0 ** -24 * (base.to(ref.device).double().reshape(ref.shape) + ref).abs()
     use = torch.where(err == 0, torch.zeros_like(err), err / bound)          # NaN (unwritten) stays NaN
+    if use.dim() == 2:
+        use = use.unsqueeze(0)
     X, R, D = use.shape
-    Rp = -(-R // 128) * 128
-    blocks = torch.nn.functional.pad(use, (0, 0, 0, Rp - R)).view(X, Rp // 128, 128, D // 64, 64).amax(dim=(2, 4))
+    Rp, Dp = -(-R // 128) * 128, -(-D // 64) * 64
+    blocks = torch.nn.functional.pad(use, (0, Dp - D, 0, Rp - R)).view(X, Rp // 128, 128, Dp // 64, 64).amax(dim=(2, 4))
     bad = ~(blocks <= 1)
     if bool(bad.any()):
         worst = torch.nan_to_num(blocks, nan=float("inf")).flatten().argmax()
@@ -148,4 +151,4 @@ def check_bound(name, got, ref, A, bf16_out=False, base=None, tau=TAU):
                              f"image/set {x}, rows {128 * rt}.., channels {64 * cb}.. at {float(blocks[x, rt, cb]):.3g} "
                              f"x the bound (worst |got-ref|/A overall {float((err / A).nan_to_num(float('inf')).max()):.3g})")
     pos = A > 0
-    return float((err[pos] / A[pos]).max()), float(blocks.max())
+    return float((err[pos] / A[pos]).max()) if bool(pos.any()) else 0.0, float(blocks.max())

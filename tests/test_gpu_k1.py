@@ -151,11 +151,12 @@ def test_linear_projection_gemm(M, K, N, out_dtype):
     assert float((y - ref_fp32).abs().max()) <= 2e-2 * float(ref_fp32.abs().max())
 
 
-@pytest.mark.parametrize("M,K,N,out_dtype", [(32768, 768, 512, torch.bfloat16), (20480, 128, 256, torch.float32),
+@pytest.mark.parametrize("M,K,N,out_dtype", [(32768, 768, 512, torch.bfloat16), (40960, 128, 256, torch.float32),
                                               (38912, 768, 512, torch.float32)])
 def test_linear_projection_gemm_two_sm_form(M, K, N, out_dtype):
-    """Shapes that take the cta_group::2 kernel (M % 256 == 0, N % 256 == 0, at least two waves of CTA pairs): same
-    checks as above, on the device (the fp32 reference of a 32768 x 768 x 512 product is computed by torch there)."""
+    """Shapes that take the cta_group::2 kernel on a 148-SM B200 (M % 256 == 0, N % 256 == 0, at least two 256 x 256
+    pair tiles per CTA pair: 148); tests/test_gpu_linear_exact.py asserts the route by kernel name.  Same checks as
+    above, on the device (the fp32 reference of a 32768 x 768 x 512 product is computed by torch there)."""
     g = torch.Generator(device=DEV).manual_seed(13)
     x = torch.randn(M, K, generator=g, device=DEV)
     w = torch.randn(N, K, generator=g, device=DEV) * K ** -0.5

@@ -1,11 +1,12 @@
 """Host side of the exact-operand K1b tests (no GPU needed): the float64 reference of tests/k1b_reference.py, fed unrounded
 float64 operands, against torch.autograd of oracle.cosine_logits in float64 - normalize on / off, shared and per-image
-prototypes, s != 1, g != 1 - plus the LC2IS_BWD_RAW_V algebra, the r / rt projection identity and the operand rounding."""
+prototypes, s != 1, g != 1 - plus the LC2IS_BWD_RAW_V algebra, the r / rt projection identity, the operand rounding and
+check_bound on partial blocks."""
 import pytest
 import torch
 import torch.nn.functional as F
 
-from k1b_reference import gemm_operand, k1b_reference, projections
+from k1b_reference import TAU, check_bound, gemm_operand, k1b_reference, projections
 from oracle import head_oracle as O
 
 f64 = torch.float64
@@ -114,3 +115,22 @@ def test_gemm_operand_rounding():
     assert torch.equal(gemm_operand(Gbf, C), op)
     with pytest.raises(ValueError):
         gemm_operand(Gbf, C, inv)
+
+
+def test_check_bound_on_partial_blocks_names_the_block():
+    """A [rows, channels] matrix whose sizes are not multiples of the [128 x 64] block: within the bound it passes and
+    reports the worst ratio; one element over the bound, or one NaN (an unwritten element), fails and names its block."""
+    g = torch.Generator().manual_seed(4)
+    R, D = 300, 272
+    ref = torch.randn(R, D, generator=g, dtype=f64)
+    A = ref.abs() + 1
+    worst, use = check_bound("within", ref + 0.5 * TAU * A, ref, A)
+    assert abs(worst - 0.5 * TAU) <= 1e-3 * TAU and 0.49 < use <= 0.5 + 1e-9
+    bad = ref.clone()
+    bad[257, 270] += 2 * TAU * A[257, 270]
+    with pytest.raises(AssertionError, match=r"1 of 15 .* rows 256\.\., channels 256\.\."):
+        check_bound("over", bad, ref, A)
+    bad = ref.clone()
+    bad[130, 3] = float("nan")
+    with pytest.raises(AssertionError, match=r"rows 128\.\., channels 0\.\."):
+        check_bound("unwritten", bad, ref, A)
