@@ -34,6 +34,13 @@
 //             rho(y+1) = rho(y) tau - four ex2 per class - and  h = sum_j U(j) rho^j,  d = dh/drho  by one Horner sweep
 //             per row pair (two FFMA2 per pixel pair, U broadcast from shared memory) give the four tap gradients in
 //             registers: no cross-lane reduction; the four source cells of the group leave as one float reduction each.
+// Border jobs (top / bottom row or left / right column of groups, 2 (h + w) of the (h + 1)(w + 1) per image) are 1-D:
+//             their two taps of one axis are the same clamped cell, so the logit is constant along that axis.  Row phase:
+//             lane (hw, i) evaluates the diagonal pixel (i, i) - row i's value (left / right) or column i's (top / bottom),
+//             with the 2-D expression, so the argmax is bit-identical - one direct ex2 per class, a running (maximum,
+//             first class) instead of chunks and rescan; shuffles then give the shared code its per-lane state.  Class
+//             phase: U summed along the constant axis gives 16 weights, and per class 16 terms give the two distinct
+//             cells' gradients (one at a corner).  Jobs are numbered interior first, so the short border jobs fill the tail.
 // Jobs whose taps are not finite or span more than K2_FAST_RANGE take exact per-pixel paths (warp-uniform, one row per
 // lane of the lower half; ATen's taps, so 0 * inf poisons the same pixels as argmax(softmax(interpolate(x)))).
 #include "common.cuh"
@@ -93,15 +100,35 @@ __device__ __forceinline__ unsigned long long rc_now() { unsigned long long t; a
 struct RCJob {
     int n, ky, kx;                   // image, group row (-1..h-1), group column (-1..w-1)
 };
+// Job order: the (h-1)(w-1) interior groups of every image first (image-major, row-major), then the 2(h+w) border groups
+// of every image (per image: top row, bottom row, left column, right column).  Border jobs are the short ones (1-D row
+// and class phases), so they fill the kernel's tail.
 __device__ __noinline__ RCJob rc_decode(const RCParams& P, long long job) {
     RCJob J;
-    const int gpr = P.w + 1;         // groups per group row
-    const int per_img = (P.h + 1) * gpr;
-    J.n = (int)(job / per_img);
-    const int rem = (int)(job - (long long)J.n * per_img);
-    const int gy = rem / gpr;
-    J.ky = gy - 1;
-    J.kx = rem - gy * gpr - 1;
+    const int iw = P.w - 1;                                   // interior groups per group row
+    const long long ninner = (long long)P.B * (P.h - 1) * iw;
+    if (job < ninner) {
+        const int per_img = (P.h - 1) * iw;
+        J.n = (int)(job / per_img);
+        const int rem = (int)(job - (long long)J.n * per_img);
+        J.ky = rem / iw;
+        J.kx = rem - J.ky * iw;
+    } else {
+        job -= ninner;
+        const int per_img = 2 * (P.h + P.w);
+        J.n = (int)(job / per_img);
+        int rem = (int)(job - (long long)J.n * per_img);
+        if (rem < 2 * (P.w + 1)) {                            // top / bottom row, corners included
+            const bool bot = rem > P.w;
+            J.ky = bot ? P.h - 1 : -1;
+            J.kx = rem - (bot ? P.w + 1 : 0) - 1;
+        } else {                                              // left / right column without the corners
+            rem -= 2 * (P.w + 1);
+            const bool right = rem >= P.h - 1;
+            J.kx = right ? P.w - 1 : -1;
+            J.ky = rem - (right ? P.h - 1 : 0);
+        }
+    }
     return J;
 }
 
@@ -269,11 +296,49 @@ k23_rc_kernel(const __grid_constant__ CUtensorMap tm, const __grid_constant__ RC
         }
         const bool any = __any_sync(FULL, vm != 0);
         const bool slow = nonfinite || (any && !((mx - mn) < K2_FAST_RANGE));
+        // Border groups: both taps of one axis are the same clamped cell, so the quads have p1 = q1 = 0 (top / bottom row
+        // of groups) or q0 = q1 = 0 (left / right column): the logit is constant along that axis (over the whole group at
+        // a corner), and the 2-D path's expression gives the same value at every pixel of a row (edge_x) or column (edge_y)
+        const bool edge_y = ky < 0 || ky == P.h - 1, edge_x = kx < 0 || kx == P.w - 1;
+        const bool border = edge_y || edge_x;
         float loss = 0.f;
         int bidx[8];                                        // predictions of the lane's 8 pixels
         float2 S2[4];                                       // fast path: S(j) of the lane's 8 pixels, column pairs
 
-        if (!slow) {
+        if (!slow && border) {
+            // ================= 1-D row phase: lane (hw, i) evaluates pixel (i, i), which carries the value of row i
+            // (edge_x) or of column i (edge_y), for the half's classes: no recurrence, no chunks, no rescan ============
+            const float Mk = mx * LOG2E, fi = (float)i;
+            const float4* const Q = Q4 + hw * CPH;
+            float s = 0.f, bv = -INFINITY;
+            int bk = 0;
+#pragma unroll 1
+            for (int k = 0; k < CPH; k += 4) {              // (CPH is a multiple of 4)
+#pragma unroll
+                for (int u = 0; u < 4; ++u) {
+                    const float4 q = Q[k + u];
+                    const float v = fmaf(fi, fmaf(ly, q.w, q.z), fmaf(ly, q.y, q.x));
+                    s += ex2f(fmaf(v, LOG2E, -Mk));
+                    if (v > bv) { bv = v; bk = k + u; }     // strictly larger: the first class of a tie stays
+                }
+            }
+            // the halves meet: both hold the same sum (fp addition commutes); the upper half's maximum wins only when
+            // strictly larger
+            bk += hw * CPH;
+            s += __shfl_xor_sync(FULL, s, 16);
+            const float ov = __shfl_xor_sync(FULL, bv, 16);
+            const int ok = __shfl_xor_sync(FULL, bk, 16);
+            if (hw ? !(bv > ov) : (ov > bv)) bk = ok;
+            // the shared code's per-lane state: row i, columns 8 hw .. 8 hw + 7 (edge_y: column j's value is on lane j,
+            // edge_x: row i's on lane i; a corner is constant)
+#pragma unroll
+            for (int jj = 0; jj < 4; ++jj) {
+                const int la = edge_y ? 8 * hw + 2 * jj : i, lb = edge_y ? 8 * hw + 2 * jj + 1 : i;
+                S2[jj] = make_float2(__shfl_sync(FULL, s, la), __shfl_sync(FULL, s, lb));
+                bidx[2 * jj] = __shfl_sync(FULL, bk, la);
+                bidx[2 * jj + 1] = __shfl_sync(FULL, bk, lb);
+            }
+        } else if (!slow) {
             // ================= row phase: pass A + running maximum, one sweep over the half's classes ===============
             const float Mk = mx * LOG2E;
             // The loops of this kernel are kept ROLLED on purpose: the warps of an SM are at different places of the job
@@ -513,8 +578,59 @@ k23_rc_kernel(const __grid_constant__ CUtensorMap tm, const __grid_constant__ RC
 #ifdef RC_STAMPS
         if (lane == 0 && sti < RC_STAMP_SLOTS - 1) stp[sti++] = rc_now();
 #endif
-        // ================= class phase (lane = class): tap gradients by Horner sweeps ==============================
-        if (!slow && P.grad != nullptr && any) {
+        // ================= class phase (lane = class): tap gradients ======================================================
+        if (!slow && P.grad != nullptr && any && border) {
+            float* gimg = P.grad + (size_t)n * C * plane;
+            const int oA = clampi(ky, 0, P.h - 1) * P.w, oC = clampi(ky + 1, 0, P.h - 1) * P.w;
+            const int cxa = clampi(kx, 0, P.w - 1), cxb = clampi(kx + 1, 0, P.w - 1);
+            const float Mk = mx * LOG2E;
+            // ---- 1-D: U summed along the constant axis gives 16 weights Ub(p) (p = column for edge_y, row for
+            // edge_x); per class G = sum_p e(p) Ub(p) and L = sum_p lambda(p) e(p) Ub(p) are the two distinct cells'
+            // gradients (G - L, L), one cell (G) at a corner.  Lane (hw, p) adds 8 of the 16 terms of Ub(p), in an
+            // order that keeps both read patterns free of bank conflicts.
+            {
+                const int p = i;
+                float t = 0.f;
+#pragma unroll
+                for (int r = 0; r < 8; ++r) {
+                    const int rr = 8 * hw + ((r + (p >> 1) + hw) & 7);
+                    t += edge_y ? Usm[p * 16 + rr] : Usm[rr * 16 + p];
+                }
+                t += __shfl_xor_sync(FULL, t, 16);
+                __syncwarp();
+                if (hw == 0) Usm[p] = t;
+                __syncwarp();
+            }
+            const float4* const Ub4 = reinterpret_cast<const float4*>(Usm);
+            const int o0 = oA + cxa, o1 = edge_y ? oA + cxb : oC + cxa;   // the same cell at a corner
+#pragma unroll 1
+            for (int k = lane; k < C; k += 32) {
+                const float4 q = Q4[k];
+                float G = 0.f, L = 0.f;
+#pragma unroll 1
+                for (int p4 = 0; p4 < 4; ++p4) {
+                    const float4 ub = Ub4[p4];
+                    const float ubv[4] = {ub.x, ub.y, ub.z, ub.w};
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const float fp = (float)(4 * p4 + u), lp = (fp + 0.5f) * RS;
+                        const float v = fmaf(fp, fmaf(lp, q.w, q.z), fmaf(lp, q.y, q.x));
+                        const float g = ex2f(fmaf(v, LOG2E, -Mk)) * ubv[u];
+                        G += g;
+                        L = fmaf(lp, g, L);
+                    }
+                }
+                float* gk = gimg + (size_t)k * plane;
+                if (o0 == o1) {
+                    if (G != 0.f) red_add_f32(gk + o0, G);
+                } else {
+                    const float g0 = G - L;
+                    if (g0 != 0.f) red_add_f32(gk + o0, g0);
+                    if (L != 0.f) red_add_f32(gk + o1, L);
+                }
+            }
+        } else if (!slow && P.grad != nullptr && any) {
+            // ---- 2-D: Horner sweeps
             float* gimg = P.grad + (size_t)n * C * plane;
             const int oA = clampi(ky, 0, P.h - 1) * P.w, oC = clampi(ky + 1, 0, P.h - 1) * P.w;
             const int cxa = clampi(kx, 0, P.w - 1), cxb = clampi(kx + 1, 0, P.w - 1);
