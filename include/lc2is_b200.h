@@ -148,6 +148,12 @@ int lc2is_cosine_logits_bwd(const void* d_grad_logits, int g_dtype, const float*
  * two GEMMs is G * inv_norm_v and the normalise-backward of the patches is folded into the dV epilogue.  Needs
  * normalize = 1 and an fp32 gradient. */
 #define LC2IS_BWD_RAW_V 2
+/* LC2IS_BWD_WS_ZEROED: the caller has zeroed the first lc2is_cosine_logits_bwd_workspace_zeroed(...) bytes of d_ws
+ * (the accumulators of the projections and of the prototype GEMM) since the workspace was last used, e.g. in the
+ * zero-fill that starts its step.  The call then enqueues kernels only, which lets each one start its prologue while
+ * the previous kernel of the stream finishes (programmatic dependent launch); without the flag it zeroes them itself. */
+#define LC2IS_BWD_WS_ZEROED 4
+int64_t lc2is_cosine_logits_bwd_workspace_zeroed(int B, int hw, int D, int n_sets, int C);
 int lc2is_cosine_logits_bwd_ex(const void* d_grad_logits, int g_dtype, const float* d_logits,
                                const void* d_v_hat, const float* d_inv_norm_v,
                                const void* d_t_hat, const float* d_inv_norm_t,

@@ -15,7 +15,7 @@ LIB_PATH = os.path.join(_HERE, "csrc", "liblc2is_b200.so")
 
 F32, BF16 = 0, 1
 BILINEAR, BICUBIC = 0, 1
-BWD_REUSE_PREP, BWD_RAW_V = 1, 2      # flags of lc2is_cosine_logits_bwd_ex
+BWD_REUSE_PREP, BWD_RAW_V, BWD_WS_ZEROED = 1, 2, 4      # flags of lc2is_cosine_logits_bwd_ex
 
 
 class Lc2isError(RuntimeError):
@@ -49,6 +49,7 @@ SIGNATURES = {
     "lc2is_linear_bwd_workspace": (c_int64, [c_int, c_int]),
     "lc2is_linear_bwd": (c_int, [_p, _p, _p, c_int64, c_int, c_int, _p, c_int, _p, _p, _p, _p]),
     "lc2is_cosine_logits_bwd_workspace": (c_int64, [c_int, c_int, c_int, c_int, c_int]),
+    "lc2is_cosine_logits_bwd_workspace_zeroed": (c_int64, [c_int, c_int, c_int, c_int, c_int]),
     "lc2is_cosine_logits_bwd": (c_int, [_p, c_int, _p, _p, _p, _p, _p, c_int, c_int, c_int, c_int, c_int, c_int,
                                         c_float, _p, _p, c_int, _p, _p, _p]),
     "lc2is_cosine_logits_bwd_ex": (c_int, [_p, c_int, _p, _p, _p, _p, _p, c_int, c_int, c_int, c_int, c_int, c_int,

@@ -51,8 +51,12 @@ __global__ void finalize_loss_kernel(const double* loss_sum, const long long* n_
 }
 
 // both scalars of a 'mean' step in one launch (the loss sum is complete once K2 has run, the gradient scale is needed by K1b)
+// Launched with launch_pdl after the CE kernel.  It lets the logits backward be scheduled at once: that kernel only runs
+// its prologue before griddep_wait(), which returns after this one-thread grid has completed.
 __global__ void mean_scale_finalize_kernel(const long long* n_valid, float mult, float* scale, const double* loss_sum,
                                            float* loss) {
+    griddep_launch_dependents();
+    griddep_wait();
     const long long n = *n_valid;
     *scale = n > 0 ? mult / (float)n : 0.f;
     *loss = (float)(*loss_sum / (double)n);
@@ -78,8 +82,8 @@ extern "C" int lc2is_mean_scale_finalize(const int64_t* d_n_valid, float mult, f
                                          float* d_loss, lc2is_stream_t stream) {
     if (int e = ensure_device()) return e;
     if (!d_n_valid || !d_scale || !d_loss_sum || !d_loss) return fail(LC2IS_ERR_ARG, "null pointer%s");
-    mean_scale_finalize_kernel<<<1, 1, 0, (cudaStream_t)stream>>>((const long long*)d_n_valid, mult, d_scale, d_loss_sum,
-                                                                   d_loss);
+    LC2IS_CUDA(launch_pdl(mean_scale_finalize_kernel, 1, 1, 0, (cudaStream_t)stream, (const long long*)d_n_valid, mult,
+                          d_scale, d_loss_sum, d_loss));
     LC2IS_CHECK_LAUNCH("mean_scale_finalize_kernel");
     return 0;
 }

@@ -112,5 +112,32 @@ __device__ __forceinline__ void cubic_coeffs(float t, float (&c)[4]) {
 }
 __device__ __forceinline__ int clampi(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
 
+// ---- programmatic dependent launch ---------------------------------------------------------------
+// A kernel started by launch_pdl may begin while the kernel before it on the stream is still running: everything up to
+// griddep_wait() (barrier init, TMEM allocation, tensor-map prefetch, loads of inputs older than the predecessor) overlaps
+// that kernel's tail.  griddep_wait() returns once the predecessor has COMPLETED and its writes are visible, so every
+// thread of such a kernel must pass it before it reads the predecessor's output or writes anything the predecessor reads;
+// a kernel that does not call it could finish before its predecessor, breaking the transitive order of a chain.
+// griddep_launch_dependents() lets the next kernel of the stream be scheduled once every CTA has issued it (or exited).
+// Without a programmatic predecessor (a memset, an event wait, a plain launch) both are no-ops.
+__device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void griddep_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+template <typename... KArgs, typename... Args>
+inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                              Args&&... args) {
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = block;
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+}
+
 
 }  // namespace lc2is

@@ -78,6 +78,8 @@ k1b_prep_f32_kernel(const float* __restrict__ G, const float* __restrict__ L, in
     // receives one reduction per (class, CTA) - with one block per CTA the 128^2 grid would hammer 150 addresses
     // with 300 K reductions
     __shared__ float racc_s[PREPF_W][PREPF_PX];
+    griddep_wait();                               // G (and the gradient scale) come from the kernels before
+    griddep_launch_dependents();                  // the GEMMs set up while this pass runs
     const int b = blockIdx.y;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int cper = ((C_pad + PREPF_CS - 1) / PREPF_CS + PREPF_W - 1) / PREPF_W * PREPF_W;
@@ -199,6 +201,8 @@ k1b_dv_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ C
     __syncthreads();
     tc::tc_fence_after();
     const uint32_t tmem_base = *tmem_ptr;
+    griddep_wait();                                      // the bf16 operand and r come from the prep kernel
+    griddep_launch_dependents();
 
     if (warp == 0) {
         if (lane == 0) {
@@ -429,6 +433,8 @@ k1b_dt_kernel(const __grid_constant__ CUtensorMap tmV, const __grid_constant__ C
     __syncthreads();
     tc::tc_fence_after();
     const uint32_t tmem_base = *tmem_ptr;
+    griddep_wait();                                      // B (and A) may come from the kernel before
+    griddep_launch_dependents();
 
     if (nkb > 0) {
         if (warp == 0) {
@@ -532,6 +538,7 @@ k1b_dt_finish_kernel(const float* __restrict__ dt_raw, const float* __restrict__
                      const __nv_bfloat16* __restrict__ t_hat, const float* __restrict__ inv_t,
                      const float* __restrict__ grad_scale, int n_sets, int C, int C_pad, int D, int normalize,
                      float scale, float* __restrict__ grad_t) {
+    griddep_wait();
     const float gs = grad_scale ? __ldg(grad_scale) : 1.f;
     const long long total = (long long)n_sets * C * D;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
@@ -653,6 +660,11 @@ extern "C" int64_t lc2is_cosine_logits_bwd_workspace(int B, int hw, int D, int n
     return (int64_t)bwd_layout(B, hw, D, n_sets, C).total;
 }
 
+// r, rt and dt_raw: the head of the workspace that LC2IS_BWD_WS_ZEROED says is zero
+extern "C" int64_t lc2is_cosine_logits_bwd_workspace_zeroed(int B, int hw, int D, int n_sets, int C) {
+    return (int64_t)bwd_layout(B, hw, D, n_sets, C).gbf;
+}
+
 extern "C" int lc2is_cosine_logits_bwd_ex(const void* d_grad_logits, int g_dtype, const float* d_logits,
                                        const void* d_v_hat, const float* d_inv_norm_v,
                                        const void* d_t_hat, const float* d_inv_norm_t,
@@ -683,7 +695,9 @@ extern "C" int lc2is_cosine_logits_bwd_ex(const void* d_grad_logits, int g_dtype
     if (raw_v && (!normalize || g_dtype != LC2IS_F32))
         return fail(LC2IS_ERR_ARG, "LC2IS_BWD_RAW_V needs normalize = 1 and an fp32 gradient (its bf16 operand is scaled by inv||v||)%s");
     if (reuse && d_grad_t) return fail(LC2IS_ERR_ARG, "LC2IS_BWD_REUSE_PREP is for a dV-only call (d_grad_t must be NULL)%s");
-    if (!reuse) LC2IS_CUDA(cudaMemsetAsync(ws + L.r, 0, L.gbf - L.r, st));  // r, rt and dt_raw
+    // r, rt and dt_raw.  The kernels below are launched with launch_pdl: a memset between two of them would break the
+    // chain, so a step that zero-fills them at its start passes LC2IS_BWD_WS_ZEROED
+    if (!reuse && !(flags & LC2IS_BWD_WS_ZEROED)) LC2IS_CUDA(cudaMemsetAsync(ws + L.r, 0, L.gbf - L.r, st));
 
     // ---- projections r, rt (and the bf16 operand copy of an fp32 gradient) -------------------------
     const void* d_grad_logits_bf16 = g_dtype == LC2IS_F32 ? (const void*)(ws + L.gbf) : d_grad_logits;
@@ -695,9 +709,9 @@ extern "C" int lc2is_cosine_logits_bwd_ex(const void* d_grad_logits, int g_dtype
         if (px_blocks < 1) px_blocks = 1;
         if (px_blocks > 16) px_blocks = 16;
         dim3 grid((nblk + px_blocks - 1) / px_blocks, B, PREPF_CS);
-        k1b_prep_f32_kernel<<<grid, PREPF_W * 32, 0, st>>>((const float*)d_grad_logits, d_logits, B, C, C_pad, hw,
-                                                           n_sets, normalize, px_blocks, (__nv_bfloat16*)(ws + L.gbf),
-                                                           d_r, d_rt, raw_v ? d_inv_norm_v : nullptr);
+        LC2IS_CUDA(launch_pdl(k1b_prep_f32_kernel, grid, PREPF_W * 32, 0, st, (const float*)d_grad_logits, d_logits, B,
+                              C, C_pad, hw, n_sets, normalize, px_blocks, (__nv_bfloat16*)(ws + L.gbf), d_r, d_rt,
+                              raw_v ? d_inv_norm_v : nullptr));
         LC2IS_CHECK_LAUNCH("k1b_prep_f32_kernel");
     } else if (normalize) {
         dim3 grid((hw + PREP_PX - 1) / PREP_PX, B);
@@ -724,7 +738,7 @@ extern "C" int lc2is_cosine_logits_bwd_ex(const void* d_grad_logits, int g_dtype
         LC2IS_CUDA(cudaFuncSetAttribute(k1b_dv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         const int total_tiles = B * P.tiles_per_img * P.n_ntiles;
         int grid = sm_count() < total_tiles ? sm_count() : total_tiles;
-        k1b_dv_kernel<<<grid, DV_THREADS, smem, st>>>(tmG, tmT, P);
+        LC2IS_CUDA(launch_pdl(k1b_dv_kernel, grid, DV_THREADS, smem, st, tmG, tmT, P));
         LC2IS_CHECK_LAUNCH("k1b_dv_kernel");
     }
     // ---- dT ----------------------------------------------------------------------------------------
@@ -752,14 +766,14 @@ extern "C" int lc2is_cosine_logits_bwd_ex(const void* d_grad_logits, int g_dtype
         size_t smem = (size_t)stages * stage_bytes + 1024 + 256;
         if (smem < 120 * 1024) smem = 120 * 1024;
         LC2IS_CUDA(cudaFuncSetAttribute(k1b_dt_kernel<false, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k1b_dt_kernel<false, 1, false><<<base_items * ksplit, KB_THREADS, smem, st>>>(tmV, tmG, P);
+        LC2IS_CUDA(launch_pdl(k1b_dt_kernel<false, 1, false>, base_items * ksplit, KB_THREADS, smem, st, tmV, tmG, P));
         LC2IS_CHECK_LAUNCH("k1b_dt_kernel");
         long long total = (long long)n_sets * C * D;
         long long blocks = (total + 255) / 256;
         if (blocks > sm_count() * 8) blocks = sm_count() * 8;
-        k1b_dt_finish_kernel<<<(unsigned)blocks, 256, 0, st>>>(d_dtraw, d_rt, (const __nv_bfloat16*)d_t_hat,
-                                                               d_inv_norm_t, d_grad_scale, n_sets, C, C_pad, D,
-                                                               normalize, logit_scale, d_grad_t);
+        LC2IS_CUDA(launch_pdl(k1b_dt_finish_kernel, (unsigned)blocks, 256, 0, st, d_dtraw, d_rt,
+                              (const __nv_bfloat16*)d_t_hat, d_inv_norm_t, d_grad_scale, n_sets, C, C_pad, D, normalize,
+                              logit_scale, d_grad_t));
         LC2IS_CHECK_LAUNCH("k1b_dt_finish_kernel");
     }
     return 0;

@@ -737,6 +737,9 @@ k23_rc_kernel(const __grid_constant__ CUtensorMap tm, const __grid_constant__ RC
 #ifdef RC_STAMPS
     if (lane == 0) stp[RC_STAMP_SLOTS - 1] = (unsigned long long)sti;
 #endif
+    // the next kernel of the step (the gradient scale, then the logits backward) may be scheduled once the warp has no
+    // job left; it reads the gradient only after griddep_wait(), i.e. after this grid's last reduction has landed
+    griddep_launch_dependents();
     retire();
 }
 

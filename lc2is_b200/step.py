@@ -19,9 +19,10 @@ from ._lib import BF16, F32, check, lib, ptr, stream_ptr
 
 
 class _Block:
-    """Everything ONE step accumulates into, in one flat buffer that is zeroed with a single fill:
+    """Everything ONE step accumulates into, in one flat buffer whose head is zeroed with a single fill:
         [ grad bucket: grad_t (C*D) | loss_sum as fp32 (1) | pad ] [ grad_low (B*C*h*w) ]
-        [ scalars: double loss_sum | int64 n_valid | float gscale | float loss ]
+        [ scalars: double loss_sum | int64 n_valid | float gscale | float loss | pad ]
+        [ logits-backward workspace: its accumulators (zeroed too: LC2IS_BWD_WS_ZEROED) | the rest ]
     HeadStep keeps TWO of them and alternates, so that the gradient-bucket all-reduce of step i can stay in flight
     while step i+1 zero-fills and fills the other one."""
 
@@ -30,7 +31,12 @@ class _Block:
         nb_pad = (nb + 3) // 4 * 4
         ngl = B * C * h * w
         ngl_pad = (ngl + 3) // 4 * 4
-        self.acc32 = torch.zeros(nb_pad + ngl_pad + 8, dtype=torch.float32, device=dev)   # zeroed as fp32: 16-byte stores
+        ws_off = (nb_pad + ngl_pad + 8 + 63) // 64 * 64                                  # 256-byte aligned
+        ws_bytes = max(int(lib.lc2is_cosine_logits_bwd_workspace(B, h * w, D, 1, C)), 256)
+        ws_zero = int(lib.lc2is_cosine_logits_bwd_workspace_zeroed(B, h * w, D, 1, C))
+        self.acc32 = torch.zeros(ws_off + (ws_bytes + 3) // 4, dtype=torch.float32, device=dev)
+        self.zero_fill = self.acc32[:ws_off + (ws_zero + 3) // 4]                         # zeroed as fp32: 16-byte stores
+        self.bwd_ws = self.acc32[ws_off:]
         acc = self.acc32.view(torch.uint8)
         f32 = self.acc32[: nb_pad + ngl_pad]
         self.bucket = dp.GradBucket([(1, C, D), (1,)], dev, flat=f32[:nb])
@@ -118,8 +124,6 @@ class HeadStep:
         self._xs = torch.cuda.Stream(device=dev) if self.comm is not None else None
         self.confmat = torch.zeros(C, C, dtype=torch.int64, device=dev)        # this rank's counts, accumulated
         self._confmat_global = torch.zeros(C, C, dtype=torch.int64, device=dev) if self.distributed else None
-        nbytes = int(lib.lc2is_cosine_logits_bwd_workspace(B, self.hw, D, 1, C))
-        self.bwd_ws = torch.empty(max(nbytes, 256), dtype=torch.uint8, device=dev)
         self.k2_events = None          # optional (start, stop) CUDA events around the K2 call
         self._open = None
         self.timers = None             # optional {name: [(start, stop) CUDA events]} per section (bench --kernel-times)
@@ -278,7 +282,7 @@ class HeadStep:
         B, C, h, w, H, W = self.B, self.C, self.h, self.w, self.H, self.W
         blk = self._blocks[k]
         self._mark("zero-fill")
-        blk.acc32.zero_()                                        # bucket, grad_low, scalars: one fill
+        blk.zero_fill.zero_()                                    # bucket, grad_low, scalars, K1b accumulators: one fill
         glow = ptr(blk.grad_low) if self.backward else None
         self._mark("label prepass / count")
         # un-scaled gradients accumulate into grad_low on the split routes; 1/N_valid is applied by K1b, so the
@@ -330,8 +334,8 @@ class HeadStep:
                                                  ptr(v) if fuse else ptr(self.v_hat),
                                                  ptr(self.inv_v), ptr(self.t_hat), ptr(self.inv_t), B, hw, D, 1, C,
                                                  int(self.normalize), self.logit_scale, ptr(blk.gscale),
-                                                 ptr(self.grad_v), BF16, ptr(blk.grad_t), ptr(self.bwd_ws), st,
-                                                 _lib.BWD_RAW_V if fuse else 0),
+                                                 ptr(self.grad_v), BF16, ptr(blk.grad_t), ptr(blk.bwd_ws), st,
+                                                 _lib.BWD_WS_ZEROED | (_lib.BWD_RAW_V if fuse else 0)),
                   "cosine_logits_bwd")
         self._mark("K3 argmax+confmat")
         check(lib.lc2is_step_argmax(ptr(self.logits), ptr(labels), ptr(self.labels_packed), B, C, h, w, H, W,
